@@ -143,5 +143,7 @@ int chol_factor_inv(Ctx* c, cudaStream_t s, int m, int mp, const double* M, doub
 // for and chol_df_enabled(m)
 size_t chol_df_aux_bytes(int m);
 bool chol_df_enabled(int m);
+// worker CTAs of a data-flow chain with at most 8 block columns (m <= 512), where the spine bounds the chain; two per SM
+constexpr int DF_SMALL_WORKERS = 16;
 
 }  // namespace accbpg

@@ -1313,10 +1313,10 @@ int accbpg_dopt_grad(void* ctx, void* stream, const double* H, int m, int64_t n,
 }
 
 // Factor M (with the inverse) and form the gradient, with the triangular GEMM started before the Cholesky chain has
-// finished: the rows of row block ib of L^{-1} are final once block column 2ib+1 has retired, and the chain keeps at
-// most ~36 SMs busy, so the persistent triangular GEMM is launched per row block on a second stream as its rows
-// become final (on sm_count - 52 SMs), lowest row blocks first; the remaining row blocks follow on the main stream
-// after the chain, heaviest first, on all SMs.  Same results as accbpg_dopt_factor + accbpg_dopt_grad.
+// finished: the rows of row block ib of L^{-1} are final once block column 2ib+1 has retired, and the chain keeps only
+// a few SMs busy, so the persistent triangular GEMM is launched per row block on a second stream as its rows become
+// final (on the SMs the chains do not need: `reserve` below), lowest row blocks first; the remaining row blocks follow
+// on the main stream after the chain, heaviest first, on all SMs.  Same results as accbpg_dopt_factor + accbpg_dopt_grad.
 static int overlap_enabled() {          // read on every call: tools/bench_configs.py times the kernels one by one with it off
     const char* e = getenv("ACCBPG_OVERLAP");
     return (e && e[0] == '0') ? 0 : 1;
@@ -1357,8 +1357,13 @@ static int dopt_factor_grad(Ctx* c, cudaStream_t s, const double* H, int m, int6
     p.Linv = Linv; p.H = H; p.part = part; p.m = m; p.mp = pl.mp; p.nib = pl.nib; p.n = n; p.ldh = ldh; p.npad = pl.npad;
     int* counters = (int*)(c->d_counter + 8);                 // words 8 .. 13 of the context's ticket block
     ACCBPG_CUDA(cudaMemsetAsync(counters, 0, 6 * sizeof(int), s));
-    static int reserve = -1;                                  // SMs left to the Cholesky chains while they run
-    if (reserve < 0) { const char* e = getenv("ACCBPG_CHAIN_SMS"); reserve = e ? atoi(e) : 52; }
+    // SMs left to the Cholesky chains while they run.  Up to 8 block columns each chain is a spine CTA (an SM of its own)
+    // and DF_SMALL_WORKERS workers at two per SM; two chains run at once (f(x) on the side stream, this one), so 2 * (1 +
+    // 8) SMs and two spare (500x50000 ABPG: 1.116 -> 1.085 ms per iteration against 52, B200).  Larger chains keep 52.
+    static int reserve_env = -2;
+    if (reserve_env == -2) { const char* e = getenv("ACCBPG_CHAIN_SMS"); reserve_env = e ? atoi(e) : -1; }
+    const int reserve = reserve_env >= 0 ? reserve_env
+                                         : ((m + 63) / 64 <= 8 ? 2 * (1 + DF_SMALL_WORKERS / 2) + 2 : 52);
     int early_grid = c->sm_count - reserve;
     if (early_grid < 1) early_grid = 1;
     if ((int64_t)early_grid > npanels) early_grid = (int)npanels;
