@@ -32,7 +32,7 @@ struct Ctx {
     cudaStream_t side;      // side stream: a second latency-bound chain (Cholesky) runs next to the main one
     cudaEvent_t ev_fork, ev_join;
     cudaStream_t side2;     // early launches of the triangular GEMM, next to the tail of the Cholesky chain
-    cudaEvent_t ev_rows[4], ev_early_done;
+    cudaEvent_t ev_early_done;
     // deferred reads (accbpg_ctx_read_async / _wait): a ring of pinned buffers, one event each
     double* h_ring;         // kReadRing * (kSlots + 1) doubles; the last double of a row carries the status word
     cudaEvent_t ring_ev[8];

@@ -3,7 +3,6 @@
 // mma.sync.m8n8k4 tiles, k-slabs of 16 staged through a 4-deep cp.async pipeline into padded (bank-conflict-free)
 // shared memory.
 #pragma once
-#include <functional>
 #include "common.cuh"
 
 namespace accbpg {
@@ -137,10 +136,9 @@ __device__ __forceinline__ void mma_nn_slab(double (&acc)[MI][NI][2], const doub
 // L^-1 is final once fX[J] and fLi[J*nb + r], r < J, carry `epoch` in their upper 24 bits and a count >= 1
 struct DfGate { const int* fX; const int* fLi; int nb; int epoch; };
 int chol_factor_inv(Ctx* c, cudaStream_t s, int m, int mp, const double* M, double* L, int want_inv, double* Linv,
-                    double* W, double* Y, double* acc, double* d_out, const std::function<int(int)>* after_step = nullptr,
-                    void* aux = nullptr, DfGate* gate = nullptr);
-// data-flow form (two launches for the whole chain): used by chol_factor_inv when `aux` is given, no hook is asked
-// for and chol_df_enabled(m)
+                    double* W, double* Y, double* acc, double* d_out, void* aux = nullptr, DfGate* gate = nullptr);
+// data-flow form (two launches for the whole chain): used by chol_factor_inv when `aux` is given and chol_df_enabled(m)
+// (64 < m <= 4096); otherwise one launch per block column
 size_t chol_df_aux_bytes(int m);
 bool chol_df_enabled(int m);
 // worker CTAs of a data-flow chain with at most 8 block columns (m <= 512), where the spine bounds the chain; two per SM

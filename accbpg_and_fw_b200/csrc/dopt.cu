@@ -575,17 +575,16 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) trmm_colnorm_kernel(TrmmParam
 }
 
 // ------------------------------------------------------------------------------------------ K4, TMA mainloop
-// Same tile and triangular stop as trmm_colnorm_kernel.  A (rows of Linv) arrives as one swizzled 2-D TMA box per
-// k-slab, read with the permuted row mapping of syrk_tma_kernel (the column sums do not care which row is which);
-// B (16 rows of the H panel, 1 KB each) arrives as sixteen 1-D bulk copies into rows padded to BT_LD doubles, so the
-// B fragments keep the conflict-free padded addressing.  Rows k >= m of the last slab are not copied: Linv is zero
-// in those columns, so whatever finite values the (zero-initialised) stage holds there contribute nothing.
+// The stage layout of trmm_persistent_kernel; same tile and triangular stop as trmm_colnorm_kernel.  A (rows of Linv)
+// arrives as one swizzled 2-D TMA box per k-slab, read with the permuted row mapping of syrk_tma_kernel (the column sums
+// do not care which row is which); B (16 rows of the H panel, 1 KB each) arrives as sixteen 1-D bulk copies into rows
+// padded to BT_LD doubles, so the B fragments keep the conflict-free padded addressing.  Rows k >= m of the last slab
+// are not copied: Linv is zero in those columns, so whatever finite values the (zero-initialised) stage holds there
+// contribute nothing.
 constexpr int TRT_STAGES = 6;
-constexpr int TRT_PREFETCH = 4;
 constexpr int TRT_A_BYTES = BM * BK * 8;                                  // 16 KB, 1024-byte aligned
 constexpr int TRT_B_BYTES = ((BK * BT_LD * 8 + 1023) / 1024) * 1024;      // 16 x 132 doubles, padded to 17 KB
 constexpr int TRT_STAGE_BYTES = TRT_A_BYTES + TRT_B_BYTES;
-constexpr int TRT_SMEM = TRT_STAGES * TRT_STAGE_BYTES + 1024 + 256;
 
 __device__ __forceinline__ void bulk_load_1d(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
@@ -606,116 +605,6 @@ __device__ __forceinline__ void trmm_tma_slab(double (&acc)[MI][NI][2], uint32_t
         for (int i = 0; i < MI; ++i)
 #pragma unroll
             for (int j = 0; j < NI; ++j) dmma884(acc[i][j][0], acc[i][j][1], a[i], bq[j]);
-    }
-}
-
-__global__ void __launch_bounds__(GEMM_THREADS, 1)
-trmm_tma_kernel(TrmmParams p, const __grid_constant__ CUtensorMap tmL) {
-    extern __shared__ unsigned char smem_raw[];
-    const uint32_t smem0 = ((uint32_t)__cvta_generic_to_shared(smem_raw) + 1023u) & ~1023u;
-    unsigned char* smem_gen = smem_raw + (smem0 - (uint32_t)__cvta_generic_to_shared(smem_raw));
-    const uint32_t bars = smem0 + TRT_STAGES * TRT_STAGE_BYTES;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int g = lane >> 2, t = lane & 3;
-    const int wm = warp >> 2, wn = warp & 3;
-    const int ib = p.nib - 1 - blockIdx.x;            // heavy row blocks first
-    const int64_t j0 = (int64_t)blockIdx.y * BN;
-    int kmax = (ib + 1) * BM;
-    const int m16 = (p.m + BK - 1) / BK * BK;
-    if (kmax > m16) kmax = m16;
-    const int KT = kmax / BK;
-    const int klim = ib * BM + wm * 32 + 32;          // this warp's rows end at this column of Linv
-    int64_t ncols = p.n - j0;                         // valid columns of the panel (even: the aligned path only)
-    if (ncols > BN) ncols = BN;
-    const uint32_t row_bytes = (uint32_t)ncols * 8;
-
-    // zero the B regions once (see above), then set up the barriers
-    for (int st = 0; st < TRT_STAGES; ++st) {
-        double* bz = reinterpret_cast<double*>(smem_gen + st * TRT_STAGE_BYTES + TRT_A_BYTES);
-        for (int e = tid; e < BK * BT_LD; e += GEMM_THREADS) bz[e] = 0.0;
-    }
-    if (tid == 0) {
-        for (int s = 0; s < TRT_STAGES; ++s) {
-            mbar_init(bars + 8 * s, 1);
-            mbar_init(bars + 8 * (TRT_STAGES + s), GEMM_THREADS / 32);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");      // generic-proxy zero fill before async-proxy writes
-    __syncthreads();
-
-    auto issue = [&](int s) {
-        const int st = s % TRT_STAGES;
-        const uint32_t base = smem0 + st * TRT_STAGE_BYTES, full = bars + 8 * st;
-        const int k0 = s * BK;
-        int rows = p.m - k0;
-        rows = rows > BK ? BK : rows;
-        mbar_arrive_expect_tx(full, TRT_A_BYTES + (uint32_t)rows * row_bytes);
-        tma_load_2d(base, &tmL, k0, ib * BM, full);
-        const double* src = p.H + (int64_t)k0 * p.ldh + j0;
-        for (int r = 0; r < rows; ++r)
-            bulk_load_1d(base + TRT_A_BYTES + r * BT_LD * 8, src + (int64_t)r * p.ldh, row_bytes, full);
-    };
-    if (tid == 0) {
-        const int pre = KT < TRT_PREFETCH ? KT : TRT_PREFETCH;
-        for (int s = 0; s < pre; ++s) issue(s);
-    }
-
-    double acc[MI][NI][2];
-#pragma unroll
-    for (int i = 0; i < MI; ++i)
-#pragma unroll
-        for (int j = 0; j < NI; ++j) acc[i][j][0] = acc[i][j][1] = 0.0;
-
-    uint32_t offA[2];
-#pragma unroll
-    for (int pq = 0; pq < 2; ++pq) {
-        const int ra = wm * 32 + 2 * g + pq;
-        offA[pq] = ra * 128 + ((((t >> 1) ^ (ra & 7))) << 4) + (t & 1) * 8;
-    }
-    const uint32_t offB = TRT_A_BYTES + (t * BT_LD + wn * 32 + g) * 8;
-
-    for (int s = 0; s < KT; ++s) {
-        const int st = s % TRT_STAGES;
-        const uint32_t base = smem0 + st * TRT_STAGE_BYTES;
-        if (tid == 0) {
-            const int sn = s + TRT_PREFETCH;
-            if (sn < KT) {
-                if (sn >= TRT_STAGES) mbar_wait(bars + 8 * (TRT_STAGES + sn % TRT_STAGES), ((sn / TRT_STAGES) + 1) & 1);
-                issue(sn);
-            }
-        }
-        mbar_wait(bars + 8 * st, (s / TRT_STAGES) & 1);
-        int k4 = (klim - s * BK) >> 2;
-        k4 = k4 < 0 ? 0 : (k4 > BK / 4 ? BK / 4 : k4);
-        if (k4 == BK / 4) trmm_tma_slab<BK / 4>(acc, base, offA, offB);       // the common case, fully unrolled
-        else if (k4 == 3) trmm_tma_slab<3>(acc, base, offA, offB);
-        else if (k4 == 2) trmm_tma_slab<2>(acc, base, offA, offB);
-        else if (k4 == 1) trmm_tma_slab<1>(acc, base, offA, offB);
-        __syncwarp();
-        if (lane == 0) mbar_arrive(bars + 8 * (TRT_STAGES + st));
-    }
-    __syncthreads();      // every stage has been consumed: reuse the front of smem for the column exchange
-
-    double* colx = reinterpret_cast<double*>(smem_gen);      // [4][128]
-#pragma unroll
-    for (int j = 0; j < NI; ++j) {
-#pragma unroll
-        for (int e = 0; e < 2; ++e) {
-            double sq = 0.0;
-#pragma unroll
-            for (int i = 0; i < MI; ++i) sq = fma(acc[i][j][e], acc[i][j][e], sq);
-            sq += __shfl_xor_sync(0xffffffffu, sq, 4);
-            sq += __shfl_xor_sync(0xffffffffu, sq, 8);
-            sq += __shfl_xor_sync(0xffffffffu, sq, 16);
-            if (g == 0) colx[wm * BN + wn * 32 + j * 8 + 2 * t + e] = sq;
-        }
-    }
-    __syncthreads();
-    if (tid < BN) {
-        int64_t col = j0 + tid;
-        if (col < p.n)
-            p.part[(size_t)ib * p.npad + col] = ((colx[tid] + colx[BN + tid]) + colx[2 * BN + tid]) + colx[3 * BN + tid];
     }
 }
 
@@ -1027,7 +916,6 @@ static int ensure_smem_attrs() {
     ACCBPG_CUDA(cudaFuncSetAttribute(syrk_dmma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, KMAJOR_SMEM));
     ACCBPG_CUDA(cudaFuncSetAttribute(syrk_dmma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, KMAJOR_SMEM));
     ACCBPG_CUDA(cudaFuncSetAttribute(syrk_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TMA_SMEM));
-    ACCBPG_CUDA(cudaFuncSetAttribute(trmm_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TRT_SMEM));
     ACCBPG_CUDA(cudaFuncSetAttribute(trmm_persistent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TRP_SMEM));
     ACCBPG_CUDA(cudaFuncSetAttribute(trmm_colnorm_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, NN_SMEM));
     ACCBPG_CUDA(cudaFuncSetAttribute(trmm_colnorm_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, NN_SMEM));
@@ -1055,14 +943,18 @@ static EncodeTiledFn encode_tiled_fn() {
     }
     return fn;
 }
-// 0: cp.async mainloop, 1: TMA mainloop (default when the operands allow it); ACCBPG_SYRK_TMA=0 switches it off
-static bool syrk_tma_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("ACCBPG_SYRK_TMA");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v == 1;
+
+// A operand of trmm_persistent_kernel: L^-1 (mp x mp, ld mp) in 128-row x 16-column boxes with the 128-byte swizzle.
+// False when the driver has no tensor-map entry point or the encoding fails.
+static bool encode_linv_tmap(CUtensorMap* tmL, const double* Linv, int mp) {
+    EncodeTiledFn fn = encode_tiled_fn();
+    if (!fn) return false;
+    cuuint64_t dimL[2] = {(cuuint64_t)mp, (cuuint64_t)mp};
+    cuuint64_t strL[1] = {(cuuint64_t)mp * 8};
+    cuuint32_t boxL[2] = {BK, BM};
+    cuuint32_t one[2] = {1, 1};
+    return fn(tmL, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, (void*)Linv, dimL, strL, boxL, one, CU_TENSOR_MAP_INTERLEAVE_NONE,
+              CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
 // 2-D FP64 tensor map (no swizzle, zero fill outside) over a row-major matrix with `cols` columns, `rows` rows and leading
@@ -1127,7 +1019,7 @@ static int syrk_partials(Ctx* c, cudaStream_t s, const double* H, int m, int64_t
     dim3 grid(pl.n_off * pl.s_off + pl.nt * pl.s_diag);
     bool al = aligned16(H) && aligned16(x) && (ldh % 2 == 0);
     bool launched = false;
-    if (al && syrk_tma_enabled() && encode_tiled_fn() && n < (1LL << 31)) {
+    if (al && encode_tiled_fn() && n < (1LL << 31)) {
         CUtensorMap tmH, tmX;
         cuuint64_t dimH[2] = {(cuuint64_t)n, (cuuint64_t)m};
         cuuint64_t strH[1] = {(cuuint64_t)ldh * 8};
@@ -1249,7 +1141,7 @@ int accbpg_dopt_factor(void* ctx, void* stream, int m, const double* M, double* 
     double* W = (double*)((char*)ws + pl.off_W);
     if (M == W || L == W) return arg_err("dopt_factor: M / L alias the factor scratch");
     return chol_factor_inv(c, s, m, pl.mp, M, L, want_inverse ? 1 : 0, (double*)((char*)ws + pl.off_Linv), W,
-                           (double*)((char*)ws + pl.off_Y), c->d_slots + 248, d_out, nullptr, (char*)ws + pl.off_aux);
+                           (double*)((char*)ws + pl.off_Y), c->d_slots + 248, d_out, (char*)ws + pl.off_aux);
 }
 
 int accbpg_dopt_grad(void* ctx, void* stream, const double* H, int m, int64_t n, int64_t ldh, void* ws, double* g) {
@@ -1268,36 +1160,18 @@ int accbpg_dopt_grad(void* ctx, void* stream, const double* H, int m, int64_t n,
     p.n = n; p.ldh = ldh; p.npad = pl.npad;
     int64_t npanels = (n + BN - 1) / BN;
     if (npanels > 65535) return arg_err("dopt_grad: n_local too large for one launch (max 65535*128 columns)");
-    dim3 grid(pl.nib, (unsigned)npanels);
-    bool al = aligned16(H) && (ldh % 2 == 0);
-    bool launched = false;
-    if (al && (n % 2 == 0) && syrk_tma_enabled() && encode_tiled_fn()) {
-        CUtensorMap tmL;
-        cuuint64_t dimL[2] = {(cuuint64_t)pl.mp, (cuuint64_t)pl.mp};
-        cuuint64_t strL[1] = {(cuuint64_t)pl.mp * 8};
-        cuuint32_t boxL[2] = {BK, BM};
-        cuuint32_t one[2] = {1, 1};
-        CUresult r1 = encode_tiled_fn()(&tmL, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, (void*)Linv, dimL, strL, boxL, one,
-                                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                                        CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r1 == CUDA_SUCCESS) {
-            const int64_t ntiles = (int64_t)pl.nib * npanels;
-            static int persistent = -1;
-            if (persistent < 0) { const char* e = getenv("ACCBPG_TRMM_PERSISTENT"); persistent = (e && e[0] == '0') ? 0 : 1; }
-            if (persistent && ntiles < (1LL << 30)) {
-                int* counter = (int*)(c->d_counter + 8);      // a second ticket word of the context
-                ACCBPG_CUDA(cudaMemsetAsync(counter, 0, sizeof(int), s));
-                const int pgrid = (int)(ntiles < c->sm_count ? ntiles : c->sm_count);
-                ProfScope ps(P_TRMM, s);
-                trmm_persistent_kernel<<<pgrid, TRP_THREADS, TRP_SMEM, s>>>(p, tmL, counter, 0, (int)ntiles);
-            } else {
-                ProfScope ps(P_TRMM, s);
-                trmm_tma_kernel<<<grid, GEMM_THREADS, TRT_SMEM, s>>>(p, tmL);
-            }
-            launched = true;
-        }
-    }
-    if (!launched) {
+    const int64_t ntiles = (int64_t)pl.nib * npanels;
+    if (ntiles >= (1LL << 30)) return arg_err("dopt_grad: m x n_local too large for one launch (2^30 128x128 tiles)");
+    const bool al = aligned16(H) && (ldh % 2 == 0);
+    CUtensorMap tmL;
+    if (al && (n % 2 == 0) && encode_linv_tmap(&tmL, Linv, pl.mp)) {
+        int* counter = (int*)(c->d_counter + 8);      // a second ticket word of the context
+        ACCBPG_CUDA(cudaMemsetAsync(counter, 0, sizeof(int), s));
+        const int pgrid = (int)(ntiles < c->sm_count ? ntiles : c->sm_count);
+        ProfScope ps(P_TRMM, s);
+        trmm_persistent_kernel<<<pgrid, TRP_THREADS, TRP_SMEM, s>>>(p, tmL, counter, 0, (int)ntiles);
+    } else {
+        const dim3 grid(pl.nib, (unsigned)npanels);
         ProfScope ps(P_TRMM, s);
         if (al) trmm_colnorm_kernel<true><<<grid, GEMM_THREADS, NN_SMEM, s>>>(p);
         else    trmm_colnorm_kernel<false><<<grid, GEMM_THREADS, NN_SMEM, s>>>(p);
@@ -1314,9 +1188,11 @@ int accbpg_dopt_grad(void* ctx, void* stream, const double* H, int m, int64_t n,
 
 // Factor M (with the inverse) and form the gradient, with the triangular GEMM started before the Cholesky chain has
 // finished: the rows of row block ib of L^{-1} are final once block column 2ib+1 has retired, and the chain keeps only
-// a few SMs busy, so the persistent triangular GEMM is launched per row block on a second stream as its rows become
-// final (on the SMs the chains do not need: `reserve` below), lowest row blocks first; the remaining row blocks follow
-// on the main stream after the chain, heaviest first, on all SMs.  Same results as accbpg_dopt_factor + accbpg_dopt_grad.
+// a few SMs busy.  With the data-flow chain, the first n_early row blocks are one persistent launch on a second stream
+// (on the SMs the chains do not need: `reserve` below) whose producer waits on the chain's progress counters before it
+// loads a row block of L^{-1}, lowest row blocks first; the remaining row blocks follow on the main stream after the
+// chain, heaviest first, on all SMs.  Same results as accbpg_dopt_factor + accbpg_dopt_grad, which is the route taken
+// whenever the overlap cannot run (one launch per block column in the chain, unaligned or odd-width H, one row block).
 static int overlap_enabled() {          // read on every call: tools/bench_configs.py times the kernels one by one with it off
     const char* e = getenv("ACCBPG_OVERLAP");
     return (e && e[0] == '0') ? 0 : 1;
@@ -1332,31 +1208,21 @@ static int dopt_factor_grad(Ctx* c, cudaStream_t s, const double* H, int m, int6
     if (early_env == -2) { const char* e = getenv("ACCBPG_EARLY_BLOCKS"); early_env = e ? atoi(e) : -1; }
     int n_early = pl.nib / 2 < 4 ? pl.nib / 2 : 4;            // row blocks 0 .. n_early-1 start under the chain
     if (early_env >= 0) n_early = early_env < pl.nib - 1 ? early_env : pl.nib - 1;
-    if (!overlap_enabled() || !al || !syrk_tma_enabled() || !encode_tiled_fn() || n_early < 1 || ntiles >= (1LL << 30)) {
+    double* Linv = (double*)((char*)ws + pl.off_Linv);
+    double* part = (double*)((char*)ws + pl.off_part);
+    CUtensorMap tmL;
+    if (!overlap_enabled() || !al || !chol_df_enabled(m) || n_early < 1 || ntiles >= (1LL << 30) ||
+        !encode_linv_tmap(&tmL, Linv, pl.mp)) {
         int rc = accbpg_dopt_factor(c, s, m, M, nullptr, 1, ws, d_f_out);
         if (rc) return rc;
         return accbpg_dopt_grad(c, s, H, m, n, ldh, ws, g);
     }
     int rc = ensure_smem_attrs();
     if (rc) return rc;
-    double* Linv = (double*)((char*)ws + pl.off_Linv);
-    double* part = (double*)((char*)ws + pl.off_part);
-    CUtensorMap tmL;
-    cuuint64_t dimL[2] = {(cuuint64_t)pl.mp, (cuuint64_t)pl.mp};
-    cuuint64_t strL[1] = {(cuuint64_t)pl.mp * 8};
-    cuuint32_t boxL[2] = {BK, BM};
-    cuuint32_t one[2] = {1, 1};
-    if (encode_tiled_fn()(&tmL, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, (void*)Linv, dimL, strL, boxL, one,
-                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) {
-        rc = accbpg_dopt_factor(c, s, m, M, nullptr, 1, ws, d_f_out);
-        if (rc) return rc;
-        return accbpg_dopt_grad(c, s, H, m, n, ldh, ws, g);
-    }
     TrmmParams p;
     p.Linv = Linv; p.H = H; p.part = part; p.m = m; p.mp = pl.mp; p.nib = pl.nib; p.n = n; p.ldh = ldh; p.npad = pl.npad;
-    int* counters = (int*)(c->d_counter + 8);                 // words 8 .. 13 of the context's ticket block
-    ACCBPG_CUDA(cudaMemsetAsync(counters, 0, 6 * sizeof(int), s));
+    int* counters = (int*)(c->d_counter + 8);                 // words 8 (late launch) and 9 (early launch) of the ticket block
+    ACCBPG_CUDA(cudaMemsetAsync(counters, 0, 2 * sizeof(int), s));
     // SMs left to the Cholesky chains while they run.  Up to 8 block columns each chain is a spine CTA (an SM of its own)
     // and DF_SMALL_WORKERS workers at two per SM; two chains run at once (f(x) on the side stream, this one), so 2 * (1 +
     // 8) SMs and two spare (500x50000 ABPG: 1.116 -> 1.085 ms per iteration against 52, B200).  Larger chains keep 52.
@@ -1367,64 +1233,32 @@ static int dopt_factor_grad(Ctx* c, cudaStream_t s, const double* H, int m, int6
     int early_grid = c->sm_count - reserve;
     if (early_grid < 1) early_grid = 1;
     if ((int64_t)early_grid > npanels) early_grid = (int)npanels;
-    // side2 must not start before the main stream has reached this point (Linv memset, counters, earlier readers of part)
+    // side2 must not start before the main stream has reached this point (counters, earlier readers of part)
     ACCBPG_CUDA(cudaEventRecord(c->ev_fork, s));
     ACCBPG_CUDA(cudaStreamWaitEvent(c->side2, c->ev_fork, 0));
     ProfScope ps_all(P_TRINV, s);                             // chain + triangular GEMM as one interval
-    if (chol_df_enabled(m)) {
-        // data-flow chain (two launches): the early row blocks are ONE gated persistent launch on the second stream that
-        // walks them lightest first and starts each as soon as the chain's counters say its rows of L^-1 are final
-        DfGate gate;
-        rc = chol_factor_inv(c, s, m, pl.mp, M, nullptr, 1, Linv, (double*)((char*)ws + pl.off_W),
-                             (double*)((char*)ws + pl.off_Y), c->d_slots + 248, d_f_out, nullptr, (char*)ws + pl.off_aux, &gate);
-        if (rc) return rc;
-        TrmmParams pe = p;
-        pe.gate_fX = gate.fX; pe.gate_fLi = gate.fLi; pe.gate_nb = gate.nb; pe.gate_epoch = gate.epoch; pe.ascending = 1;
-        // panels of row block 0 kept for the end of the late launch (ACCBPG_TRMM_HOLD, per cent of the panels; only when the
-        // tiles are long against the whole gradient, i.e. few tiles per SM: at m = 2000 a tile is 0.2 % of an SM's share)
-        static int hold_pct = -1;
-        if (hold_pct < 0) { const char* e = getenv("ACCBPG_TRMM_HOLD"); hold_pct = e ? atoi(e) : 35; if (hold_pct < 0 || hold_pct > 90) hold_pct = 0; }
-        int hold0 = 0;
-        if (n_early >= 2 && ntiles < 64LL * c->sm_count) hold0 = (int)(npanels * hold_pct / 100);
-        pe.hold0 = hold0;
-        trmm_persistent_kernel<<<early_grid, TRP_THREADS, TRP_SMEM, c->side2>>>(pe, tmL, counters + 1, 0, (int)(n_early * npanels) - hold0);
-        ACCBPG_LAUNCHED("trmm_persistent_kernel");
-        ACCBPG_CUDA(cudaEventRecord(c->ev_early_done, c->side2));
-        const int limit = (int)((pl.nib - n_early) * npanels) + hold0;
-        const int pgrid = (int)((int64_t)c->sm_count < (int64_t)limit ? c->sm_count : limit);
-        TrmmParams pl2 = p;
-        pl2.ext_cnt = hold0;
-        trmm_persistent_kernel<<<pgrid, TRP_THREADS, TRP_SMEM, s>>>(pl2, tmL, counters, 0, limit);
-        ACCBPG_LAUNCHED("trmm_persistent_kernel");
-        ACCBPG_CUDA(cudaStreamWaitEvent(s, c->ev_early_done, 0));
-        int fgd = grid_for(c, n, 256, 2, 8);
-        grad_finalize_kernel<<<fgd, 256, 0, s>>>(part, pl.nib, pl.npad, n, g);
-        ACCBPG_LAUNCHED("grad_finalize_kernel");
-        return ACCBPG_OK;
-    }
-    std::function<int(int)> hook = [&](int J) -> int {
-        if ((J & 1) == 0) return 0;
-        const int ib = J >> 1;                                // rows of row block ib are final
-        if (ib >= n_early) return 0;
-        if (cudaEventRecord(c->ev_rows[ib], s) != cudaSuccess) return -ACCBPG_E_CUDA;
-        if (cudaStreamWaitEvent(c->side2, c->ev_rows[ib], 0) != cudaSuccess) return -ACCBPG_E_CUDA;
-        // LPT numbering: row block ib owns tiles [(nib-1-ib) npanels, (nib-ib) npanels)
-        const int first = (int)((pl.nib - 1 - ib) * npanels), limit = (int)((pl.nib - ib) * npanels);
-        trmm_persistent_kernel<<<early_grid, TRP_THREADS, TRP_SMEM, c->side2>>>(p, tmL, counters + 1 + ib, first, limit);
-        ++g_launches;
-        if (cudaGetLastError() != cudaSuccess) return -ACCBPG_E_CUDA;
-        return 1;
-    };
+    DfGate gate;
     rc = chol_factor_inv(c, s, m, pl.mp, M, nullptr, 1, Linv, (double*)((char*)ws + pl.off_W),
-                         (double*)((char*)ws + pl.off_Y), c->d_slots + 248, d_f_out, &hook);
+                         (double*)((char*)ws + pl.off_Y), c->d_slots + 248, d_f_out, (char*)ws + pl.off_aux, &gate);
     if (rc) return rc;
+    TrmmParams pe = p;
+    pe.gate_fX = gate.fX; pe.gate_fLi = gate.fLi; pe.gate_nb = gate.nb; pe.gate_epoch = gate.epoch; pe.ascending = 1;
+    // panels of row block 0 kept for the end of the late launch (ACCBPG_TRMM_HOLD, per cent of the panels; only when the
+    // tiles are long against the whole gradient, i.e. few tiles per SM: at m = 2000 a tile is 0.2 % of an SM's share)
+    static int hold_pct = -1;
+    if (hold_pct < 0) { const char* e = getenv("ACCBPG_TRMM_HOLD"); hold_pct = e ? atoi(e) : 35; if (hold_pct < 0 || hold_pct > 90) hold_pct = 0; }
+    int hold0 = 0;
+    if (n_early >= 2 && ntiles < 64LL * c->sm_count) hold0 = (int)(npanels * hold_pct / 100);
+    pe.hold0 = hold0;
+    trmm_persistent_kernel<<<early_grid, TRP_THREADS, TRP_SMEM, c->side2>>>(pe, tmL, counters + 1, 0, (int)(n_early * npanels) - hold0);
+    ACCBPG_LAUNCHED("trmm_persistent_kernel");
     ACCBPG_CUDA(cudaEventRecord(c->ev_early_done, c->side2));
-    {   // the late row blocks, heaviest first, on every SM that is free
-        const int limit = (int)((pl.nib - n_early) * npanels);
-        const int pgrid = (int)((int64_t)c->sm_count < (int64_t)limit ? c->sm_count : limit);
-        trmm_persistent_kernel<<<pgrid, TRP_THREADS, TRP_SMEM, s>>>(p, tmL, counters, 0, limit);
-        ACCBPG_LAUNCHED("trmm_persistent_kernel");
-    }
+    const int limit = (int)((pl.nib - n_early) * npanels) + hold0;
+    const int pgrid = (int)((int64_t)c->sm_count < (int64_t)limit ? c->sm_count : limit);
+    TrmmParams pl2 = p;
+    pl2.ext_cnt = hold0;
+    trmm_persistent_kernel<<<pgrid, TRP_THREADS, TRP_SMEM, s>>>(pl2, tmL, counters, 0, limit);
+    ACCBPG_LAUNCHED("trmm_persistent_kernel");
     ACCBPG_CUDA(cudaStreamWaitEvent(s, c->ev_early_done, 0));
     int fg = grid_for(c, n, 256, 2, 8);
     grad_finalize_kernel<<<fg, 256, 0, s>>>(part, pl.nib, pl.npad, n, g);
@@ -1447,6 +1281,18 @@ int accbpg_dopt_func_grad(void* ctx, void* stream, const double* H, int m, int64
     return accbpg_dopt_factor(ctx, stream, m, M, NULL, 0, ws, d_f_out ? d_f_out : (c->d_slots + 249));
 }
 
+// -log det M (value only) on the context's side stream, started after the work queued so far on s; ev_join marks
+// its end.  Uses the second set of factor buffers (off_W2, off_aux2), so it can run next to a factorisation on s.
+static int value_on_side(Ctx* c, cudaStream_t s, const DoptPlan& pl, int m, const double* M, void* ws, double* d_out) {
+    ACCBPG_CUDA(cudaEventRecord(c->ev_fork, s));
+    ACCBPG_CUDA(cudaStreamWaitEvent(c->side, c->ev_fork, 0));
+    int rc = chol_factor_inv(c, c->side, m, pl.mp, M, NULL, 0, NULL, (double*)((char*)ws + pl.off_W2), NULL,
+                             c->d_slots + 246, d_out, (char*)ws + pl.off_aux2);
+    if (rc) return rc;
+    ACCBPG_CUDA(cudaEventRecord(c->ev_join, c->side));
+    return ACCBPG_OK;
+}
+
 // f(xf) and (f(yg), grad f(yg)) in one call: the two Gram matrices are formed back to back on the main stream, then
 // the value-only Cholesky runs on the context's side stream while the main stream factors M(yg), inverts L and
 // streams the gradient.  Both chains are latency bound on a handful of SMs, so they overlap almost completely.
@@ -1462,12 +1308,8 @@ int accbpg_dopt_pair(void* ctx, void* stream, const double* H, int m, int64_t n,
     double* M2 = (double*)((char*)ws + pl.off_M2);
     int rc = accbpg_dopt_gram(ctx, stream, H, m, n, ldh, xf, ws, M2);
     if (rc) return rc;
-    ACCBPG_CUDA(cudaEventRecord(c->ev_fork, s));
-    ACCBPG_CUDA(cudaStreamWaitEvent(c->side, c->ev_fork, 0));
-    rc = chol_factor_inv(c, c->side, m, pl.mp, M2, NULL, 0, NULL, (double*)((char*)ws + pl.off_W2), NULL,
-                         c->d_slots + 246, d_fx_out, nullptr, (char*)ws + pl.off_aux2);
+    rc = value_on_side(c, s, pl, m, M2, ws, d_fx_out);
     if (rc) return rc;
-    ACCBPG_CUDA(cudaEventRecord(c->ev_join, c->side));
     rc = accbpg_dopt_gram(ctx, stream, H, m, n, ldh, yg, ws, M1);
     if (rc) return rc;
     rc = dopt_factor_grad(c, s, H, m, n, ldh, M1, ws, d_fy_out ? d_fy_out : (c->d_slots + 249), g);
@@ -1490,12 +1332,8 @@ int accbpg_dopt_pair_from_gram(void* ctx, void* stream, const double* H, int m, 
     DoptPlan pl = make_plan(m, n, c->sm_count);
     int rc;
     if (Mx) {
-        ACCBPG_CUDA(cudaEventRecord(c->ev_fork, s));
-        ACCBPG_CUDA(cudaStreamWaitEvent(c->side, c->ev_fork, 0));
-        rc = chol_factor_inv(c, c->side, m, pl.mp, Mx, NULL, 0, NULL, (double*)((char*)ws + pl.off_W2), NULL,
-                             c->d_slots + 246, d_fx_out, nullptr, (char*)ws + pl.off_aux2);
+        rc = value_on_side(c, s, pl, m, Mx, ws, d_fx_out);
         if (rc) return rc;
-        ACCBPG_CUDA(cudaEventRecord(c->ev_join, c->side));
     }
     if (flag_y >= 1) rc = dopt_factor_grad(c, s, H, m, n, ldh, My, ws, d_fy_out ? d_fy_out : (c->d_slots + 249), g);
     else rc = accbpg_dopt_factor(ctx, stream, m, My, NULL, 0, ws, d_fy_out ? d_fy_out : (c->d_slots + 249));

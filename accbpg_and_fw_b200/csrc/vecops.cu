@@ -817,7 +817,6 @@ int accbpg_ctx_create(void** out) {
     ACCBPG_CUDA(cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
     ACCBPG_CUDA(cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming));
     ACCBPG_CUDA(cudaStreamCreateWithFlags(&c->side2, cudaStreamNonBlocking));
-    for (int i = 0; i < 4; ++i) ACCBPG_CUDA(cudaEventCreateWithFlags(&c->ev_rows[i], cudaEventDisableTiming));
     ACCBPG_CUDA(cudaEventCreateWithFlags(&c->ev_early_done, cudaEventDisableTiming));
     c->coop_blocks_burg = 0;
     c->burg_calls = 0;
@@ -835,7 +834,6 @@ int accbpg_ctx_destroy(void* ctx) {
     cudaFreeHost(c->h_slots); cudaFreeHost(c->h_status);
     cudaStreamDestroy(c->side); cudaEventDestroy(c->ev_fork); cudaEventDestroy(c->ev_join);
     cudaStreamDestroy(c->side2); cudaEventDestroy(c->ev_early_done);
-    for (int i = 0; i < 4; ++i) cudaEventDestroy(c->ev_rows[i]);
     delete c;
     return ACCBPG_OK;
 }

@@ -27,7 +27,9 @@ def rel(a, b):
 @pytest.mark.parametrize("m,n,seed", [(80, 200, 10), (30, 1000, 3), (129, 517, 7), (5, 6, 1), (64, 4096, 2),
                                       (200, 3001, 4), (300, 20000, 5),
                                       # TMA mainloops with ragged tiles: m just past a 128 / 64 boundary, n not a multiple of 16
-                                      (129, 520, 8), (257, 1030, 9), (65, 130, 11), (384, 4098, 12), (1, 2, 13)])
+                                      (129, 520, 8), (257, 1030, 9), (65, 130, 11), (384, 4098, 12), (1, 2, 13),
+                                      # 65 block columns: one launch per block column, then the gradient after the chain
+                                      (4160, 8322, 14)])
 def test_dopt_func_grad_vs_oracle(acc, m, n, seed):
     rng = np.random.RandomState(seed)
     f, h, L, x0 = acc.D_opt_design(m, n, randseed=seed)

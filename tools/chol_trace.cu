@@ -61,7 +61,7 @@ int main(int argc, char** argv) {
         for (int want = 1; want >= 0; --want) {
             for (int rep = 0; rep < 3; ++rep) {
                 cudaEventRecord(e0, s);
-                int rc = chol_factor_inv(&c, s, m, mp, dM, nullptr, want, dLinv, dW, dY, dacc, dacc + 1, nullptr, aux);
+                int rc = chol_factor_inv(&c, s, m, mp, dM, nullptr, want, dLinv, dW, dY, dacc, dacc + 1, aux);
                 cudaEventRecord(e1, s);
                 cudaStreamSynchronize(s);
                 float ms; cudaEventElapsedTime(&ms, e0, e1);
