@@ -172,17 +172,34 @@ class SparseDOptimalObj(RSmoothFunction):
     (accbpg_dopt_sparse_gram / accbpg_dopt_sparse_grad); the m x m factorisation is the dense chain.  m <= 128, one GPU.
 
     indptr / indices / values: the CSC arrays of H (= the CSR arrays of the samples-by-features matrix X), or pass a
-    scipy.sparse matrix H as the first argument.  `f.H` is the scipy CSC matrix (host); `f.toarray()` the dense H."""
+    scipy.sparse matrix H as the first argument.  `f.H` is the scipy CSC matrix (host); `f.toarray()` the dense H.
+    Either form is brought to canonical CSC on the host (rows sorted within a column, duplicate (row, column) entries
+    summed, as scipy's toarray() does); the caller's arrays are not modified."""
 
     _lin_capable = True
 
     def __init__(self, indptr, indices=None, values=None, m=None, device=None):
+        import scipy.sparse as sp
         self.rt = Runtime.get(device)
         self.shard = None
         if indices is None:                                   # a scipy.sparse matrix
-            Hs = indptr.tocsc()
-            Hs.sort_indices()
-            indptr, indices, values, m = Hs.indptr, Hs.indices, Hs.data, Hs.shape[0]
+            Hs = sp.csc_matrix(indptr, dtype=np.float64, copy=True)
+        else:
+            indptr = np.asarray(indptr, dtype=np.int64)
+            indices = np.asarray(indices)
+            values = np.asarray(values, dtype=np.float64)
+            assert indptr.ndim == 1 and indptr.size >= 1 and indptr[0] == 0 and np.all(np.diff(indptr) >= 0), \
+                "SparseDOptimalObj: indptr must start at 0 and be non-decreasing"
+            assert indices.size == values.size == int(indptr[-1]), "SparseDOptimalObj: indices / values / indptr sizes"
+            assert indices.size == 0 or (indices.min() >= 0 and indices.max() < int(m)), \
+                "SparseDOptimalObj: row index outside [0, m)"
+            Hs = sp.csc_matrix((values.copy(), indices.copy(), indptr.copy()), shape=(int(m), indptr.size - 1))
+        assert Hs.indices.size == 0 or (Hs.indices.min() >= 0 and Hs.indices.max() < Hs.shape[0]), \
+            "SparseDOptimalObj: row index outside [0, m)"
+        # The Gram kernel scatters a column's entries into a dense tile (one write per (row, column)) while the gradient
+        # kernel sums over every stored entry: duplicates must be merged here for the two to describe the same H.
+        Hs.sum_duplicates()
+        indptr, indices, values, m = Hs.indptr, Hs.indices, Hs.data, Hs.shape[0]
         self._indptr_h = np.ascontiguousarray(indptr, dtype=np.int64)
         self._indices_h = np.ascontiguousarray(indices, dtype=np.int32)
         self._values_h = np.ascontiguousarray(values, dtype=np.float64)
