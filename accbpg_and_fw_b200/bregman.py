@@ -199,10 +199,7 @@ class BurgEntropySimplex(BurgEntropy):
         # column-sharded: every rank gathers all slices of gg = (g [+ L/y]) / L (padding +inf) - pushed straight into every
         # rank's gathered vector over NVLink peer memory, else an NCCL all-gather - and replays the whole recurrence on
         # the gathered vector, so there is ONE exchange per prox call, no host round trip, and the multiplier c is
-        # bit-identical on every rank (and independent of the sharding).  (config.burg_exchange switches to the fully
-        # distributed form, accbpg_burg_simplex_prox_peer: per-rank work O(n / world), but one NVLink exchange per Newton
-        # step - measured slower on 2 and 8 B200: 85 / 130 us against 74 / 94 us per prox at 50000 columns per GPU.)
-        from . import config
+        # bit-identical on every rank (and independent of the sharding).
         sh = self.shard
         key = (n, sh.width, sh.world)
         if getattr(self, "_gg_key", None) != key:
@@ -214,17 +211,7 @@ class BurgEntropySimplex(BurgEntropy):
             self._gg_peer = peer_buffers(sh, rt.device, [(2 * sh.world * sh.width, torch.float64),
                                                          (sh.world, torch.int64)],
                                          cache_key=("burg_gg", sh.width), reset=False)
-            self._slot_peer = None
-            if config.burg_exchange:
-                self._slot_peer = peer_buffers(sh, rt.device, [(lib.accbpg_burg_simplex_peer_doubles(sh.world), torch.float64)],
-                                               cache_key=("burg_slots", sh.world), reset=False)
         info = rt.slot(rt.S_AUX1)
-        if self._slot_peer is not None:
-            pb = self._slot_peer
-            nat.check(lib.accbpg_burg_simplex_prox_peer(rt.ctx, rt.stream, n, sh.width, yp, gd.data_ptr(), L,
-                                                        float(self.eps), sh.rank, sh.world, pb.tables[0], pb.next_epoch(),
-                                                        out.data_ptr(), info))
-            return
         gg = self._gg_loc
         if self._gg_peer is not None:
             pb = self._gg_peer

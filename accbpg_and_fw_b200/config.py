@@ -22,12 +22,6 @@ peer_allreduce
     (accbpg_dopt_gram_allreduce), and D_opt_FW(_away) exchanges its selection records and the chosen column
     (accbpg_fw_run_peer).  Falls back to NCCL when symmetric memory cannot be set up.
 
-burg_exchange
-    Column-sharded Burg-simplex prox as ONE kernel per rank that exchanges the two partial sums of every bisection /
-    Newton step with all ranks (accbpg_burg_simplex_prox_peer) instead of gathering gg once and replaying the recurrence
-    on the gathered vector on every rank.  Off by default: an NVLink exchange per Newton step costs more than the
-    replicated arithmetic at the shapes measured (85 / 130 us against 74 / 94 us per prox on 2 / 8 B200).
-
 fused_small
     BPG on a D-optimal design objective with the Burg kernel on the simplex whose H fits in the shared memory of one SM
     (configs[0], 80 x 200, does): the whole solve is ONE kernel launch (accbpg_dopt_bpg_small) instead of a dozen launches
@@ -38,5 +32,4 @@ linear_images = True
 reanchor_every = 64
 pipeline = True
 peer_allreduce = __import__('os').environ.get('ACCBPG_PEER_ALLREDUCE', '1') != '0'
-burg_exchange = __import__('os').environ.get('ACCBPG_BURG_EXCHANGE', '0') == '1'
 fused_small = __import__('os').environ.get('ACCBPG_FUSED_SMALL', '1') != '0'

@@ -26,9 +26,8 @@ struct Ctx {
     unsigned int* d_counter;// "last block done" ticket
     double* h_slots;        // pinned mirror (kSlots doubles)
     uint32_t* h_status;     // pinned
-    int coop_blocks_burg;   // co-resident grid size for the Burg-simplex kernel
-    unsigned long long burg_calls;   // token base of the exchange-form root-find (one per call)
-    double* d_burg_slots;   // its slot table on one GPU (2 x 296 slots of 4 doubles)
+    unsigned long long burg_calls;   // Burg-simplex root-finds launched: token base of the next one (one per call)
+    double* d_burg_slots;   // their slot table (2 x 296 block-partial slots + 2 result slots, 4 doubles each)
     cudaStream_t side;      // side stream: a second latency-bound chain (Cholesky) runs next to the main one
     cudaEvent_t ev_fork, ev_join;
     cudaStream_t side2;     // early launches of the triangular GEMM, next to the tail of the Cholesky chain

@@ -161,18 +161,6 @@ struct BurgProxF {
         out[i] = r;
     }
 };
-struct BurgSimplexSumsF {
-    const double* gg; double c;
-    __device__ void operator()(int64_t i, double* acc, uint32_t&) const {
-        double t = gg[i] + c;
-        acc[0] += 1.0 / t;
-        acc[1] += -1.0 / (t * t);
-    }
-};
-struct BurgSimplexFinishF {
-    const double* gg; double c; double* out;
-    __device__ void operator()(int64_t i, uint32_t&) const { out[i] = 1.0 / (gg[i] + c); }
-};
 struct BurgSimplexFinishDevF {
     const double* gg; const double* c; double* out;
     __device__ void operator()(int64_t i, uint32_t&) const { out[i] = 1.0 / (gg[i] + ld_cg(c)); }
@@ -344,27 +332,21 @@ __global__ void __launch_bounds__(kThreads) argext_kernel(int64_t n, const doubl
     }
 }
 
-constexpr int kBurgThreads = 512;
-
-// ---------------------------------------------------------------- Burg-simplex root-find, exchange form
-// The same recurrence (functions.py:341-356) with the iterate held in REGISTERS and the grid-wide reductions done by a
-// two-level exchange of partial sums through a slot table instead of grid.sync + a second pass over L2 (burgx_round):
-// blocks -> their rank's leader block -> all leaders (NVLink peer memory when the vector is column-sharded) -> one result
-// word per rank.  Sums are added in block order, then in rank order, so the multiplier c and the step counts are
-// bit-identical on every rank, per-rank work is O(n / world), and a Newton step costs three store -> poll hops (two on one
-// GPU) instead of a grid barrier plus an L2 round trip.
+// ---------------------------------------------------------------- Burg-simplex root-find
+// The recurrence of functions.py:341-356 in one persistent kernel with the iterate held in REGISTERS; the grid-wide sums
+// of a step go through a slot table (burgx_round) instead of grid.sync + a second pass over L2.  Sums are added in block
+// order, so the multiplier c and the step counts do not depend on which block finishes first, and a Newton step costs one
+// store -> poll hop (two above 128 blocks) instead of a grid barrier plus an L2 round trip.
 // Launched as an ordinary kernel with at most as many blocks as are co-resident on an idle GPU: blocks that are not
 // resident yet are waited for by the others (nothing they wait for depends on this kernel), cooperative launches of
 // different streams would serialise against each other.
-constexpr int kMaxPeerRanks = 16;
-constexpr int kPeerScalars = 16;
+constexpr int kBurgThreads = 512;
 constexpr int kBurgSlot = 4;                           // doubles per slot: a, token, b, token
-constexpr int kBurgMaxG = kMaxBlocks / 4;              // 296 blocks per rank at most
+constexpr int kBurgMaxG = kMaxBlocks / 4;              // 296 blocks at most
 struct BurgX {
-    double* tab[kMaxPeerRanks];                        // every rank's table (layout at burgx_round)
-    int rank, world;
-    int onehop;                                        // world == 1: every block gathers the block partials itself
-    unsigned long long base;                           // token of round r is base + r (unique per call on these tables)
+    double* tab;                                       // the slot table (layout at burgx_round)
+    int onehop;                                        // every block gathers the block partials itself
+    unsigned long long base;                           // token of round r is base + r (unique per call on this table)
 };
 
 // a value and its round token travel together in one aligned 16-byte word (single transaction: the reader sees both or
@@ -375,19 +357,9 @@ __device__ __forceinline__ void st_pair(double* p, double v, unsigned long long 
 __device__ __forceinline__ void ld_pair(const double* p, unsigned long long& v, unsigned long long& tok) {
     asm volatile("ld.volatile.global.v2.u64 {%0, %1}, [%2];" : "=l"(v), "=l"(tok) : "l"(p) : "memory");
 }
-__device__ __forceinline__ void st_release_scope(unsigned long long* p, unsigned long long v, bool sys) {
-    if (sys) asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-    else asm volatile("st.release.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ unsigned long long ld_acquire_scope(const unsigned long long* p, bool sys) {
-    unsigned long long v;
-    if (sys) asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    else asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
 
 // wait until the 16-byte word at p carries `token`; returns its value
-__device__ __forceinline__ double wait_pair(const double* p, unsigned long long token, bool sys) {
+__device__ __forceinline__ double wait_pair(const double* p, unsigned long long token) {
     unsigned long long v, tk, t0 = 0;
     unsigned spin = 0;
     for (;;) {
@@ -398,7 +370,7 @@ __device__ __forceinline__ double wait_pair(const double* p, unsigned long long 
             unsigned long long now;
             asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
             if (t0 == 0) t0 = now;
-            else if (now - t0 > (sys ? 120000000000ULL : 4000000000ULL)) __trap();
+            else if (now - t0 > 4000000000ULL) __trap();
         }
     }
 }
@@ -406,7 +378,7 @@ __device__ __forceinline__ double wait_pair(const double* p, unsigned long long 
 // gather `count` slots (a, b pairs) starting at `slots` in increasing index: the 32 lanes of one warp take slots
 // lane, lane + 32, ... (four in flight each), add them up in that order, then a fixed shuffle tree
 template <bool IS_MIN>
-__device__ __forceinline__ void gather_slots(const double* slots, int count, unsigned long long token, bool sys, double& ra,
+__device__ __forceinline__ void gather_slots(const double* slots, int count, unsigned long long token, double& ra,
                                              double& rb) {
     const int lane = threadIdx.x & 31;
     double sa = IS_MIN ? kInf : 0.0, sb = 0.0;
@@ -437,7 +409,7 @@ __device__ __forceinline__ void gather_slots(const double* slots, int count, uns
                 unsigned long long now;
                 asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
                 if (t0 == 0) t0 = now;
-                else if (now - t0 > (sys ? 120000000000ULL : 4000000000ULL)) __trap();
+                else if (now - t0 > 4000000000ULL) __trap();
             }
         }
 #pragma unroll
@@ -451,21 +423,20 @@ __device__ __forceinline__ void gather_slots(const double* slots, int count, uns
     else { ra = warp_sum(sa); rb = warp_sum(sb); }
 }
 
-// One exchange round; (a, b) are this thread's partial sums (IS_MIN: a is a partial minimum, b unused).  Two levels, so
-// that no cache line is polled by more than one block except the single result word:
-//   every block delivers its partials to its rank's leader (block 0), which adds them in block order;
-//   the leader delivers the rank's sums into every rank's table (NVLink when column-sharded);
-//   every block waits for the `world` rank sums in its own rank's table and adds them in rank order.
-// Every store carries its value and the round's token in one 16-byte word: no fences.  Table of a rank (kBurgSlot doubles
-// per slot):  A [2][kBurgMaxG] block partials, then B [2][kMaxPeerRanks] rank sums.
-constexpr int kBurgOffB = 2 * kBurgMaxG;
-constexpr int kBurgOffC = kBurgOffB + 2 * kMaxPeerRanks;
-constexpr int kBurgTableSlots = kBurgOffC + 2;
+// One exchange round; (a, b) are this thread's partial sums (IS_MIN: a is a partial minimum, b unused).  One block adds
+// its warps' sums in shared memory.  Otherwise every block stores its partials into its slot, and then
+//   onehop: every block gathers all block partials itself (G polls per block and round);
+//   leader: block 0 gathers them and stores the total into the result slot, which every other block polls,
+// so that above 128 blocks no cache line is polled by more than one block except the result slot.  Both forms add the
+// block partials in the same order (same lanes, same shuffle tree), so they give the same bits.  Every store carries
+// its value and the round's token in one 16-byte word: no fences.  Table (kBurgSlot doubles per slot): [2][kBurgMaxG]
+// block partials, then [2] result slots, both indexed by the round's parity.
+constexpr int kBurgOffR = 2 * kBurgMaxG;
+constexpr int kBurgTableSlots = kBurgOffR + 2;
 template <bool IS_MIN>
 __device__ __forceinline__ void burgx_round(const BurgX& X, int round, double a, double b, double* sh, int& flip, double& ra,
                                             double& rb) {
     const int G = gridDim.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5, nw = blockDim.x >> 5;
-    const bool sys = X.world > 1;
     double* s = sh + flip * 64;
     flip ^= 1;
     if (IS_MIN) {
@@ -477,7 +448,7 @@ __device__ __forceinline__ void burgx_round(const BurgX& X, int round, double a,
         if (lane == 0) { s[wid] = a; s[32 + wid] = b; }
     }
     __syncthreads();
-    if (G == 1 && X.world == 1) {                      // one block holds the whole vector (n <= 4096): no exchange at all
+    if (G == 1) {                                      // one block holds the whole vector (n <= 4096): no exchange at all
         if (IS_MIN) { ra = warp_min((lane < nw) ? s[lane] : kInf); rb = 0.0; }
         else { ra = warp_sum((lane < nw) ? s[lane] : 0.0); rb = warp_sum((lane < nw) ? s[32 + lane] : 0.0); }
         return;                                        // (the buffers alternate, so the next round needs no second barrier)
@@ -488,40 +459,22 @@ __device__ __forceinline__ void burgx_round(const BurgX& X, int round, double a,
         else { ba = warp_sum((lane < nw) ? s[lane] : 0.0); bb = warp_sum((lane < nw) ? s[32 + lane] : 0.0); }
         const unsigned long long token = X.base + (unsigned long long)round;
         const int par = round & 1;
-        double* tab = X.tab[X.rank];
+        const double* parts = X.tab + (size_t)par * kBurgMaxG * kBurgSlot;
+        double* res = X.tab + ((size_t)kBurgOffR + par) * kBurgSlot;
         if (lane == 0) {
-            double* dst = tab + ((size_t)par * kBurgMaxG + blockIdx.x) * kBurgSlot;
+            double* dst = X.tab + ((size_t)par * kBurgMaxG + blockIdx.x) * kBurgSlot;
             st_pair(dst, ba, token);
             st_pair(dst + 2, bb, token);
         }
         double ta, tb;
-        if (X.world == 1 && X.onehop) {
-            // one rank: every block gathers all block partials itself, in the order the leader would (same lanes, same
-            // shuffle tree, and 0 + t = t in the rank sum: same bits), so a round costs one store -> poll hop, not two
-            gather_slots<IS_MIN>(tab + (size_t)par * kBurgMaxG * kBurgSlot, G, token, false, ta, tb);
-        } else {
-            if (blockIdx.x == 0) {                     // the leader adds its rank's block partials and tells every rank
-                gather_slots<IS_MIN>(tab + (size_t)par * kBurgMaxG * kBurgSlot, G, token, false, ta, tb);
-                if (lane < X.world) {
-                    double* dst = X.tab[lane] + ((size_t)kBurgOffB + par * kMaxPeerRanks + X.rank) * kBurgSlot;
-                    st_pair(dst, ta, token);
-                    st_pair(dst + 2, tb, token);
-                }
-            }
-            // every block (the leader included) waits for the `world` rank sums in its own table, adds them in rank order
-            double va = 0.0, vb = 0.0;
-            if (lane < X.world) {
-                const double* src = tab + ((size_t)kBurgOffB + par * kMaxPeerRanks + lane) * kBurgSlot;
-                va = wait_pair(src, token, sys);
-                vb = wait_pair(src + 2, token, sys);
-            }
-            ta = IS_MIN ? kInf : 0.0;
-            tb = 0.0;
-            for (int r = 0; r < X.world; ++r) {
-                const double ar = __shfl_sync(0xffffffffu, va, r), br = __shfl_sync(0xffffffffu, vb, r);
-                if (IS_MIN) ta = fmin(ta, ar);
-                else { ta += ar; tb += br; }
-            }
+        if (X.onehop) {
+            gather_slots<IS_MIN>(parts, G, token, ta, tb);
+        } else if (blockIdx.x == 0) {                  // the leader adds the block partials and posts the total
+            gather_slots<IS_MIN>(parts, G, token, ta, tb);
+            if (lane == 0) { st_pair(res, ta, token); st_pair(res + 2, tb, token); }
+        } else if (lane == 0) {                        // only lane 0's total is used below
+            ta = wait_pair(res, token);
+            tb = wait_pair(res + 2, token);
         }
         double* o = sh + flip * 64;                    // the other buffer: nobody reads it before the barrier below
         if (lane == 0) { o[0] = ta; o[1] = tb; }
@@ -651,6 +604,8 @@ __global__ void __launch_bounds__(kThreads) burg_prepare_kernel(int64_t n, const
 }
 
 // ---- exchanges over NVLink peer memory (column-sharded runs; buffers mapped into every rank) ----
+constexpr int kMaxPeerRanks = 16;
+constexpr int kPeerScalars = 16;
 struct PeerVec {
     double* buf[kMaxPeerRanks];                    // every rank's receive buffer, double-buffered on the epoch's parity
     unsigned long long* flags[kMaxPeerRanks];      // every rank's flag words, one per sender
@@ -818,7 +773,6 @@ int accbpg_ctx_create(void** out) {
     ACCBPG_CUDA(cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming));
     ACCBPG_CUDA(cudaStreamCreateWithFlags(&c->side2, cudaStreamNonBlocking));
     ACCBPG_CUDA(cudaEventCreateWithFlags(&c->ev_early_done, cudaEventDisableTiming));
-    c->coop_blocks_burg = 0;
     c->burg_calls = 0;
     ACCBPG_CUDA(cudaDeviceSynchronize());
     *out = c;
@@ -988,14 +942,10 @@ int accbpg_burg_prox(void* ctx, void* stream, int64_t n, int kind, double lamda,
     double lamL = lamda / L;
     return launch_map(c, s, n, BurgProxF{kind, lamda, L, 4 * lamL, 2 * lamL, y, g, out}, "burg_prox");
 }
-static int burgx_launch(Ctx* c, cudaStream_t s, int64_t n, int64_t width, const double* y, const double* g, double L, double eps,
-                        double* out, double* info, const BurgX& X0, const double* gg_in = nullptr) {
-    BurgX X = X0;
-    static int onehop = -1;                            // ACCBPG_BURG_ONEHOP=0: the two-level exchange on one rank too
-    if (onehop < 0) { const char* e = getenv("ACCBPG_BURG_ONEHOP"); onehop = (e && e[0] == '0') ? 0 : 1; }
-    // the grid depends on `width` only (the widest slice), so every rank uses the same slot layout
-    int64_t want = (width + kBurgThreads - 1) / kBurgThreads;
-    static int per_sm_x = 0;                           // co-resident blocks per SM of the exchange-form kernel (all variants)
+static int burgx_launch(Ctx* c, cudaStream_t s, int64_t n, const double* y, const double* g, double L, double eps,
+                        double* out, double* info, const double* gg_in = nullptr) {
+    int64_t want = (n + kBurgThreads - 1) / kBurgThreads;
+    static int per_sm_x = 0;                           // co-resident blocks per SM of burg_simplex_x_kernel (all variants)
     if (per_sm_x == 0) {
         int a = 0, b = 0;
         ACCBPG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a, burg_simplex_x_kernel<8>, kBurgThreads, 0));
@@ -1008,10 +958,13 @@ static int burgx_launch(Ctx* c, cudaStream_t s, int64_t n, int64_t width, const 
     if (cap > kBurgMaxG) cap = kBurgMaxG;
     int grid = (int)(want < cap ? want : cap);
     if (grid < 1) grid = 1;
-    if (width <= 8 * kBurgThreads && X.world == 1) grid = 1;      // small vectors: one block, no exchange (shared memory only)
-    const int64_t per = (width + (int64_t)grid * kBurgThreads - 1) / ((int64_t)grid * kBurgThreads);
+    if (n <= 8 * kBurgThreads) grid = 1;               // small vectors: one block, no exchange (shared memory only)
+    const int64_t per = (n + (int64_t)grid * kBurgThreads - 1) / ((int64_t)grid * kBurgThreads);
+    BurgX X;
+    X.tab = c->d_burg_slots;
+    X.base = (++c->burg_calls) << 12;                  // at most 2201 rounds per call
     // one hop costs G polls per block and round (G^2 in all): measured 2 us faster per call at 98 blocks, slower at 196
-    X.onehop = onehop && grid <= 128;
+    X.onehop = grid <= 128;
     ProfScope ps(P_BURG_SIMPLEX, s);
     if (per <= 1) burg_simplex_x_kernel<1><<<grid, kBurgThreads, 0, s>>>(n, y, g, L, eps, out, info, c->d_status, X, gg_in);
     else if (per <= 2) burg_simplex_x_kernel<2><<<grid, kBurgThreads, 0, s>>>(n, y, g, L, eps, out, info, c->d_status, X, gg_in);
@@ -1029,51 +982,18 @@ int accbpg_burg_simplex_prox(void* ctx, void* stream, int64_t n, const double* y
     CTX_STREAM
     if (!(L > 0.0)) return arg_err("L must be positive");
     if (n < 1) return arg_err("n must be >= 1");
-    BurgX X;
-    X.tab[0] = c->d_burg_slots;
-    X.rank = 0; X.world = 1;
-    X.base = (++c->burg_calls) << 12;                  // at most 2201 rounds per call
-    return burgx_launch(c, s, n, n, y, g, L, eps, out, info, X);
-}
-
-size_t accbpg_burg_simplex_peer_doubles(int world) {
-    return world < 1 ? 0 : (size_t)kBurgTableSlots * kBurgSlot;
-}
-
-int accbpg_burg_simplex_prox_peer(void* ctx, void* stream, int64_t n_local, int64_t width, const double* y, const double* g,
-                                  double L, double eps, int rank, int world, void* const* peer_slots, uint64_t epoch,
-                                  double* out, double* info) {
-    Ctx* c = (Ctx*)ctx;
-    cudaStream_t s = (cudaStream_t)stream;
-    if (!c) return arg_err("ctx is NULL");
-    ACCBPG_ON_DEVICE(c);
-    if (!g || !out || !peer_slots) return arg_err("burg_simplex_prox_peer: NULL pointer");
-    if (!(L > 0.0)) return arg_err("L must be positive");
-    if (n_local < 0 || width < n_local || width < 1) return arg_err("burg_simplex_prox_peer: width");
-    if (world < 1 || world > kMaxPeerRanks || rank < 0 || rank >= world || epoch < 1) return arg_err("burg_simplex_prox_peer: rank / world / epoch");
-    BurgX X;
-    for (int r = 0; r < world; ++r) {
-        X.tab[r] = (double*)peer_slots[r];
-        if (!X.tab[r]) return arg_err("burg_simplex_prox_peer: NULL peer pointer");
-    }
-    X.rank = rank; X.world = world;
-    X.base = (unsigned long long)epoch << 12;
-    return burgx_launch(c, s, n_local, width, y, g, L, eps, out, info, X);
+    return burgx_launch(c, s, n, y, g, L, eps, out, info);
 }
 int accbpg_burg_simplex_root(void* ctx, void* stream, int64_t n, const double* gg, double eps, double* d_info) {
     CTX_STREAM
     if (!gg || !d_info) return arg_err("burg_simplex_root: NULL pointer");
     if (n < 1) return arg_err("n must be >= 1");
-    BurgX X;
-    X.tab[0] = c->d_burg_slots;
-    X.rank = 0; X.world = 1;
-    X.base = (++c->burg_calls) << 12;
-    return burgx_launch(c, s, n, n, nullptr, nullptr, 1.0, eps, nullptr, d_info, X, gg);
+    return burgx_launch(c, s, n, nullptr, nullptr, 1.0, eps, nullptr, d_info, gg);
 }
 
 // Column-sharded prox over NVLink peer memory, in two calls.  push: the prepare kernel stores this rank's (padded) slice
 // of gg straight into every rank's gathered vector and releases a flag word there.  root: a one-warp kernel waits for
-// the `world` flags (so the cooperative root-find never spins on a peer while it holds the whole GPU), then the
+// the `world` flags (so the root-find's blocks never spin on a peer while they occupy the GPU), then the
 // root-find runs on the gathered vector.
 static int peer_vec_fill(PeerVec& pv, int rank, int world, void* const* bufs, void* const* flags, uint64_t epoch,
                          const char* what) {
@@ -1123,11 +1043,7 @@ int accbpg_burg_simplex_root_peer(void* ctx, void* stream, int64_t width, double
     }
     const int64_t n = width * world;
     const double* gg = pv.buf[rank] + (size_t)(epoch & 1ULL) * (size_t)n;
-    BurgX X;
-    X.tab[0] = c->d_burg_slots;
-    X.rank = 0; X.world = 1;
-    X.base = (++c->burg_calls) << 12;
-    return burgx_launch(c, s, n, n, nullptr, nullptr, 1.0, eps, nullptr, d_info, X, gg);
+    return burgx_launch(c, s, n, nullptr, nullptr, 1.0, eps, nullptr, d_info, gg);
 }
 
 // Sum `count` (<= 15) per-rank partial scalars over the ranks through peer memory, in rank order: one CTA stores its
@@ -1222,15 +1138,6 @@ int accbpg_burg_simplex_prepare(void* ctx, void* stream, int64_t n, const double
     burg_prepare_kernel<<<grid, kThreads, 0, s>>>(n, y, g, L, gg, c->d_partials, c->d_counter, d_out, c->d_status);
     ACCBPG_LAUNCHED("burg_simplex_prepare");
     return ACCBPG_OK;
-}
-int accbpg_burg_simplex_sums(void* ctx, void* stream, int64_t n, const double* gg, double cc, double* d_out) {
-    CTX_STREAM
-    return launch_reduce<2>(c, s, n, BurgSimplexSumsF{gg, cc}, d_out, "burg_simplex_sums");
-}
-int accbpg_burg_simplex_finish(void* ctx, void* stream, int64_t n, const double* gg, double cc, double* out) {
-    CTX_STREAM
-    if (n == 0) return ACCBPG_OK;
-    return launch_map(c, s, n, BurgSimplexFinishF{gg, cc, out}, "burg_simplex_finish");
 }
 
 // ---- Shannon

@@ -36,7 +36,7 @@
 extern "C" {
 #endif
 
-#define ACCBPG_ABI_VERSION 2
+#define ACCBPG_ABI_VERSION 3
 
 /* return codes */
 #define ACCBPG_OK      0
@@ -123,24 +123,20 @@ int accbpg_burg_divergence(void* ctx, void* stream, int64_t n, const double* d_x
 int accbpg_burg_prox(void* ctx, void* stream, int64_t n, int kind, double lamda,
                      const double* d_y, const double* d_g, double L, double* d_out_vec);
 /* BurgEntropySimplex.prox_map / inherited div_prox_map (functions.py:336-356): one persistent kernel replays cmin,
- * bisection and Newton with the iterate in registers; the grid-wide sums of a step go through a slot table (block
- * partials to a leader block, total back in one word; value + round token per 16-byte store, fixed-order adds): no host
- * round trip and no grid barrier per Newton step.
+ * bisection and Newton with the iterate in registers; the grid-wide sums of a step go through a slot table (every block
+ * gathers the block partials itself, or above 128 blocks a leader block adds them and posts the total in one slot;
+ * value + round token per 16-byte store, block-order adds): no host round trip and no grid barrier per Newton step.
  * d_info (3 slots, may be NULL): bisection steps, Newton steps, final c. */
 int accbpg_burg_simplex_prox(void* ctx, void* stream, int64_t n, const double* d_y, const double* d_g,
                              double L, double eps, double* d_out_vec, double* d_info);
-/* column-sharded building blocks of the same root-find (one rank's slice; the caller
- * all-reduces the scalars):  prepare: out = gg = (g [+ L/y]) / L, d_out[0] = min(gg);
- * sums: d_out[0] = sum 1/(gg+c), d_out[1] = sum -1/(gg+c)^2;  finish: out = 1/(gg+c). */
+/* column-sharded building block of the same root-find, on one rank's slice:
+ * d_gg = (g [+ L/y]) / L, d_out[0] = min(gg). */
 int accbpg_burg_simplex_prepare(void* ctx, void* stream, int64_t n, const double* d_y, const double* d_g,
                                 double L, double* d_gg, double* d_out);
-int accbpg_burg_simplex_sums(void* ctx, void* stream, int64_t n, const double* d_gg, double c, double* d_out);
-int accbpg_burg_simplex_finish(void* ctx, void* stream, int64_t n, const double* d_gg, double c,
-                               double* d_out_vec);
 /* the same root-find without a host round trip: every rank all-gathers the slices of gg (padding entries +inf),
- * runs the whole recurrence of functions.py:341-356 on the gathered vector in one cooperative kernel -- the result
- * does not depend on how the columns are sharded -- and finishes its own slice with the c left on the device.
- * d_info (3 slots): bisection steps, Newton steps, c. */
+ * runs the whole recurrence of functions.py:341-356 on the gathered vector with the kernel of accbpg_burg_simplex_prox
+ * -- the result does not depend on how the columns are sharded -- and finishes its own slice, out = 1/(gg + c), with
+ * the c left on the device.  d_info (3 slots): bisection steps, Newton steps, c. */
 int accbpg_burg_simplex_root(void* ctx, void* stream, int64_t n, const double* d_gg, double eps, double* d_info);
 int accbpg_burg_simplex_finish_dev(void* ctx, void* stream, int64_t n, const double* d_gg, const double* d_c,
                                    double* d_out_vec);
@@ -157,16 +153,6 @@ int accbpg_burg_simplex_push_peer(void* ctx, void* stream, int64_t n_local, int6
                                   void* const* peer_flags, uint64_t epoch, double* d_gg_local);
 int accbpg_burg_simplex_root_peer(void* ctx, void* stream, int64_t width, double eps, int rank, int world,
                                   void* const* peer_gg, void* const* peer_flags, uint64_t epoch, double* d_info);
-/* The column-sharded prox as ONE kernel per rank (functions.py:336-356 with the vector split over the ranks): the blocks
- * of a rank deliver their partial (sum 1/(gg+c), sum -1/(gg+c)^2) of a step to the rank's leader block, the leaders
- * exchange the rank sums over NVLink (one 16-byte store per value and peer, value and round token in one word) and add
- * them in rank order: the multiplier and the step counts are bit-identical on every rank, per-rank work is O(n_local).  `width` = the widest slice (the same on every
- * rank: it fixes the grid).  peer_slots: host array of `world` device pointers to every rank's symmetric table of
- * accbpg_burg_simplex_peer_doubles(world) doubles, zeroed once; epoch 1, 2, 3, ... per call, the same on every rank. */
-size_t accbpg_burg_simplex_peer_doubles(int world);
-int accbpg_burg_simplex_prox_peer(void* ctx, void* stream, int64_t n_local, int64_t width, const double* d_y,
-                                  const double* d_g, double L, double eps, int rank, int world, void* const* peer_slots,
-                                  uint64_t epoch, double* d_out_vec, double* d_info);
 /* Sum `count` (<= 15) per-rank partial scalars at d_in over the ranks through peer memory, in rank order, into d_out
  * (may equal d_in) (the batched divergence / dot-product partials of a driver iteration, algorithms.py:53,153-154,...):
  * one small kernel instead of an NCCL all-reduce.  The exchange also carries every rank's status word and ORs them into

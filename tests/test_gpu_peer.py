@@ -233,63 +233,6 @@ def test_burg_simplex_prox_gather_over_peer_buffers_emulated_ranks(acc, world, n
             rk.close()
 
 
-@pytest.mark.parametrize("world,n", [(2, 1000), (3, 1499), (8, 4001), (2, 40000), (2, 70000)])
-def test_burg_simplex_prox_exchange_form_emulated_ranks(acc, world, n):
-    """accbpg_burg_simplex_prox_peer: ONE kernel per rank, the iterate in registers, the two sums of every bisection /
-    Newton step exchanged through the slot tables: multiplier and step counts bit-identical on every rank, the assembled
-    prox equal to the oracle's on the whole vector and to the one-GPU kernel's step counts.  (All emulated ranks' blocks
-    must be resident on the one GPU at once, which bounds n here; on separate GPUs each rank has its own.)"""
-    from accbpg_and_fw_b200 import _native as nat
-    from accbpg_and_fw_b200.runtime import Runtime
-    from oracle import accbpg_oracle as orc
-    lib = nat.lib
-    dev = torch.device("cuda")
-    rng = np.random.RandomState(5 + world)
-    sh = acc.ColumnShard(n, rank=0, world=world)
-    width, off = sh.width, sh.offsets
-    ho = orc.make_burg("simplex")
-    rt = Runtime.get()
-    ranks = [_Rank(nat) for _ in range(world)]
-    try:
-        slots = [torch.zeros(lib.accbpg_burg_simplex_peer_doubles(world), dtype=F64, device=dev) for _ in range(world)]
-        t_slots = _table(slots)
-        for epoch in range(1, 5):
-            y = rng.rand(n) + 0.05
-            y /= y.sum()
-            g = rng.randn(n)
-            L = 0.5 + epoch
-            use_y = epoch != 2                                        # prox_map (no y) on one of the calls
-            yd = [torch.tensor(y[off[r]:off[r + 1]], device=dev) for r in range(world)]
-            gd = [torch.tensor(g[off[r]:off[r + 1]], device=dev) for r in range(world)]
-            info = [torch.zeros(8, dtype=F64, device=dev) for _ in range(world)]
-            out = [torch.empty(off[r + 1] - off[r], dtype=F64, device=dev) for r in range(world)]
-            torch.cuda.synchronize()
-            for r in range(world):
-                nl = off[r + 1] - off[r]
-                nat.check(lib.accbpg_burg_simplex_prox_peer(ranks[r].ctx, ranks[r].stream.cuda_stream, nl, width,
-                                                            yd[r].data_ptr() if use_y else None, gd[r].data_ptr(), L, 1e-8,
-                                                            r, world, t_slots, epoch, out[r].data_ptr(), info[r].data_ptr()))
-            torch.cuda.synchronize()
-            infos = [tuple(i[:3].tolist()) for i in info]
-            assert len(set(infos)) == 1, infos                        # same bisections, Newton steps and c everywhere
-            x = np.concatenate([o.cpu().numpy() for o in out])
-            xo = ho.div_prox_map(y, g, L) if use_y else ho.prox_map(g, L)
-            assert float(np.max(np.abs(x - xo) / np.abs(xo))) <= 1e-10
-            assert abs(x.sum() - 1.0) <= 2e-8
-            # the one-GPU kernel on the whole vector takes the same number of steps
-            full_out = torch.empty(n, dtype=F64, device=dev)
-            y_all, g_all = torch.tensor(y, device=dev), torch.tensor(g, device=dev)
-            nat.check(lib.accbpg_burg_simplex_prox(rt.ctx, rt.stream, n, y_all.data_ptr() if use_y else None,
-                                                   g_all.data_ptr(), L, 1e-8, full_out.data_ptr(), rt.slot(44)))
-            one = rt.read(44, 3)
-            assert (one[0], one[1]) == (infos[0][0], infos[0][1]), (one, infos[0])
-            assert abs(one[2] - infos[0][2]) <= 1e-9 * max(1.0, abs(one[2])), (one[2], infos[0][2])
-    finally:
-        torch.cuda.synchronize()
-        for rk in ranks:
-            rk.close()
-
-
 @pytest.mark.parametrize("world,n", [(2, 17), (4, 1000), (8, 100000)])
 def test_vector_sum_over_peer_buffers_emulated_ranks(acc, world, n):
     from accbpg_and_fw_b200 import _native as nat
