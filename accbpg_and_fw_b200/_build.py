@@ -22,6 +22,7 @@ COMMON = ["-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC", "-Xcompiler",
 SOURCES = {
     "vecops.cu": ["-fmad=false"],
     "linreg.cu": ["-fmad=false"],
+    "linreg_small.cu": ["-fmad=false"],
     "fw.cu": ["-fmad=false"],
     "dopt.cu": [],
     "chol.cu": [],

@@ -27,6 +27,10 @@ fused_small
     (configs[0], 80 x 200, does): the whole solve is ONE kernel launch (accbpg_dopt_bpg_small) instead of a dozen launches
     and a host decision per line-search trip.  Same control flow and histories; T is stamped evenly over the solve's
     wall time (the host does not see individual iterations).
+    The same holds for BPG on PoissonRegression / KLdivRegression with BurgEntropy, BurgEntropyL1, BurgEntropyL2,
+    ShannonEntropy, ShannonEntropyL1 or ShannonEntropySimplex when A fits the shared memory of a cluster of at most 8 SMs
+    (accbpg_linreg_bpg_small; the notebook instances, Poisson 200 x 100 and KL 1000 x 100, do).  There T[k] is the
+    device clock at the top of iteration k.
 """
 linear_images = True
 reanchor_every = 64

@@ -190,22 +190,21 @@ class _Loop:
         return like_input(x, self.host)
 
 
-def _bpg_small(f, h, L, x0, maxitrs, epsilon, linesearch, ls_ratio, verbose, verbskip):
-    """config.fused_small: the whole BPG solve as one launch of accbpg_dopt_bpg_small when the instance is a dense,
-    unsharded D-optimal design with the Burg kernel on the simplex and fits one SM's shared memory.  Returns None when
-    the fast path does not apply."""
-    from .objectives import DOptimalObj
-    from .bregman import BurgEntropySimplex
-    if not config.fused_small or type(f) is not DOptimalObj or type(h) is not BurgEntropySimplex:
-        return None
-    if f.shard is not None or h.shard is not None or maxitrs < 1 or not (L > 0) or not (ls_ratio > 1):
-        return None
+def _small_hkind(h):
+    """ACCBPG_SMALL_H_* of the Legendre kernel h, or None when the linear-inverse fused solve does not cover its type."""
+    from . import bregman as br
+    names = {br.BurgEntropy: "BURG", br.BurgEntropyL1: "BURG_L1", br.BurgEntropyL2: "BURG_L2",
+             br.ShannonEntropy: "SHANNON", br.ShannonEntropyL1: "SHANNON_L1",
+             br.ShannonEntropySimplex: "SHANNON_SIMPLEX"}
+    name = names.get(type(h))
+    return None if name is None else nat.MACROS["ACCBPG_SMALL_H_" + name]
+
+
+def _dopt_bpg_small(f, h, L, x, maxitrs, epsilon, linesearch, ls_ratio, t0):
+    """accbpg_dopt_bpg_small: F, Ls, and T stamped evenly over the solve's wall time; None when H does not fit."""
     if lib.accbpg_dopt_bpg_small_smem_bytes(f.m, f.n) == 0:
         return None
     rt = f.rt
-    t0 = time.time()
-    host = is_host(x0)
-    x = rt.to_device(x0).clone()
     hist = torch.empty(2 * maxitrs + 16, dtype=torch.float64, device=rt.device)
     H = f._Hd
     with rt.on_device():
@@ -220,8 +219,61 @@ def _bpg_small(f, h, L, x0, maxitrs, epsilon, linesearch, ls_ratio, verbose, ver
     F = hh[0:k].copy()
     Ls = hh[maxitrs:maxitrs + k].copy() if linesearch else np.ones(k) * L
     T = np.linspace(0.0, time.time() - t0, k + 1)[1:]
+    return F, Ls, T
+
+
+def _linreg_bpg_small(f, h, L, x, maxitrs, epsilon, linesearch, ls_ratio, t0):
+    """accbpg_linreg_bpg_small: F, Ls, and T from the device clock at the top of each iteration, offset by the host time
+    at which the solve was launched; None when A does not fit."""
+    if lib.accbpg_linreg_bpg_small_smem_bytes(f.m, f.n) == 0:
+        return None
+    rt = f.rt
+    hist = torch.empty(3 * maxitrs + 16, dtype=torch.float64, device=rt.device)
+    A = f._Ad
+    base = hist.data_ptr()
+    with rt.on_device():
+        t_launch = time.time() - t0
+        nat.check(lib.accbpg_linreg_bpg_small(rt.ctx, rt.stream, f._kind, A.data_ptr(), f.m, f.n, A.stride(0),
+                                              f._bd.data_ptr(), _small_hkind(h), float(h.lamda),
+                                              float(getattr(h, "delta", 0.0)), x.data_ptr(), float(L), float(ls_ratio),
+                                              1 if linesearch else 0, int(maxitrs), float(epsilon), base,
+                                              base + 8 * maxitrs, base + 16 * maxitrs, base + 24 * maxitrs))
+    rt.read(rt.S_F, 1)                                   # synchronises and raises on a status bit
+    hh = hist.cpu().numpy()
+    k = int(hh[3 * maxitrs])
+    _bpg_small.last_info = hh[3 * maxitrs:3 * maxitrs + 4].copy()
+    F = hh[0:k].copy()
+    Ls = hh[maxitrs:maxitrs + k].copy()
+    T = t_launch + hh[2 * maxitrs:2 * maxitrs + k] * 1e-9
+    return F, Ls, T
+
+
+def _bpg_small(f, h, L, x0, maxitrs, epsilon, linesearch, ls_ratio, verbose, verbskip):
+    """config.fused_small: the whole BPG solve as one kernel launch when the instance is dense, unsharded and fits the
+    shared memory of one SM (or of a small cluster): a D-optimal design with the Burg kernel on the simplex
+    (accbpg_dopt_bpg_small), or Poisson / KL regression with a Burg or Shannon kernel (accbpg_linreg_bpg_small).
+    Returns None when no fused solve applies.  `_bpg_small.last_info` keeps the kernel's info array."""
+    from .objectives import DOptimalObj, PoissonRegression, KLdivRegression
+    from .bregman import BurgEntropySimplex
+    if not config.fused_small or maxitrs < 1 or not (L > 0) or not (ls_ratio > 1):
+        return None
+    if type(f) is DOptimalObj and type(h) is BurgEntropySimplex:
+        solve = _dopt_bpg_small
+    elif type(f) in (PoissonRegression, KLdivRegression) and _small_hkind(h) is not None:
+        solve = _linreg_bpg_small
+    else:
+        return None
+    if f.shard is not None or h.shard is not None:
+        return None
+    t0 = time.time()
+    host = is_host(x0)
+    x = f.rt.to_device(x0).clone()
+    out = solve(f, h, L, x, maxitrs, epsilon, linesearch, ls_ratio, t0)
+    if out is None:
+        return None
+    F, Ls, T = out
     if verbose:
-        for i in range(0, k, max(int(verbskip), 1)):
+        for i in range(0, len(F), max(int(verbskip), 1)):
             print("{0:6d}  {1:10.3e}  {2:10.3e}  {3:6.1f}".format(i, F[i], Ls[i], T[i]))
     return like_input(x, host), F, Ls, T
 

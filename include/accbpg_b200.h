@@ -36,7 +36,7 @@
 extern "C" {
 #endif
 
-#define ACCBPG_ABI_VERSION 3
+#define ACCBPG_ABI_VERSION 4
 
 /* return codes */
 #define ACCBPG_OK      0
@@ -306,6 +306,34 @@ int accbpg_linreg_value_resid(void* ctx, void* stream, int kind, int64_t m, cons
 /* K6: g = A^T r, one pass over A (the reference materialises an m x n broadcast product) */
 int accbpg_linreg_rmatvec(void* ctx, void* stream, const double* d_A, int64_t m, int64_t n_local, int64_t lda,
                           const double* d_r, void* d_ws, double* d_g);
+
+/* ---- small shapes: the WHOLE BPG solve in one launch (accbpg/algorithms.py:11-72) with PoissonRegression /
+ *      KLdivRegression (functions.py:85-158) and a Burg or Shannon kernel (functions.py:238-323, :398-490).  When A and
+ *      the solve's vectors fit in the shared memory of one SM - or of a cluster of 2, 4 or 8 CTAs, each holding a
+ *      contiguous slice of A's columns, the smallest that fits - one persistent launch runs every iteration: gradient
+ *      A^T r(Ax) from the carried A x (:112, :150), div_prox_map (:264-271, :290-298, :316-323, :430-438, :464-466,
+ *      :475-490), A x1 and f(x1), dot(g, x1 - x) and divergence (:250-253, :415-421), the line-search test
+ *      (algorithms.py:53), the stopping test (algorithms.py:66).  The per-CTA partials of A x and of the n-sums are added
+ *      in rank order through distributed shared memory: two solves of one instance are bit-identical.
+ *      d_x: x0 in, last iterate out.  d_F, d_Ls, d_T: maxitrs entries each; d_T[k] = %globaltimer nanoseconds at the top
+ *      of iteration k since the kernel started.  d_info (16 doubles): [0] entries written, [1] line-search trials,
+ *      [2] last L, [3] cluster size.  lamda: the kernel's lambda (0 for BURG, SHANNON, SHANNON_SIMPLEX); delta: the
+ *      Shannon kernels' delta (unused for Burg).  linesearch = 0: L stays fixed (algorithms.py:57-58).
+ *      The reference's assertions arrive in the status word (the operator path's bits) and end the solve at that
+ *      iteration. */
+#define ACCBPG_SMALL_H_BURG             0   /* BurgEntropy             functions.py:238-271 */
+#define ACCBPG_SMALL_H_BURG_L1          1   /* BurgEntropyL1           functions.py:274-298 */
+#define ACCBPG_SMALL_H_BURG_L2          2   /* BurgEntropyL2           functions.py:301-323 */
+#define ACCBPG_SMALL_H_SHANNON          3   /* ShannonEntropy          functions.py:398-438 */
+#define ACCBPG_SMALL_H_SHANNON_L1       4   /* ShannonEntropyL1        functions.py:441-466 */
+#define ACCBPG_SMALL_H_SHANNON_SIMPLEX  5   /* ShannonEntropySimplex   functions.py:469-490 */
+/* 0 when no cluster of <= 8 CTAs holds A (m x n doubles) and the solve's vectors in shared memory */
+size_t accbpg_linreg_bpg_small_smem_bytes(int64_t m, int64_t n);
+/* kind: ACCBPG_LINREG_POISSON / _KL; hkind: ACCBPG_SMALL_H_* */
+int accbpg_linreg_bpg_small(void* ctx, void* stream, int kind, const double* d_A, int64_t m, int64_t n, int64_t lda,
+                            const double* d_b, int hkind, double lamda, double delta, double* d_x, double L,
+                            double ls_ratio, int linesearch, int maxitrs, double epsilon,
+                            double* d_F, double* d_Ls, double* d_T, double* d_info);
 
 /* ---- D_opt_FW / D_opt_FW_away (accbpg/D_opt_alg.py:9-88, :91-185) -------
  * State lives in caller-owned device buffers: x, w (n), Hinv (m x m, ld m), a control block of
