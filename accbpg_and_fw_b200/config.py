@@ -31,6 +31,10 @@ fused_small
     ShannonEntropy, ShannonEntropyL1 or ShannonEntropySimplex when A fits the shared memory of a cluster of at most 8 SMs
     (accbpg_linreg_bpg_small; the notebook instances, Poisson 200 x 100 and KL 1000 x 100, do).  There T[k] is the
     device clock at the top of iteration k.
+    ABPG and ABPG_gain on the same objectives and kernels run as one launch too (accbpg_linreg_abpg_small, a plan of
+    its own that holds more vectors) when linear_images is also on: the kernel follows that scheme - carried A x and
+    A z, A x re-formed every `reanchor_every` iterations - so results differ from the operator loop only in the order
+    of sums.  With linear_images off the operator loop evaluates every point from scratch, as that switch says.
 """
 linear_images = True
 reanchor_every = 64

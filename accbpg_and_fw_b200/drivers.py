@@ -278,6 +278,54 @@ def _bpg_small(f, h, L, x0, maxitrs, epsilon, linesearch, ls_ratio, verbose, ver
     return like_input(x, host), F, Ls, T
 
 
+def _abpg_small(gain, f, h, L, x0, gamma, maxitrs, epsilon, theta_eq, restart, restart_rule, G0=1.0, ls_inc=1.2,
+                ls_dec=1.2, checkdiv=False):
+    """config.fused_small: the whole ABPG / ABPG_gain solve as one kernel launch (accbpg_linreg_abpg_small) on a
+    PoissonRegression / KLdivRegression instance whose A fits the shared memory of a cluster of at most 8 SMs, with a
+    kernel that accbpg_linreg_bpg_small covers.  It reproduces the operator loop's default scheme (carried linear
+    images), so it is taken only with config.linear_images on.  Returns None when no fused solve applies, else
+    (x, hist rows, k, T): the history rows F, G / Gain, Gdiv, theta, D(x,y), D(z,z-) truncated to the k entries written,
+    and T from the device clock at the top of each iteration, offset by the host time of the launch.
+    `_abpg_small.last_info` keeps the kernel's info array."""
+    from .objectives import PoissonRegression, KLdivRegression
+    if not (config.fused_small and config.linear_images) or maxitrs < 1:
+        return None
+    if type(f) not in (PoissonRegression, KLdivRegression) or _small_hkind(h) is None:
+        return None
+    if f.shard is not None or h.shard is not None:
+        return None
+    if not all(np.isfinite(v) and v > 0 for v in (L, gamma, G0, ls_inc, ls_dec)):
+        return None
+    if lib.accbpg_linreg_abpg_small_smem_bytes(f.m, f.n) == 0:
+        return None
+    t0 = time.time()
+    rt = f.rt
+    x = rt.to_device(x0).clone()
+    hist = torch.empty(7 * maxitrs + 16, dtype=torch.float64, device=rt.device)
+    base = hist.data_ptr()
+    A = f._Ad
+    rule = {'f': "F", 'g': "G"}.get(restart_rule, "NONE")
+    drv = "ABPG_GAIN" if gain else "ABPG"
+    with rt.on_device():
+        t_launch = time.time() - t0
+        nat.check(lib.accbpg_linreg_abpg_small(
+            rt.ctx, rt.stream, nat.MACROS["ACCBPG_SMALL_DRV_" + drv], f._kind, A.data_ptr(), f.m, f.n, A.stride(0),
+            f._bd.data_ptr(), _small_hkind(h), float(h.lamda), float(getattr(h, "delta", 0.0)), x.data_ptr(), float(L),
+            float(gamma), int(maxitrs), float(epsilon), 1 if theta_eq else 0, 1 if restart else 0,
+            nat.MACROS["ACCBPG_SMALL_RESTART_" + rule], float(G0), float(ls_inc), float(ls_dec), 1 if checkdiv else 0,
+            max(int(config.reanchor_every), 1), base, base + 8 * 7 * maxitrs))
+    rt.read(rt.S_F, 1)                                   # synchronises and raises on a status bit
+    hh = hist.cpu().numpy()
+    info = hh[7 * maxitrs:7 * maxitrs + 16].copy()
+    _abpg_small.last_info = info
+    if info[3]:
+        raise UnboundLocalError("cannot access local variable 'Gdr' where it is not associated with a value")
+    k = int(info[0])
+    rows = [hh[r * maxitrs:r * maxitrs + k].copy() for r in range(6)]
+    T = t_launch + hh[6 * maxitrs:6 * maxitrs + k] * 1e-9
+    return like_input(x, is_host(x0)), rows, k, T
+
+
 def BPG(f, h, L, x0, maxitrs, epsilon=1e-14, linesearch=True, ls_ratio=1.2,
         verbose=True, verbskip=1):
     """Bregman proximal gradient.   accbpg/algorithms.py:11-72.   Returns (x, F, Ls, T)."""
@@ -380,6 +428,14 @@ def ABPG(f, h, L, x0, gamma, maxitrs, epsilon=1e-14, theta_eq=False,
     if verbose:
         print("\nABPG method for minimize_{x in C} F(x) = f(x) + Psi(x)")
         print("     k      F(x)       theta        TSG       D(x+,y)     D(z+,z)     time")
+    fused = _abpg_small(False, f, h, L, x0, gamma, maxitrs, epsilon, theta_eq, restart, restart_rule)
+    if fused is not None:
+        x, (F, G, _, Th, Dxy, Dzz), k, T = fused
+        if verbose:
+            for i in range(0, k, max(int(verbskip), 1)):
+                print("{0:6d}  {1:10.3e}  {2:10.3e}  {3:10.3e}  {4:10.3e}  {5:10.3e}  {6:6.1f}".format(
+                    i, F[i], Th[i], G[i], Dxy[i], Dzz[i], T[i]))
+        return x, F, G, T
     lp = _Loop(f, h, x0)
     rt = lp.rt
     F = np.zeros(maxitrs)
@@ -543,6 +599,20 @@ def ABPG_gain(f, h, L, x0, gamma, maxitrs, epsilon=1e-14, G0=1,
     if verbose:
         print("\nABPG_gain method for min_{x in C} F(x) = f(x) + Psi(x)")
         print("     k      F(x)       theta         Gk         TSG       D(x+,y)     D(z+,z)      Gavg       time")
+    fused = _abpg_small(True, f, h, L, x0, gamma, maxitrs, epsilon, theta_eq, restart, restart_rule, G0, ls_inc, ls_dec,
+                        checkdiv)
+    if fused is not None:
+        x, (F, Gain, Gdiv, Th, Dxy, Dzz), k, T = fused
+        Gavg = np.zeros(k)
+        sumlogG = gamma * np.log(G0)
+        for i in range(k):
+            sumlogG += np.log(Gain[i])
+            Gavg[i] = np.exp(sumlogG / (gamma + i))
+        if verbose:
+            for i in range(0, k, max(int(verbskip), 1)):
+                print("{0:6d}  {1:10.3e}  {2:10.3e}  {3:10.3e}  {4:10.3e}  {5:10.3e}  {6:10.3e}  {7:10.3e}  {8:6.1f}".format(
+                    i, F[i], Th[i], Gain[i], Gdiv[i], Dxy[i], Dzz[i], Gavg[i], T[i]))
+        return x, F, Gain, Gdiv, Gavg, T
     lp = _Loop(f, h, x0)
     rt = lp.rt
     F = np.zeros(maxitrs)

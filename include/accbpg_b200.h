@@ -36,7 +36,7 @@
 extern "C" {
 #endif
 
-#define ACCBPG_ABI_VERSION 4
+#define ACCBPG_ABI_VERSION 5
 
 /* return codes */
 #define ACCBPG_OK      0
@@ -334,6 +334,40 @@ int accbpg_linreg_bpg_small(void* ctx, void* stream, int kind, const double* d_A
                             const double* d_b, int hkind, double lamda, double delta, double* d_x, double L,
                             double ls_ratio, int linesearch, int maxitrs, double epsilon,
                             double* d_F, double* d_Ls, double* d_T, double* d_info);
+
+/* ---- small shapes: the WHOLE ABPG (accbpg/algorithms.py:94-180) or ABPG_gain (:295-420) solve in one launch, on the
+ *      instances and kernels of accbpg_linreg_bpg_small, in a shared-memory plan of its own (more vectors: a cluster
+ *      may be larger than BPG's for one shape).  It follows the drivers' default evaluation scheme (linear images):
+ *      A x- and A z- are carried, A y and A x are their combinations (:147, :150, :369, :374), A z is one matvec per
+ *      trip, and A x is re-formed from x at the end of every iteration k with (k+1) % reanchor_every == 0.  Per trip:
+ *      f(y) and g = A^T r(A y) (:112, :150), z = div_prox_map(z-, g, theta^(gamma-1) [G] L), x, D(x, y), D(z, z-)
+ *      (:250-253, :415-421), and for ABPG_gain the gain line search (:387) with G /= ls_dec per iteration and
+ *      G *= ls_inc per rejected trip; theta = gamma/(k+gamma), solve_theta (:75-91) when theta_eq, the alpha form
+ *      (:367) otherwise; checkdiv; restart rules 'f' and 'g' (:168, :406; ABPG from k = 1, ABPG_gain from k = 0);
+ *      the stop D(z, z-) < epsilon.  All decisions are taken redundantly in every CTA from
+ *      the same exchanged bits.
+ *      driver: ACCBPG_SMALL_DRV_*; restart_rule: ACCBPG_SMALL_RESTART_* (the reference never restarts on other rules).
+ *      G0, ls_inc, ls_dec and checkdiv are read by ABPG_gain only.
+ *      d_x: x0 in, last iterate out.  d_hist: 7 rows of maxitrs doubles, row r at d_hist + r * maxitrs:
+ *      [0] F, [1] G (ABPG) or Gain (ABPG_gain), [2] Gdiv (ABPG_gain; the previous value when a trip stops on
+ *      D(z, z-) < epsilon), [3] theta, [4] D(x, y), [5] D(z, z-), [6] T (%globaltimer nanoseconds at the top of the
+ *      iteration since the kernel started).  d_info (16 doubles): [0] entries written, [1] trips, [2] cluster size,
+ *      [3] 1 when the very first trip stopped on D(z, z-) < epsilon, where the reference's Gdr is unbound (the solve
+ *      ends there), [4] the last G (ABPG) or gain (ABPG_gain).  Assertions arrive in the status word as for BPG and end
+ *      the solve.  ACCBPG_E_ARG on NULL pointers, a shape that does not fit, non-finite or non-positive L, gamma, G0,
+ *      ls_inc or ls_dec, maxitrs < 1 or reanchor_every < 1. */
+#define ACCBPG_SMALL_DRV_ABPG        0
+#define ACCBPG_SMALL_DRV_ABPG_GAIN   1
+#define ACCBPG_SMALL_RESTART_NONE    0
+#define ACCBPG_SMALL_RESTART_F       1   /* F[k] > F[k-1]                algorithms.py:168, :406 */
+#define ACCBPG_SMALL_RESTART_G       2   /* dot(g, x - x-) > 0           algorithms.py:168, :406 */
+/* 0 when no cluster of <= 8 CTAs holds A and the accelerated solve's vectors in shared memory (host only) */
+size_t accbpg_linreg_abpg_small_smem_bytes(int64_t m, int64_t n);
+int accbpg_linreg_abpg_small(void* ctx, void* stream, int driver, int kind, const double* d_A, int64_t m, int64_t n,
+                             int64_t lda, const double* d_b, int hkind, double lamda, double delta, double* d_x,
+                             double L, double gamma, int maxitrs, double epsilon, int theta_eq, int restart,
+                             int restart_rule, double G0, double ls_inc, double ls_dec, int checkdiv,
+                             int reanchor_every, double* d_hist, double* d_info);
 
 /* ---- D_opt_FW / D_opt_FW_away (accbpg/D_opt_alg.py:9-88, :91-185) -------
  * State lives in caller-owned device buffers: x, w (n), Hinv (m x m, ld m), a control block of
