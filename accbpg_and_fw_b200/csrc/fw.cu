@@ -150,11 +150,9 @@ struct FwParams {
     int64_t col_offset;       // global index of local column 0
     int sharded;              // decide: the chosen column may live on another rank (then v <- 0 here)
     int reverse;              // pass kernel: walk the column blocks from the end
-    int dbg;                  // fw_pass_ring_kernel: write timing stamps (experiment)
-    int ring_3d;              // fw_pass_ring_kernel: the tensor map is 3-D (columns, rows of a group, row groups)
-    int ring_stages;          // fw_pass_ring_kernel: stages of the shared-memory ring (0: that kernel is not used)
-    int early;                // pass kernel: rows of V fetched before the dependency wait (registers: the first batch; L2:
-                              // `early - FWP_UNROLL` more rows); 0 = nothing is touched before the wait
+    int early;                // pass kernel: rows of V fetched before the dependency wait, always FWP_EARLY (a launch
+                              // parameter rather than the constant: compiled in, it costs fw_pass_kernel<true> two
+                              // registers and a different schedule)
 };
 
 // The decision of iteration p.k from the merged candidates (thread 0 of the last CTA), then the gather of the chosen
@@ -351,8 +349,6 @@ __global__ void __launch_bounds__(FW_THREADS) fw_select_kernel(FwParams p) {
     fw_select_tail(p, cd, blockIdx.x, gridDim.x, sh_c, &sh_last, &sh_go, &sh_idx);
 }
 
-__device__ unsigned long long g_fwr_dbg[512 * 8];   // timing experiment (ACCBPG_FW_DBG=4)
-
 // u = Hinv v (warp per row)            D_opt_alg.py:78 / :165 / :174
 __global__ void __launch_bounds__(256) fw_hv_kernel(const double* __restrict__ Hinv, int m, const double* __restrict__ v,
                                                     double* __restrict__ u, const double* ctrl,
@@ -385,6 +381,9 @@ __global__ void __launch_bounds__(256) fw_hv_kernel(const double* __restrict__ H
 constexpr int FWP_THREADS = 256;
 constexpr int FWP_COLS = 128;
 constexpr int FWP_UNROLL = 16;       // rows in flight per thread (16 x 16 B)
+// rows per row group fetched before the dependency wait: the first FWP_UNROLL into registers, the rest as L2 prefetches
+// (measured at 500 x 50000: 48 rows 19.2 k iterations per second, 80 rows 18.8 k, 125 rows 17.6 k)
+constexpr int FWP_EARLY = 48;
 
 template <bool VEC2>
 __global__ void __launch_bounds__(FWP_THREADS) fw_pass_kernel(FwParams p) {
@@ -514,23 +513,46 @@ __global__ void __launch_bounds__(FWP_THREADS) fw_pass_kernel(FwParams p) {
 }
 
 // ------------------------------------------------------------------------------------------------------------------
-// The pass as one CTA per SM fed by a bulk-copy ring (the default when V is 16-byte aligned with even n and ldv).
-// A CTA owns the column blocks b = blockIdx.x, blockIdx.x + G, ...; a producer warp streams their rows into a shared
-// memory ring (one 2-D tensor copy per row group: a stage holds FWR_ROWS rows of each of the four row groups; single
-// row copies issued per lane serialise in the TMA unit and reach 3 TB/s only),
-// eight consuming warps form p_j = u^T v_j from the ring with the summation order of fw_pass_kernel (four row groups,
-// rows in order, groups merged ((0+1)+2)+3), so w, x and the vertex sequence are bit-identical.  Bytes in flight are
-// bounded by shared memory (6 x 32 KB per SM) instead of registers, which keeps HBM busy through the tail of the pass,
-// and the ring is filled BEFORE the dependency wait: launched programmatically behind u = Hinv v (which releases its
-// dependents before its own wait), a CTA becomes resident as soon as the previous pass leaves its SM and pulls the
-// first 192 KB of its columns while that pass drains, takes its decision and u = Hinv v is formed (V never changes).
-// The rank-one update of Hinv is shared by all CTAs (a grid-stride slice each, before the first stage is consumed).
+// The same loop as ONE persistent launch per batch of iterations (one GPU; accbpg_fw_run takes it when V is 16-byte
+// aligned with even n and ldv, n < 2^31, m <= 4096 and at least three ring stages fit in shared memory).  One CTA per SM
+// owns the column blocks b = blockIdx.x, blockIdx.x + G, ... of W columns; one producer thread streams their rows into a
+// shared-memory ring (one 3-D tensor copy per stage when 4 | m, else one 2-D copy per row group: a stage holds FWR_ROWS
+// rows of each of the four row groups; single row copies issued per lane serialise in the TMA unit and reach 3 TB/s
+// only).  Bytes in flight are bounded by shared memory (6 x 32 KB per SM) instead of registers.
+// Measured with this ring feeding the pass of the launch chain at 500 x 50000 (DESIGN.md section 11): the ring streams the
+// 200 MB of V in 29.6 us (6.8 TB/s, the copy roof), but an iteration takes 53 us because the decision tail (13.5 us after
+// the last CTA has finished streaming) and the u = Hinv v launch (8.6 us between the decision and the next pass) are
+// serial.  Here nothing is launched between iterations:
+//   records   every CTA reads all G selection records itself (one store -> poll hop), merges them and takes the
+//             decision of iteration k on its own copy of the log-det accumulator (CTA 0 writes the history entry and the
+//             control block), then gathers the chosen column
+//   u         rows cta + i G of Hinv times the column (warp per row), delivered as (value, token) words every CTA collects
+//   pass      warps 0-7 consume the ring (row groups and summation order of fw_pass_kernel: four row groups, rows in
+//             order, groups merged ((0+1)+2)+3, so w, x and the vertex sequence are bit-identical), lane 0 of warp 8
+//             feeds it and, towards the end of the pass, already issues the first stages of the NEXT iteration (V never
+//             changes), which land during the exchanges; warps 9-15 apply the rank-one update to the own rows of Hinv
+//   record    of the updated columns, for the next decision
+// The arithmetic is that of the launch chain, operation for operation.  Exchanges are stores followed by a release of a
+// token word that the consumer polls; tokens are unique per launch and iteration, buffers alternate on the iteration's
+// parity.
 constexpr int FWR_ROWS = 8;                                  // rows per row group and stage (one tensor box)
 constexpr int FWR_BOX_BYTES = FWR_ROWS * FWP_COLS * 8;       // bytes reserved per box (rows packed at width * 8 bytes)
 constexpr int FWR_STAGE_BYTES = 4 * FWR_BOX_BYTES;           // 32 KB
 constexpr int FWR_MAX_STAGES = 6;
-constexpr int FWR_THREADS = FWP_THREADS + 64;                // eight consuming warps, the producer warp, the Hinv warp
 constexpr int FWR_STATIC_SMEM = 12 * 1024;                   // part, records, barriers (upper bound used by the host)
+constexpr int FWS_THREADS = 512;
+constexpr int FWS_CONS = 256;                                // consuming threads (warps 0-7)
+constexpr int FWQ_REC_DOUBLES = 16;                          // a selection record's slot: one 128-byte line
+
+struct FwPersist {
+    double* ux;                    // [2][m] (value, token) pairs: the entries of u, each written by the CTA that owns the row
+    double* recs;                  // [2][G][FWQ_REC_DOUBLES] selection records
+    unsigned long long* tok;       // [2][256] flag words, one per CTA, released after its record
+    unsigned long long base;
+    int G, k_start, k_count;
+    int stages;                    // stages of the shared-memory ring
+    int ring_3d;                   // the tensor map is 3-D (columns, rows of a group, row groups)
+};
 
 __device__ __forceinline__ void fwr_mbar_init(uint32_t bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
@@ -559,230 +581,6 @@ __device__ __forceinline__ void fwr_tma_load_2d(uint32_t dst, const void* tmap, 
                  ::"r"(dst), "l"(tmap), "r"(c0), "r"(c1), "r"(bar) : "memory");
 }
 
-// timing experiment (ACCBPG_FW_DBG=4, tools/exp_s2.py stamps): globaltimer stamps of the last pass, per CTA
-__device__ __forceinline__ void fwr_stamp(int on, int slot) {      // on: 1 = first stamped pass, 2 = the one after it
-    if (on) {
-        unsigned long long ns;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns));
-        g_fwr_dbg[((on - 1) * 256 + blockIdx.x) * 8 + slot] = ns;
-    }
-}
-
-__global__ void __launch_bounds__(FWR_THREADS, 1) fw_pass_ring_kernel(FwParams p, const __grid_constant__ CUtensorMap tmV) {
-    extern __shared__ __align__(128) unsigned char fwr_raw[];      // ring [S][4][FWR_BOX_BYTES], then u (m doubles)
-    __shared__ double part[2][4][FWP_COLS];
-    __shared__ FwCand sh_c[32];
-    __shared__ __align__(8) unsigned long long bar_mem[2 * FWR_MAX_STAGES];
-    __shared__ bool sh_last;
-    __shared__ int sh_go;
-    __shared__ long long sh_idx;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int m = p.m, S = p.ring_stages, G = (int)gridDim.x;
-    const uint32_t ring = (uint32_t)__cvta_generic_to_shared(fwr_raw);
-    double* us = reinterpret_cast<double*>(fwr_raw + (size_t)S * FWR_STAGE_BYTES);
-    const uint32_t bars = (uint32_t)__cvta_generic_to_shared(bar_mem);
-    const int rows_per = (m + 3) / 4;
-    const int chunks = (rows_per + FWR_ROWS - 1) / FWR_ROWS;          // stages per column block
-    const int nmine = ((int)blockIdx.x < p.nblk) ? (p.nblk - 1 - (int)blockIdx.x) / G + 1 : 0;
-    const int total = nmine * chunks;
-    const int dbg = (p.dbg && tid == 0 && (p.k == 101 || p.k == 102)) ? p.k - 100 : 0;
-    fwr_stamp(dbg, 0);
-    if (tid == 0) {
-        for (int s = 0; s < S; ++s) {
-            fwr_mbar_init(bars + 8 * s, 1);                            // full: the producer's arrive.expect_tx
-            fwr_mbar_init(bars + 8 * (FWR_MAX_STAGES + s), FWP_THREADS / 32);   // empty: one arrival per consuming warp
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    FwCand cd;
-    fw_cand_init(cd);
-    if (warp == FWP_THREADS / 32) {
-        // ---- producer warp: lane 0 issues the four boxes of a stage (rows beyond a row group's end - the last box of a
-        // group when rows_per is not a multiple of FWR_ROWS - and columns beyond n are loaded or zero-filled and ignored)
-        const uint32_t stage_tx = 4u * FWR_ROWS * (uint32_t)p.width * 8u;
-        const uint32_t box_pitch = FWR_ROWS * (uint32_t)p.width * 8u;      // boxes packed as the 3-D copy lays them out
-        auto issue = [&](int c) {
-            if (lane != 0) return;
-            const int st = c % S;
-            const int bi = c / chunks, ch = c - bi * chunks;
-            const int b = (int)blockIdx.x + bi * G;
-            const int cb = p.reverse ? (p.nblk - 1 - b) : b;
-            const int j0 = cb * p.width;
-            if (c >= S) fwr_mbar_wait(bars + 8 * (FWR_MAX_STAGES + st), ((c / S) + 1) & 1);
-            fwr_mbar_expect(bars + 8 * st, stage_tx);
-            if (p.ring_3d) {                                 // m = 4 rows_per: one box over (columns, rows, row groups)
-                fwr_tma_load_3d(ring + st * FWR_STAGE_BYTES, &tmV, j0, ch * FWR_ROWS, 0, bars + 8 * st);
-            } else {
-#pragma unroll
-                for (int g4 = 0; g4 < 4; ++g4)
-                    fwr_tma_load_2d(ring + st * FWR_STAGE_BYTES + g4 * box_pitch, &tmV, j0, g4 * rows_per + ch * FWR_ROWS,
-                                    bars + 8 * st);
-            }
-        };
-        int c = 0;
-        if (p.early > 0) {                                   // V only: nothing here depends on the kernels in front
-            const int pre = total < S ? total : S;
-            for (; c < pre; ++c) issue(c);
-        }
-        asm volatile("griddepcontrol.wait;" ::: "memory");
-        asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-        if (ld_cg(&p.ctrl[C_STOP]) != 0.0) {                 // uniform over the grid: let the copies in flight land, then leave
-            if (lane == 0)
-                for (int q = 0; q < c; ++q) fwr_mbar_wait(bars + 8 * q, 0);
-            return;
-        }
-        for (; c < total; ++c) issue(c);
-    } else if (warp == FWP_THREADS / 32 + 1) {
-        // ---- Hinv <- (Hinv - cs u u^T)/den  (D_opt_alg.py:79 / :166 / :175): a grid-stride slice per CTA, off the
-        // consumers' path; eight independent elements in flight per lane
-        asm volatile("griddepcontrol.wait;" ::: "memory");
-        asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-        if (ld_cg(&p.ctrl[C_STOP]) != 0.0) return;
-        const double cs = ld_cg(&p.ctrl[C_CS]), den = ld_cg(&p.ctrl[C_DEN]);
-        const unsigned tot = (unsigned)m * (unsigned)m, um = (unsigned)m;      // m <= 20480 here (u fits shared memory)
-        const unsigned stride = (unsigned)G * 32u;
-        for (unsigned e0 = blockIdx.x * 32u + lane; e0 < tot; e0 += 8u * stride) {
-            double h[8], o[8];
-#pragma unroll
-            for (int q = 0; q < 8; ++q) {
-                const unsigned e = e0 + q * stride;
-                if (e < tot) {
-                    const unsigned r = e / um, cc = e - r * um;
-                    h[q] = __ldcg(p.Hinv + e);
-                    o[q] = __ldcg(p.u + r) * __ldcg(p.u + cc);
-                }
-            }
-#pragma unroll
-            for (int q = 0; q < 8; ++q) {
-                const unsigned e = e0 + q * stride;
-                if (e < tot) p.Hinv[e] = (h[q] - cs * o[q]) / den;
-            }
-        }
-    } else {
-        // ---- consuming warps
-        asm volatile("griddepcontrol.wait;" ::: "memory");
-        asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-        fwr_stamp(dbg, 1);
-        if (ld_cg(&p.ctrl[C_STOP]) != 0.0) return;
-        const double cs = ld_cg(&p.ctrl[C_CS]), den = ld_cg(&p.ctrl[C_DEN]);
-        for (int r = tid; r < m; r += FWP_THREADS) us[r] = __ldcg(p.u + r);
-        asm volatile("bar.sync 1, %0;" ::"n"(FWP_THREADS) : "memory");
-        const int rg = tid >> 6, ct = tid & 63;
-        const int r0 = rg * rows_per, r1 = min(m, r0 + rows_per);
-        const double thr = p.away ? 1.0e-8 : 0.0;
-        const int64_t idx = (int64_t)ld_cg(&p.ctrl[C_IDX]);
-        const double tsign = ld_cg(&p.ctrl[C_TSIGN]);
-        const uint32_t seg = (uint32_t)p.width * 8u;         // row pitch inside a box
-        int c = 0;
-        for (int bi = 0; bi < nmine; ++bi) {
-            const int b = (int)blockIdx.x + bi * G;
-            const int cb = p.reverse ? (p.nblk - 1 - b) : b;
-            const int64_t j = (int64_t)cb * p.width + ct * 2;
-            const bool owns = (ct * 2 < p.width) && (j < p.n);
-            double s0 = 0.0, s1 = 0.0;
-            for (int ch = 0; ch < chunks; ++ch, ++c) {
-                const int st = c % S;
-                fwr_mbar_wait(bars + 8 * st, (c / S) & 1);
-                if (c == 0) fwr_stamp(dbg, 2);
-                if (owns) {
-                    const uint32_t base = ring + st * FWR_STAGE_BYTES + rg * (FWR_ROWS * seg) + ct * 16;
-                    const int rb = r0 + ch * FWR_ROWS;
-#pragma unroll
-                    for (int q = 0; q < FWR_ROWS; ++q) {
-                        if (rb + q < r1) {
-                            double ax, ay;
-                            asm volatile("ld.shared.v2.f64 {%0,%1}, [%2];" : "=d"(ax), "=d"(ay) : "r"(base + q * seg));
-                            const double uq = us[rb + q];
-                            s0 += uq * ax;
-                            s1 += uq * ay;
-                        }
-                    }
-                }
-                __syncwarp();
-                if (lane == 0) fwr_mbar_arrive(bars + 8 * (FWR_MAX_STAGES + st));
-            }
-            const int buf = bi & 1;
-            part[buf][rg][2 * ct] = s0;
-            part[buf][rg][2 * ct + 1] = s1;
-            asm volatile("bar.sync 1, %0;" ::"n"(FWP_THREADS) : "memory");
-            if (rg == 0 && owns) {
-#pragma unroll
-                for (int e = 0; e < 2; ++e) {
-                    if (j + e < p.n) {
-                        const double pj = ((part[buf][0][2 * ct + e] + part[buf][1][2 * ct + e]) + part[buf][2][2 * ct + e]) +
-                                          part[buf][3][2 * ct + e];
-                        const double wn = (p.w[j + e] - cs * (pj * pj)) / den;
-                        double xn = p.x[j + e] * den;
-                        if (j + e + p.col_offset == idx) xn = xn + tsign;
-                        p.w[j + e] = wn;
-                        p.x[j + e] = xn;
-                        fw_cand_add(cd, wn, xn, j + e + p.col_offset, thr);
-                    }
-                }
-            }
-        }
-    }
-    fwr_stamp(dbg, 3);
-    if (!p.decide) return;
-    fw_select_tail(p, cd, (int)blockIdx.x, G, sh_c, &sh_last, &sh_go, &sh_idx);
-    fwr_stamp(dbg, 4);
-}
-
-// ------------------------------------------------------------------------------------------------------------------
-// The same loop as ONE persistent launch per batch of iterations (one GPU): one CTA per SM owns a fixed block of columns
-// of V for the whole batch and keeps part of it in shared memory, so an iteration reads less than all of V from HBM and
-// costs no kernel launches.  Per iteration k (the leader is CTA 0):
-//   every CTA gathers all CTAs' selection records, merges them and takes the decision of iteration k with the step rule of
-//            fw_decide on its own copy of the log-det accumulator (the same inputs give the same decision everywhere;
-//            CTA 0 writes the history entry and the control block), then gathers the chosen column v itself
-//   u_r = Hinv[r,:] v for the rows r = CTA + i G a CTA owns (warp per row), delivered as (value, token) words that
-//            every CTA collects: u is complete everywhere after one store -> poll hop
-//   rank-one update of the own rows of Hinv; the pass over the own columns (p_j = u^T v_j with the same four row groups
-//            and the same summation order as fw_pass_kernel, w_j and x_j updates); selection record of the updated
-//            slice published for the next decision
-// The arithmetic is that of the five-kernel iteration above, operation for operation: histories, vertex sequences and
-// iterates are bit-identical.  Exchanges are stores followed by a release of a token word that the consumer polls; tokens
-// are unique per launch and iteration, buffers alternate on the iteration's parity.
-constexpr int FWQ_THREADS = 512;
-constexpr int FWQ_TEAM = 256;
-constexpr int FWQ_REPL = 16;                            // replicas of the merged record (one line each)
-constexpr int FWQ_REC_DOUBLES = 16;                     // a selection record: 8 (value, token) words of 16 bytes = one 128-byte line
-
-struct FwPersist {
-    double* ux;                    // [2][m] (value, token) pairs: the entries of u, each written by the CTA that owns the row
-    double* bcast;                 // [2][FWQ_REPL][FWQ_REC_DOUBLES] the merged record of an iteration, replicated
-    double* recs;                  // [2][G][FWQ_REC_DOUBLES]
-    unsigned long long* tok;       // (unused)
-    unsigned long long base;
-    int G, k_start, k_count;
-    int per;                       // columns per CTA (even)
-    int rc4;                       // rows of every row group kept in shared memory
-    int dbg;                       // ACCBPG_FW_DBG: 1 print phase times of one iteration (CTA 0 and 1), 3 all CTAs via dbg_buf
-    unsigned long long* dbg_buf;
-};
-
-__device__ __forceinline__ void fwq_wait(const unsigned long long* p, unsigned long long token) {
-    unsigned long long t0 = 0;
-    unsigned spin = 0;
-    for (;;) {
-        unsigned long long v;
-        asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-        if (v == token) return;
-        __nanosleep(32);
-        if ((++spin & 0x3ffu) == 0) {
-            unsigned long long now;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-            if (t0 == 0) t0 = now;
-            else if (now - t0 > 4000000000ULL) __trap();
-        }
-    }
-}
-__device__ __forceinline__ unsigned long long fwq_ld_acquire(const unsigned long long* p) {
-    unsigned long long v;
-    asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
 __device__ __forceinline__ void fwq_post(unsigned long long* p, unsigned long long token) {
     asm volatile("st.release.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(token) : "memory");
 }
@@ -803,43 +601,6 @@ __device__ __forceinline__ double fwq_wait_pair(const double* p, unsigned long l
             else if (now - t0 > 4000000000ULL) __trap();
         }
     }
-}
-
-// rows [r, r1) of a column pair streamed from HBM, sixteen 16-byte loads in flight per thread; accumulates in row order.
-// Kept out of line so that its schedule (all sixteen loads issued before the first use) does not depend on the register
-// pressure of the exchange code around it.
-__device__ __noinline__ void fwq_stream(const double* col, int64_t ldv, const double* us, int r, int r1, double& s0, double& s1) {
-    double a0 = s0, a1 = s1;
-    for (; r + FWP_UNROLL <= r1; r += FWP_UNROLL) {
-        double2 a[FWP_UNROLL];
-#pragma unroll
-        for (int e = 0; e < FWP_UNROLL; ++e)
-            asm volatile("ld.global.nc.L1::no_allocate.v2.f64 {%0,%1}, [%2];"
-                         : "=d"(a[e].x), "=d"(a[e].y) : "l"(col + (int64_t)(r + e) * ldv));
-#pragma unroll
-        for (int e = 0; e < FWP_UNROLL; ++e) {
-            const double uq = us[r + e];
-            a0 += uq * a[e].x;
-            a1 += uq * a[e].y;
-        }
-    }
-    const int rem = r1 - r;                              // < 16 rows left: one more batch, predicated (a rolled loop would pay
-    if (rem > 0) {                                       // the HBM latency once per row)
-        double2 a[FWP_UNROLL];
-#pragma unroll
-        for (int e = 0; e < FWP_UNROLL; ++e)
-            if (e < rem)
-                asm volatile("ld.global.nc.L1::no_allocate.v2.f64 {%0,%1}, [%2];"
-                             : "=d"(a[e].x), "=d"(a[e].y) : "l"(col + (int64_t)(r + e) * ldv));
-#pragma unroll
-        for (int e = 0; e < FWP_UNROLL; ++e)
-            if (e < rem) {
-                const double uq = us[r + e];
-                a0 += uq * a[e].x;
-                a1 += uq * a[e].y;
-            }
-    }
-    s0 = a0; s1 = a1;
 }
 
 // the step rule of fw_decide on a copy of the log-det accumulator kept by every CTA (all CTAs take the same decision from
@@ -911,280 +672,6 @@ __device__ __forceinline__ void fwq_decide(const FwParams& p, const FwCand& cd, 
     d.cs = cs; d.den = den; d.tsign = tsign; d.idx = chosen;
 }
 
-__global__ void __launch_bounds__(FWQ_THREADS, 1) fw_persistent_kernel(FwParams p, FwPersist q) {
-    extern __shared__ __align__(16) double fsm[];
-    const int m = p.m;
-    const int mpad = (m + 1) / 2 * 2;
-    double* us = fsm;                                   // u
-    double* vs = us + mpad;                             // v (the chosen column)
-    double* part = vs + mpad;                           // [2 teams][4 row groups][128]
-    double* vc = part + 2 * 4 * FWP_COLS;               // [4 row groups][rc4][per]: rows kept from HBM
-    __shared__ FwCand sh_c[32];
-    __shared__ FwDec sh_dec;
-    __shared__ double sh_logdet[2];
-    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    const int G = q.G, cta = blockIdx.x;
-    if (ld_cg(&p.ctrl[C_STOP]) != 0.0) return;          // stopped in an earlier batch: uniform over the grid
-    if (tid == 0) { sh_logdet[0] = ld_cg(&p.ctrl[C_LOGDET_HI]); sh_logdet[1] = ld_cg(&p.ctrl[C_LOGDET_LO]); }
-    const int64_t c0 = (int64_t)cta * q.per;
-    const int64_t c1 = c0 + q.per < p.n ? c0 + q.per : p.n;
-    const int ncol = c1 > c0 ? (int)(c1 - c0) : 0;
-    const int rows_per = (m + 3) / 4;
-    const double thr = p.away ? 1.0e-8 : 0.0;
-    const int team = tid >> 8, tt = tid & 255, rg = tt >> 6, ct = tt & 63;
-    const int r0 = rg * rows_per, r1 = min(m, r0 + rows_per);
-    const int rcn = min(q.rc4, max(r1 - r0, 0));        // cached rows of this row group
-    const int nown = cta < m ? (m - cta + G - 1) / G : 0;      // rows of Hinv / entries of u this CTA owns: cta + i G
-    // ---- the cached rows of the own column block
-    for (int g2 = 0; g2 < 4; ++g2) {
-        const int rr0 = g2 * rows_per, rrn = min(q.rc4, max(min(m, rr0 + rows_per) - rr0, 0));
-        for (int e = tid; e < rrn * (q.per / 2); e += FWQ_THREADS) {
-            const int rr = e / (q.per / 2), cp = (e - rr * (q.per / 2)) * 2;
-            double2 a = make_double2(0.0, 0.0);
-            if (c0 + cp < p.n) {
-                if (c0 + cp + 1 < p.n) a = *reinterpret_cast<const double2*>(p.V + (int64_t)(rr0 + rr) * p.ldv + c0 + cp);
-                else a.x = p.V[(int64_t)(rr0 + rr) * p.ldv + c0 + cp];
-            }
-            *reinterpret_cast<double2*>(vc + ((size_t)g2 * q.rc4 + rr) * q.per + cp) = a;
-        }
-    }
-    // ---- the record of the first decision: candidates of the own columns from (w, x) as they are
-    FwCand cd;
-    fw_cand_init(cd);
-    for (int64_t j = c0 + tid; j < c1; j += FWQ_THREADS) fw_cand_add(cd, p.w[j], p.x[j], j, thr);
-    auto deliver_record = [&](int it) {                 // record for the decision of batch iteration `it`
-        fw_cand_block(cd, sh_c);
-        if (tid < 8) {                                   // warp 0 holds the merged record in every lane: one word per lane
-            double* dst = q.recs + ((size_t)(it & 1) * G + cta) * FWQ_REC_DOUBLES;
-            const double f8[8] = {cd.amax, __longlong_as_double(cd.imax), cd.smin, __longlong_as_double(cd.imin), cd.xmin,
-                                  __longlong_as_double(cd.fmask), cd.wmask, cd.xmask};
-            double val = f8[0];
-#pragma unroll
-            for (int e = 1; e < 8; ++e) if (tid == e) val = f8[e];
-            fwq_st_pair(dst + 2 * tid, val, q.base + 4ULL * (unsigned long long)it);
-        }
-    };
-    deliver_record(0);
-    unsigned long long ts[10];
-#define FWQ_STAMP(i) do { if (q.dbg && tid == 0 && (cta < 2 || q.dbg == 3) && it == 5) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ts[i])); } while (0)
-    for (int it = 0; it < q.k_count; ++it) {
-        const int par = it & 1;
-        const unsigned long long tokD = q.base + 4ULL * it, tokB = tokD + 2;
-        FWQ_STAMP(0);
-        // ---- CTA 0 gathers the records (one private line per CTA) and merges them; the merged record goes out in
-        //      FWQ_REPL replicas so that no line is polled by more than a handful of CTAs
-        const unsigned long long tokA = tokD + 1;
-        auto read_record = [&](const double* src, unsigned long long token, int sleep_ns, FwCand& o) {
-            double f8[8];
-            unsigned done = 0;
-            unsigned long long t0 = 0;
-            unsigned spin = 0;
-            while (done != 0xffu) {                      // eight loads in flight; a word counts once it carries the token
-                unsigned long long v[8], tk[8];
-#pragma unroll
-                for (int e = 0; e < 8; ++e)
-                    if (!(done & (1u << e)))
-                        asm volatile("ld.volatile.global.v2.u64 {%0, %1}, [%2];" : "=l"(v[e]), "=l"(tk[e]) : "l"(src + 2 * e) : "memory");
-#pragma unroll
-                for (int e = 0; e < 8; ++e)
-                    if (!(done & (1u << e)) && tk[e] == token) { f8[e] = __longlong_as_double((long long)v[e]); done |= 1u << e; }
-                if (done != 0xffu) {
-                    __nanosleep(sleep_ns);
-                    if ((++spin & 0x3ffu) == 0) {
-                        unsigned long long now;
-                        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-                        if (t0 == 0) t0 = now;
-                        else if (now - t0 > 4000000000ULL) __trap();
-                    }
-                }
-            }
-            o.amax = f8[0]; o.imax = __double_as_longlong(f8[1]);
-            o.smin = f8[2]; o.imin = __double_as_longlong(f8[3]); o.xmin = f8[4];
-            o.fmask = __double_as_longlong(f8[5]); o.wmask = f8[6]; o.xmask = f8[7];
-        };
-        if (cta == 0) {
-            fw_cand_init(cd);
-            for (int b = tid; b < G; b += FWQ_THREADS) {
-                FwCand o;
-                read_record(q.recs + ((size_t)par * G + b) * FWQ_REC_DOUBLES, tokD, 40, o);
-                fw_cand_merge(cd, o);
-            }
-            fw_cand_block(cd, sh_c);                      // merged record in every lane of warp 0
-                    if (wid == 0 && lane == 0) sh_c[0] = cd;
-            __syncthreads();
-            if (tid < 8 * FWQ_REPL) {
-                const FwCand mc = sh_c[0];
-                const int e = tid & 7, rep = tid >> 3;
-                const double f8[8] = {mc.amax, __longlong_as_double(mc.imax), mc.smin, __longlong_as_double(mc.imin), mc.xmin,
-                                      __longlong_as_double(mc.fmask), mc.wmask, mc.xmask};
-                double val = f8[0];
-#pragma unroll
-                for (int k2 = 1; k2 < 8; ++k2) if (e == k2) val = f8[k2];
-                fwq_st_pair(q.bcast + ((size_t)par * FWQ_REPL + rep) * FWQ_REC_DOUBLES + 2 * e, val, tokA);
-            }
-        }
-        // ---- every CTA: the merged record (its replica), then the decision of iteration k (CTA 0 records it)
-        fw_cand_init(cd);
-        if (tid == 0) {
-            FwCand o;
-            read_record(q.bcast + ((size_t)par * FWQ_REPL + (cta % FWQ_REPL)) * FWQ_REC_DOUBLES, tokA, 100, o);
-            sh_c[1] = o;
-        }
-        __syncthreads();
-        cd = sh_c[1];
-        FWQ_STAMP(1);
-        if (tid == 0) {
-            FwDec d;
-            d.cs = d.den = d.tsign = 0.0; d.idx = 0; d.go = 0;
-            fwq_decide(p, cd, q.k_start + it, sh_logdet[0], sh_logdet[1], cta == 0, d);
-            sh_dec = d;
-        }
-        __syncthreads();
-        if (!sh_dec.go) return;                          // the optimality test fired at this iteration: uniform
-        const double cs = sh_dec.cs, den = sh_dec.den, tsign = sh_dec.tsign;
-        const int64_t idx = sh_dec.idx;
-        for (int r = tid; r < m; r += FWQ_THREADS) vs[r] = __ldg(p.V + (int64_t)r * p.ldv + idx);      // the chosen column
-        __syncthreads();
-        FWQ_STAMP(2);
-        // ---- u_r = Hinv[r,:] v for the own rows (warp per row, as fw_hv_kernel), delivered to every CTA's view
-        for (int i = wid; i < nown; i += FWQ_THREADS / 32) {
-            const int r = cta + i * G;
-            const double* hr = p.Hinv + (size_t)r * m;
-            double sacc = 0.0;
-            for (int c = lane; c < m; c += 32) sacc += __ldcg(hr + c) * vs[c];
-            sacc = warp_sum(sacc);
-            if (lane == 0) fwq_st_pair(q.ux + ((size_t)par * m + r) * 2, sacc, tokB);
-        }
-        FWQ_STAMP(3);
-        for (int r = tid; r < m; r += FWQ_THREADS) us[r] = fwq_wait_pair(q.ux + ((size_t)par * m + r) * 2, tokB);
-        __syncthreads();
-        FWQ_STAMP(4);
-        // ---- Hinv <- (Hinv - cs u u^T)/den on the own rows      D_opt_alg.py:79 / :166 / :175
-        for (int e0 = tid; e0 < nown * m; e0 += FWQ_THREADS * 4) {
-            double hv[4];
-#pragma unroll
-            for (int u4 = 0; u4 < 4; ++u4) {
-                const int e = e0 + u4 * FWQ_THREADS;
-                if (e < nown * m) { const int i = e / m, c = e - i * m; hv[u4] = __ldcg(p.Hinv + (size_t)(cta + i * G) * m + c); }
-            }
-#pragma unroll
-            for (int u4 = 0; u4 < 4; ++u4) {
-                const int e = e0 + u4 * FWQ_THREADS;
-                if (e < nown * m) {
-                    const int i = e / m, c = e - i * m, r = cta + i * G;
-                    const double o = us[r] * us[c];
-                    p.Hinv[(size_t)r * m + c] = (hv[u4] - cs * o) / den;
-                }
-            }
-        }
-        // ---- the pass over the own columns: two teams of 256 threads take alternate 128-column sub-blocks
-        FWQ_STAMP(5);
-        fw_cand_init(cd);
-        const int nsub = (ncol + FWP_COLS - 1) / FWP_COLS;
-        const int nsub2 = (nsub + 1) / 2 * 2;             // both teams run the same number of rounds
-        for (int sb = team; sb < nsub2; sb += 2) {
-            const int jrel = sb * FWP_COLS + ct * 2;
-            const int64_t j = c0 + jrel;
-            const bool owns = (sb < nsub) && (jrel < ncol);
-            double s0 = 0.0, s1 = 0.0;
-            if (owns) {
-                const bool two = (j + 1 < p.n) && (jrel + 1 < ncol);
-                const double* vcr = vc + (size_t)rg * q.rc4 * q.per + jrel;
-                for (int rr = 0; rr < rcn; ++rr) {
-                    const double2 a = *reinterpret_cast<const double2*>(vcr + (size_t)rr * q.per);
-                    const double uq = us[r0 + rr];
-                    s0 += uq * a.x;
-                    s1 += uq * a.y;
-                }
-                const double* col = p.V + j;
-                int r = r0 + rcn;
-                if (two) {
-                    fwq_stream(col, p.ldv, us, r, r1, s0, s1);
-                } else {
-                    for (; r < r1; ++r) s0 += us[r] * __ldcs(col + (int64_t)r * p.ldv);
-                }
-            }
-            double* pt = part + (size_t)team * 4 * FWP_COLS;
-            pt[rg * FWP_COLS + 2 * ct] = s0;
-            pt[rg * FWP_COLS + 2 * ct + 1] = s1;
-            asm volatile("bar.sync %0, %1;" ::"r"(1 + team), "n"(FWQ_TEAM) : "memory");
-            if (rg == 0 && owns) {
-#pragma unroll
-                for (int e = 0; e < 2; ++e) {
-                    if (j + e < p.n && jrel + e < ncol) {
-                        const double pj = ((pt[2 * ct + e] + pt[FWP_COLS + 2 * ct + e]) + pt[2 * FWP_COLS + 2 * ct + e]) +
-                                          pt[3 * FWP_COLS + 2 * ct + e];
-                        const double wn = (p.w[j + e] - cs * (pj * pj)) / den;
-                        double xn = p.x[j + e] * den;
-                        if (j + e == idx) xn = xn + tsign;
-                        p.w[j + e] = wn;
-                        p.x[j + e] = xn;
-                        fw_cand_add(cd, wn, xn, j + e, thr);
-                    }
-                }
-            }
-            asm volatile("bar.sync %0, %1;" ::"r"(1 + team), "n"(FWQ_TEAM) : "memory");
-        }
-        __syncthreads();
-        FWQ_STAMP(6);
-        deliver_record(it + 1);
-        FWQ_STAMP(7);
-        if (q.dbg == 3 && tid == 0 && it == 5 && q.dbg_buf) {
-            for (int i = 0; i < 8; ++i) q.dbg_buf[cta * 8 + i] = ts[i];
-        }
-        if (q.dbg == 1 && tid == 0 && cta < 2 && it == 5)
-            printf("fw persistent cta %d: records %llu ns, decide + column %llu, u rows %llu, u gather %llu, Hinv rows %llu, pass %llu, record %llu | iteration %llu ns\n",
-                   cta, ts[1] - ts[0], ts[2] - ts[1], ts[3] - ts[2], ts[4] - ts[3], ts[5] - ts[4], ts[6] - ts[5], ts[7] - ts[6], ts[7] - ts[0]);
-    }
-}
-
-// ------------------------------------------------------------------------------------------------------------------
-// The persistent loop with the pass fed by the tensor-copy ring of fw_pass_ring_kernel (the default on one GPU when the
-// operands allow it).  Measured on the two-launch chain at 500 x 50000 (globaltimer stamps, tools/exp_s2.py stamps): the
-// ring streams the 200 MB of V in 29.6 us (6.8 TB/s, the copy roof), but an iteration takes 53 us because the decision
-// tail (13.5 us after the last CTA has finished streaming) and the u = Hinv v launch (8.6 us between the decision and the
-// next pass) are serial.  Here nothing is launched between iterations:
-//   records   every CTA reads all G selection records itself (one store -> poll hop), merges them and takes the
-//             decision of iteration k on its own copy of the log-det accumulator (CTA 0 writes the history entry and the
-//             control block), then gathers the chosen column
-//   u         rows cta + i G of Hinv times the column (warp per row), delivered as (value, token) words every CTA collects
-//   pass      a CTA owns q column blocks of W columns; warps 0-7 consume the ring (row groups and summation order of
-//             fw_pass_kernel: bit-identical w, x, vertex sequence), lane 0 of warp 8 feeds it and, towards the end of
-//             the pass, already issues the first stages of the NEXT iteration (V never changes), which land during the
-//             exchanges; warps 9-15 apply the rank-one update to the own rows of Hinv meanwhile
-//   record    of the updated columns, for the next decision
-constexpr int FWS_THREADS = 512;
-constexpr int FWS_CONS = 256;                           // consuming threads (warps 0-7)
-
-__device__ __forceinline__ void fwq_read_record(const double* src, unsigned long long token, int sleep_ns, FwCand& o) {
-    double f8[8];
-    unsigned done = 0;
-    unsigned long long t0 = 0;
-    unsigned spin = 0;
-    while (done != 0xffu) {                              // eight loads in flight; a word counts once it carries the token
-        unsigned long long v[8], tk[8];
-#pragma unroll
-        for (int e = 0; e < 8; ++e)
-            if (!(done & (1u << e)))
-                asm volatile("ld.volatile.global.v2.u64 {%0, %1}, [%2];" : "=l"(v[e]), "=l"(tk[e]) : "l"(src + 2 * e) : "memory");
-#pragma unroll
-        for (int e = 0; e < 8; ++e)
-            if (!(done & (1u << e)) && tk[e] == token) { f8[e] = __longlong_as_double((long long)v[e]); done |= 1u << e; }
-        if (done != 0xffu) {
-            __nanosleep(sleep_ns);
-            if ((++spin & 0x3ffu) == 0) {
-                unsigned long long now;
-                asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-                if (t0 == 0) t0 = now;
-                else if (now - t0 > 4000000000ULL) __trap();
-            }
-        }
-    }
-    o.amax = f8[0]; o.imax = __double_as_longlong(f8[1]);
-    o.smin = f8[2]; o.imin = __double_as_longlong(f8[3]); o.xmin = f8[4];
-    o.fmask = __double_as_longlong(f8[5]); o.wmask = f8[6]; o.xmask = f8[7];
-}
-
 __global__ void __launch_bounds__(FWS_THREADS, 1)
 fw_persist_ring_kernel(FwParams p, FwPersist q, const __grid_constant__ CUtensorMap tmV) {
     extern __shared__ __align__(128) unsigned char fws_raw[];      // ring [S][32 KB], then u, v, second v (mpad each)
@@ -1195,7 +682,7 @@ fw_persist_ring_kernel(FwParams p, FwPersist q, const __grid_constant__ CUtensor
     __shared__ double sh_logdet[2];
     __shared__ __align__(8) unsigned long long bar_mem[2 * FWR_MAX_STAGES];
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    const int m = p.m, S = p.ring_stages, G = q.G, cta = blockIdx.x;
+    const int m = p.m, S = q.stages, G = q.G, cta = blockIdx.x;
     const int mpad = (m + 1) / 2 * 2;
     const uint32_t ring = (uint32_t)__cvta_generic_to_shared(fws_raw);
     double* us = reinterpret_cast<double*>(fws_raw + (size_t)S * FWR_STAGE_BYTES);
@@ -1235,7 +722,7 @@ fw_persist_ring_kernel(FwParams p, FwPersist q, const __grid_constant__ CUtensor
         const int j0 = (cta + (p_rev ? nsub - 1 - p_sb : p_sb) * G) * W;
         if (p_use > 0) fwr_mbar_wait(bars + 8 * (FWR_MAX_STAGES + p_st), (uint32_t)((p_use + 1) & 1));
         fwr_mbar_expect(bars + 8 * p_st, stage_tx);
-        if (p.ring_3d) {
+        if (q.ring_3d) {
             fwr_tma_load_3d(ring + p_st * FWR_STAGE_BYTES, &tmV, j0, p_ch * FWR_ROWS, 0, bars + 8 * p_st);
         } else {
 #pragma unroll
@@ -1301,12 +788,9 @@ fw_persist_ring_kernel(FwParams p, FwPersist q, const __grid_constant__ CUtensor
         }
     };
     deliver_record(0);
-    unsigned long long ts[8];
-#define FWS_STAMP(i) do { if (q.dbg && tid == 0 && (cta < 2 || q.dbg == 3) && it == 5) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ts[i])); } while (0)
     for (int it = 0; it < q.k_count; ++it) {
         const int par = it & 1;
         const unsigned long long tokD = q.base + 4ULL * it, tokB = tokD + 2;
-        FWS_STAMP(0);
         // ---- every CTA gathers the G records itself and merges them (any order: the combines are total orders on
         //      (value, index)), then takes the decision of iteration k
         if (wid == 0) wait_flags(frec + (size_t)par * 256, tokD);
@@ -1323,7 +807,6 @@ fw_persist_ring_kernel(FwParams p, FwPersist q, const __grid_constant__ CUtensor
         fw_cand_block(cd, sh_c);                          // merged record in every lane of warp 0
         if (wid == 0 && lane == 0) sh_merged = cd;
         __syncthreads();
-        FWS_STAMP(1);
         // Thread 0 takes the decision (a few hundred dependent FP64 instructions) while the other warps fetch BOTH columns
         // the step rule can choose (argmax w, or the away vertex).  (Forming the own rows of u for both candidates under
         // the decision as well was measured slower: 17.7 k against 19.9 k iterations per second.)
@@ -1361,7 +844,6 @@ fw_persist_ring_kernel(FwParams p, FwPersist q, const __grid_constant__ CUtensor
         const double cs = sh_dec.cs, den = sh_dec.den, tsign = sh_dec.tsign;
         const int64_t idx = sh_dec.idx;
         const double* vc = (idx == sh_merged.imax) ? vs : vs2;      // (when both candidates coincide the columns are equal)
-        FWS_STAMP(2);
         // ---- u_r = Hinv[r,:] v for the own rows (warp per row, summation order of fw_hv_kernel), delivered to every CTA
         for (int i = wid; i < nown; i += FWS_THREADS / 32) {
             const int r = cta + i * G;
@@ -1383,11 +865,9 @@ fw_persist_ring_kernel(FwParams p, FwPersist q, const __grid_constant__ CUtensor
             sacc = warp_sum(sacc);
             if (lane == 0) fwq_st_pair(q.ux + ((size_t)par * m + r) * 2, sacc, tokB);
         }
-        FWS_STAMP(3);
         // (value, token) words: one hop; everybody waits here together, so the polling does not disturb a pass
         for (int r = tid; r < m; r += FWS_THREADS) us[r] = fwq_wait_pair(q.ux + ((size_t)par * m + r) * 2, tokB);
         __syncthreads();
-        FWS_STAMP(4);
         fw_cand_init(cd);
         if (tid < FWS_CONS) {
             // ---- the pass over the own column blocks
@@ -1471,14 +951,7 @@ fw_persist_ring_kernel(FwParams p, FwPersist q, const __grid_constant__ CUtensor
             c_st = adv % S;
         }
         __syncthreads();
-        FWS_STAMP(5);
         deliver_record(it + 1);
-        FWS_STAMP(6);
-        if (q.dbg == 3 && tid == 0 && it == 5 && q.dbg_buf)
-            for (int i = 0; i < 7; ++i) q.dbg_buf[cta * 8 + i] = ts[i];
-        if (q.dbg == 1 && tid == 0 && cta < 2 && it == 5)
-            printf("fw persistent ring cta %d: records %llu ns, decide + column %llu, u rows %llu, u gather %llu, pass %llu, record %llu | iteration %llu ns\n",
-                   cta, ts[1] - ts[0], ts[2] - ts[1], ts[3] - ts[2], ts[4] - ts[3], ts[5] - ts[4], ts[6] - ts[5], ts[6] - ts[0]);
     }
 }
 
@@ -1535,9 +1008,10 @@ size_t accbpg_fw_workspace_bytes(int m, int64_t n_local) {
     // dopt workspace (gram / factor / Linv / gradient partials) + v and u vectors
     size_t base = accbpg_dopt_workspace_bytes(m, n_local);
     const size_t nparts = (size_t)((n_local + 127) / 128) + 4096;        // selection candidates, one per selecting CTA
-    // + the exchange tables of the persistent loop: u parts (2 x m pairs), u (2 x m), records (2 x 256 CTAs x 128 B), tokens
-    return base + 2 * (((size_t)m + 31) / 32 * 32 * 8) + nparts * 64 + 256 + (size_t)6 * m * 8 + 2 * 256 * 128 + 2 * 16 * 128 + 512 +
-           4 * 256 * 8 /* flag words of the ring-fed persistent loop */ + 128;
+    // + the exchange tables of the persistent loop, each on a 128-byte boundary (accbpg_fw_run): u as (value, token)
+    //   pairs (2 x m), records (2 x 256 CTAs x 128 B), flag words (2 x 256)
+    return base + 2 * (((size_t)m + 31) / 32 * 32 * 8) + nparts * 64 + 128 + (size_t)4 * m * 8 + 128 + 2 * 256 * 128 +
+           2 * 256 * 8;
 }
 
 // D_opt_alg.py:39-45 / :123-129:  M = V diag(x0) V^T, Hinv = M^{-1}, w_j = v_j^T Hinv v_j, log det M
@@ -1571,11 +1045,6 @@ struct FwLaunch {
     int sel_grid, hv_grid, nblk, r1_ctas;
     size_t pass_smem;
     bool pass_vec;
-    bool ring_ok;              // the ring-fed kernels can run on this instance (tensor map encoded, shared memory fits)
-    bool use_ring;             // launch chain: fw_pass_ring_kernel (one CTA per SM, tensor-copy ring) instead of fw_pass_kernel
-    CUtensorMap tmV;           // V as a 2-D tensor, box = width columns x FWR_ROWS rows
-    int ring_grid;
-    size_t ring_smem;
     double* persist_mem;       // exchange tables of the persistent loop (inside the workspace)
 };
 
@@ -1620,124 +1089,21 @@ static int fw_prepare(Ctx* c, const double* V, int m, int64_t n, int64_t ldv, in
     p.V = V; p.m = m; p.n = n; p.ldv = ldv; p.x = x; p.w = w; p.Hinv = Hinv; p.u = u; p.v = v; p.ctrl = ctrl;
     p.hist_F = hist_F; p.hist_SP = hist_SP; p.hist_SN = hist_SN; p.hist_T = hist_T;
     p.parts = parts; p.counter = c->d_counter; p.away = away; p.eps = eps; p.nblk = L->nblk; p.nr1 = L->r1_ctas;
-    p.k = 0; p.decide = 0; p.reverse = 0; p.cand_out = nullptr; p.col_offset = 0; p.sharded = 0;
+    p.k = 0; p.decide = 0; p.reverse = 0; p.cand_out = nullptr; p.col_offset = 0; p.sharded = 0; p.early = FWP_EARLY;
     p.peer.world = 0; p.peer.rank = 0;
-    {
-        static int early = -1;                                // ACCBPG_FW_EARLY: rows per row group fetched before the wait
-        if (early < 0) { const char* e = getenv("ACCBPG_FW_EARLY"); early = e ? atoi(e) : 48; if (early < 0) early = 0; }
-        p.early = early;
-        static int ring = -1;                                 // ACCBPG_FW_RING=0: the register-fed pass kernel
-        if (ring < 0) {                                       // the launch chain keeps the register-fed pass unless asked:
-            const char* e = getenv("ACCBPG_FW_RING");         // 19.2 k against 17.7 k iterations per second at 500 x 50000
-            ring = (e && e[0] == '1') ? 1 : 0;
-        }
-        int max_optin = 0;
-        cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device);
-        const long long room = (long long)max_optin - FWR_STATIC_SMEM - (long long)m * 8;
-        int stages = room > 0 ? (int)(room / FWR_STAGE_BYTES) : 0;
-        if (stages > FWR_MAX_STAGES) stages = FWR_MAX_STAGES;
-        static int ring_w = -1;                               // ACCBPG_FW_RING_W: columns per block of the ring kernel
-        if (ring_w < 0) { const char* e = getenv("ACCBPG_FW_RING_W"); ring_w = e ? atoi(e) : 0; }
-        int64_t rw = width;
-        if (ring_w >= 16 && ring_w <= FWP_COLS && ring_w % 2 == 0) rw = ring_w;
-        L->ring_ok = L->pass_vec && (n % 2 == 0) && stages >= 3 && n < (1LL << 31) && !getenv("ACCBPG_FW_L2_MB");
-        p.ring_3d = 0;
-        if (L->ring_ok) {
-            static int no3d = -1;
-            if (no3d < 0) { const char* e = getenv("ACCBPG_FW_RING_3D"); no3d = (e && e[0] == '0') ? 1 : 0; }
-            // a box of FWR_ROWS x rw doubles must keep the 128-byte alignment of the next box when they are packed
-            if (m % 4 == 0 && !no3d && ((FWR_ROWS * rw * 8) % 128 == 0) &&
-                encode_tmap_f64_3d(&L->tmV, V, (uint64_t)n, (uint64_t)(m / 4), 4, (uint64_t)ldv, (uint32_t)rw, FWR_ROWS, 4))
-                p.ring_3d = 1;
-            else if (((FWR_ROWS * rw * 8) % 128 != 0) ||
-                     !encode_tmap_f64_2d(&L->tmV, V, (uint64_t)n, (uint64_t)m, (uint64_t)ldv, (uint32_t)rw, FWR_ROWS))
-                L->ring_ok = false;
-        }
-        L->use_ring = L->ring_ok && ring;
-        if (L->ring_ok && rw != width) {                       // (experiment) block width of the ring kernels
-            L->nblk = (int)((n + rw - 1) / rw);
-            p.nblk = L->nblk;
-            p.width = (int)rw;
-        }
-        p.ring_stages = L->use_ring ? stages : 0;
-        {
-            static int fdbg = -1;
-            if (fdbg < 0) { const char* e = getenv("ACCBPG_FW_DBG"); fdbg = e ? atoi(e) : 0; }
-            p.dbg = fdbg == 4;
-        }
-        L->ring_grid = L->nblk < c->sm_count ? L->nblk : c->sm_count;
-        L->ring_smem = (size_t)stages * FWR_STAGE_BYTES + (size_t)m * 8;
-        if (L->use_ring) {
-            static bool attr_done[kMaxDevices] = {};
-            if (c->device >= 0 && c->device < kMaxDevices && !attr_done[c->device]) {
-                ACCBPG_CUDA(cudaFuncSetAttribute(fw_pass_ring_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                 FWR_MAX_STAGES * FWR_STAGE_BYTES + 24 * 1024));
-                attr_done[c->device] = true;
-            }
-        }
-    }
     return ACCBPG_OK;
 }
 
-// L2 residency of V across iterations.  Every iteration streams all of V once; with 126 MB of L2 a pass over a 200 MB V
-// evicts itself.  The pass kernel is launched with an access-policy window over V whose hit ratio equals
-// (persisting L2 carve-out) / (bytes of V): that share of V's lines is kept resident from one iteration to the next, the
-// rest is streamed past them, so HBM serves only the non-resident share.  ACCBPG_FW_L2_MB: carve-out in MB.
-// OFF by default: measured at 500x50000 (tools/fw_l2_probe.py) the window costs 7 % (17.9 k against 19.2 k it/s) at every
-// hit ratio from 0.2 to 1.0 with the 79 MB maximum carve-out and is neutral at 32 MB - the pass at this size is bound
-// by requests in flight, not by DRAM bandwidth, and the two L2 partitions duplicate lines read from the far die.
-struct FwL2 { bool on; cudaAccessPolicyWindow win; };
-static FwL2 fw_l2_window(const double* V, int m, int64_t ldv) {
-    static int init = 0;
-    static size_t carve = 0, max_win = 0;
-    FwL2 r;
-    r.on = false;
-    if (!init) {
-        init = 1;
-        int dev = 0, max_persist = 0, max_window = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, dev);
-        cudaDeviceGetAttribute(&max_window, cudaDevAttrMaxAccessPolicyWindowSize, dev);
-        size_t want = 0;
-        const char* e = getenv("ACCBPG_FW_L2_MB");
-        if (e) { long mb = atol(e); want = mb <= 0 ? 0 : (size_t)mb << 20; if (want > (size_t)max_persist) want = (size_t)max_persist; }
-        if (want > 0 && max_window > 0 && cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want) == cudaSuccess) {
-            carve = want; max_win = (size_t)max_window;
-        }
-        (void)cudaGetLastError();
-        if (getenv("ACCBPG_VERBOSE"))
-            fprintf(stderr, "accbpg: FW L2 carve-out %zu MB (device max %d MB, window max %d MB)\n", carve >> 20,
-                    max_persist >> 20, max_window >> 20);
-    }
-    if (!carve) return r;
-    size_t bytes = (size_t)m * (size_t)ldv * sizeof(double);
-    if (bytes > max_win) bytes = max_win;
-    static float hit_env = -1.0f;
-    if (hit_env < 0.0f) { const char* e = getenv("ACCBPG_FW_L2_HIT"); hit_env = e ? (float)atof(e) : 0.0f; }
-    float ratio = hit_env > 0.0f ? hit_env : (float)((double)carve / (double)bytes);
-    if (ratio > 1.0f) ratio = 1.0f;
-    r.on = true;
-    r.win.base_ptr = (void*)V;
-    r.win.num_bytes = bytes;
-    r.win.hitRatio = ratio;
-    r.win.hitProp = cudaAccessPropertyPersisting;
-    r.win.missProp = cudaAccessPropertyStreaming;
-    return r;
-}
-
-// one pass launch (either kernel) on the configuration the caller prepared (stream, launch attributes)
+// one pass launch on the configuration the caller prepared (stream, launch attributes)
 static cudaError_t fw_launch_pass(const FwLaunch& L, cudaLaunchConfig_t cfg, const FwParams& p) {
-    if (L.use_ring) {
-        cfg.gridDim = dim3(L.ring_grid); cfg.blockDim = dim3(FWR_THREADS); cfg.dynamicSmemBytes = L.ring_smem;
-        return cudaLaunchKernelEx(&cfg, fw_pass_ring_kernel, p, L.tmV);
-    }
     cfg.gridDim = dim3(L.nblk + L.r1_ctas); cfg.blockDim = dim3(FWP_THREADS); cfg.dynamicSmemBytes = L.pass_smem;
     return cudaLaunchKernelEx(&cfg, L.pass_vec ? fw_pass_kernel<true> : fw_pass_kernel<false>, p);
 }
 
-// run iterations k_start .. k_start+k_count-1 (no-ops after the stop flag is raised):
+// run iterations k_start .. k_start+k_count-1 (no-ops after the stop flag is raised), as one persistent launch when the
+// ring of fw_persist_ring_kernel can run on this instance, else as the launch chain
 //   select+decide(k_start);  then per iteration  u = Hinv v;  pass (+ rank-one update of Hinv, + decision of k+1)
-// Launches are chained with programmatic dependent launch.
+// chained with programmatic dependent launch.
 int accbpg_fw_run(void* ctx, void* stream, const double* V, int m, int64_t n, int64_t ldv, int away, double eps,
                   int k_start, int k_count, void* ws, double* Hinv, double* x, double* w, double* ctrl,
                   double* hist_F, double* hist_SP, double* hist_SN, double* hist_T) {
@@ -1752,12 +1118,9 @@ int accbpg_fw_run(void* ctx, void* stream, const double* V, int m, int64_t n, in
     int rc = fw_prepare(c, V, m, n, ldv, away, eps, ws, Hinv, x, w, ctrl, hist_F, hist_SP, hist_SN, hist_T, &L);
     if (rc) return rc;
     FwParams& p = L.p;
-    cudaLaunchAttribute attr[2];
+    cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
-    const FwL2 l2 = fw_l2_window(V, m, ldv);
-    if (l2.on) { attr[1].id = cudaLaunchAttributeAccessPolicyWindow; attr[1].val.accessPolicyWindow = l2.win; }
-    const int pass_attrs = l2.on ? 2 : 1;
     cudaLaunchConfig_t cfg = {};
     cfg.stream = s;
     cfg.attrs = attr;
@@ -1770,130 +1133,50 @@ int accbpg_fw_run(void* ctx, void* stream, const double* V, int m, int64_t n, in
         fw_zero_lo_kernel<<<1, 1, 0, s>>>(ctrl);
         ACCBPG_LAUNCHED("fw_zero_lo_kernel");
     }
-    // ---- one persistent launch for the whole batch: OPT-IN (ACCBPG_FW_PERSIST=1).  Results are bit-identical to the launch
-    //      chain below (tests/test_gpu_fw.py passes either way), but at 500 x 50000 it reaches 11-14 k iterations per second
-    //      against 19.2 k: its exchanges (records -> merge -> replicas, u all-gather) cost 13 us per iteration and a
-    //      statically partitioned CTA streams its strip of V at 3.0-4.9 TB/s only (DESIGN.md, tried and dropped)
-    {
-        static int persist = -1;                              // unset: ring-fed persistent loop when it can run; 0: launch chain;
-        if (persist < 0) {                                    // 1: a persistent loop in any case (register-fed without the ring)
-            const char* e = getenv("ACCBPG_FW_PERSIST");
-            persist = !e ? 2 : (e[0] == '1' ? 1 : 0);
-        }
-        const int G = c->sm_count < 256 ? c->sm_count : 256;
-        int64_t per = (n + G - 1) / G;
-        per = (per + 1) / 2 * 2;
+    // ---- one persistent launch for the whole batch when V is 16-byte aligned with even n and ldv, n < 2^31, m <= 4096,
+    //      at least three ring stages fit in shared memory next to u and the two candidate columns, and the tensor map
+    //      of V encodes
+    if (L.pass_vec && n % 2 == 0 && n < (1LL << 31) && m <= 4096) {
         const int mpad = (m + 1) / 2 * 2;
-        if (persist && L.ring_ok && !l2.on && m <= 4096) {
-            // the ring-fed form: q column blocks of W = p.width columns per CTA
-            int max_optin = 0;
-            cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device);
-            const long long room = (long long)max_optin - FWR_STATIC_SMEM - 3LL * mpad * 8;
-            int stages = room > 0 ? (int)(room / FWR_STAGE_BYTES) : 0;
-            if (stages > FWR_MAX_STAGES) stages = FWR_MAX_STAGES;
-            if (stages >= 3) {
-                static bool attr_done[kMaxDevices] = {};
-                if (c->device >= 0 && c->device < kMaxDevices && !attr_done[c->device]) {
-                    ACCBPG_CUDA(cudaFuncSetAttribute(fw_persist_ring_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                     max_optin - FWR_STATIC_SMEM));
-                    attr_done[c->device] = true;
-                }
-                FwPersist q;
-                q.ux = L.persist_mem;
-                q.recs = q.ux + (size_t)4 * m;
-                q.recs = reinterpret_cast<double*>((reinterpret_cast<uintptr_t>(q.recs) + 127) / 128 * 128);
-                q.bcast = q.recs + (size_t)2 * 256 * FWQ_REC_DOUBLES;
-                q.tok = reinterpret_cast<unsigned long long*>(
-                    (reinterpret_cast<uintptr_t>(q.bcast + (size_t)2 * FWQ_REPL * FWQ_REC_DOUBLES) + 127) / 128 * 128);
-                static unsigned long long calls_r = 0;
-                q.base = ((++calls_r) << 24) | (1ULL << 62);  // never a token of the other persistent kernel
-                q.G = G; q.k_start = k_start; q.k_count = k_count; q.per = 0; q.rc4 = 0;
-                static int fdbg = -1;
-                if (fdbg < 0) { const char* e = getenv("ACCBPG_FW_DBG"); fdbg = e ? atoi(e) : 0; }
-                q.dbg = (fdbg == 1 || fdbg == 3) ? fdbg : 0;
-                q.dbg_buf = nullptr;
-                static unsigned long long* dbg_dev = nullptr;
-                if (fdbg == 3) {
-                    if (!dbg_dev) cudaMalloc(&dbg_dev, 256 * 8 * 8);
-                    cudaMemsetAsync(dbg_dev, 0, 256 * 8 * 8, s);
-                    q.dbg_buf = dbg_dev;
-                }
-                p.k = k_start; p.decide = 1; p.reverse = 0; p.ring_stages = stages;
-                const size_t smem = (size_t)stages * FWR_STAGE_BYTES + (size_t)3 * mpad * 8;
-                ProfScope ps(P_FW_BATCH, s);
-                fw_persist_ring_kernel<<<G, FWS_THREADS, smem, s>>>(p, q, L.tmV);
-                ACCBPG_LAUNCHED("fw_persist_ring_kernel");
-                if (fdbg == 3 && k_count > 6) {              // timing experiment only: per-CTA stamps of batch iteration 5
-                    static unsigned long long h[256 * 8];
-                    cudaStreamSynchronize(s);
-                    cudaMemcpy(h, dbg_dev, sizeof(h), cudaMemcpyDeviceToHost);
-                    unsigned long long t0 = ~0ULL;
-                    for (int b = 0; b < G; ++b) if (h[b * 8] && h[b * 8] < t0) t0 = h[b * 8];
-                    const char* nm[7] = {"loop top", "records merged", "decided + column", "own u rows sent", "u gathered", "pass done",
-                                         "record posted"};
-                    for (int i = 0; i < 7; ++i) {
-                        unsigned long long lo = ~0ULL, hi = 0; int amax = 0, amin = 0;
-                        for (int b = 0; b < G; ++b) {
-                            unsigned long long v = h[b * 8 + i] - t0;
-                            if (v < lo) { lo = v; amin = b; }
-                            if (v > hi) { hi = v; amax = b; }
-                        }
-                        fprintf(stderr, "[fw ring dbg] %-18s min %7llu ns (cta %d)  max %7llu ns (cta %d)\n", nm[i], lo, amin, hi, amax);
-                    }
-                }
-                return ACCBPG_OK;
+        int max_optin = 0;
+        cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device);
+        const long long room = (long long)max_optin - FWR_STATIC_SMEM - 3LL * mpad * 8;
+        int stages = room > 0 ? (int)(room / FWR_STAGE_BYTES) : 0;
+        if (stages > FWR_MAX_STAGES) stages = FWR_MAX_STAGES;
+        // V in boxes of p.width columns x FWR_ROWS rows; p.width is even, so boxes packed in a stage stay 128-byte aligned
+        CUtensorMap tmV;
+        int ring_3d = 0;
+        bool tmap = false;
+        if (stages >= 3) {
+            // one box over (columns, rows of a group, row groups) per stage when 4 | m, else one box per row group
+            if (m % 4 == 0 &&
+                encode_tmap_f64_3d(&tmV, V, (uint64_t)n, (uint64_t)(m / 4), 4, (uint64_t)ldv, (uint32_t)p.width, FWR_ROWS, 4)) {
+                ring_3d = 1;
+                tmap = true;
+            } else {
+                tmap = encode_tmap_f64_2d(&tmV, V, (uint64_t)n, (uint64_t)m, (uint64_t)ldv, (uint32_t)p.width, FWR_ROWS);
             }
         }
-        const size_t fixed = ((size_t)2 * mpad + 2 * 4 * FWP_COLS) * sizeof(double);
-        const size_t budget = 200 * 1024;
-        if (persist == 1 && L.pass_vec && !l2.on && m <= 4096 && per >= 2 && per < (1 << 28) && fixed + 1024 < budget) {
-            const int rows_per = (m + 3) / 4;
-            int64_t rc4 = (int64_t)((budget - fixed) / ((size_t)32 * per));
-            if (rc4 > rows_per) rc4 = rows_per;
-            if (rc4 < 0) rc4 = 0;
-            const size_t smem = fixed + (size_t)4 * rc4 * per * sizeof(double);
+        if (tmap) {
             static bool attr_done[kMaxDevices] = {};
             if (c->device >= 0 && c->device < kMaxDevices && !attr_done[c->device]) {
-                ACCBPG_CUDA(cudaFuncSetAttribute(fw_persistent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 201 * 1024));
+                ACCBPG_CUDA(cudaFuncSetAttribute(fw_persist_ring_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                 max_optin - FWR_STATIC_SMEM));
                 attr_done[c->device] = true;
             }
             FwPersist q;
             q.ux = L.persist_mem;
-            q.recs = q.ux + (size_t)4 * m;
-            q.recs = reinterpret_cast<double*>((reinterpret_cast<uintptr_t>(q.recs) + 127) / 128 * 128);
-            q.bcast = q.recs + (size_t)2 * 256 * FWQ_REC_DOUBLES;
-            q.tok = nullptr;
+            q.recs = reinterpret_cast<double*>((reinterpret_cast<uintptr_t>(q.ux + (size_t)4 * m) + 127) / 128 * 128);
+            q.tok = reinterpret_cast<unsigned long long*>(q.recs + (size_t)2 * 256 * FWQ_REC_DOUBLES);
             static unsigned long long calls = 0;
             q.base = (++calls) << 24;
-            q.G = G; q.k_start = k_start; q.k_count = k_count; q.per = (int)per; q.rc4 = (int)rc4;
-            static int fdbg = -1;
-            if (fdbg < 0) { const char* e = getenv("ACCBPG_FW_DBG"); fdbg = e ? atoi(e) : 0; }
-            q.dbg = fdbg;
-            q.dbg_buf = nullptr;
-            static unsigned long long* dbg_dev = nullptr;
-            if (fdbg == 3) {
-                if (!dbg_dev) { cudaMalloc(&dbg_dev, 256 * 8 * 8); }
-                cudaMemsetAsync(dbg_dev, 0, 256 * 8 * 8, s);
-                q.dbg_buf = dbg_dev;
-            }
+            q.G = c->sm_count < 256 ? c->sm_count : 256;
+            q.k_start = k_start; q.k_count = k_count; q.stages = stages; q.ring_3d = ring_3d;
             p.k = k_start; p.decide = 1; p.reverse = 0;
+            const size_t smem = (size_t)stages * FWR_STAGE_BYTES + (size_t)3 * mpad * 8;
             ProfScope ps(P_FW_BATCH, s);
-            fw_persistent_kernel<<<G, FWQ_THREADS, smem, s>>>(p, q);
-            ACCBPG_LAUNCHED("fw_persistent_kernel");
-            if (fdbg == 3 && k_count > 6) {              // timing experiment only: per-CTA stamps of batch iteration 5
-                static unsigned long long h[256 * 8];
-                cudaStreamSynchronize(s);
-                cudaMemcpy(h, dbg_dev, sizeof(h), cudaMemcpyDeviceToHost);
-                unsigned long long t0 = ~0ULL;
-                for (int b = 0; b < G; ++b) if (h[b * 8] && h[b * 8] < t0) t0 = h[b * 8];
-                const char* nm[8] = {"loop top", "records gathered", "decided + column", "u rows sent", "u gathered", "Hinv rows done",
-                                     "pass done", "record posted"};
-                for (int i = 0; i < 8; ++i) {
-                    unsigned long long lo = ~0ULL, hi = 0; int amax = 0;
-                    for (int b = 0; b < G; ++b) { unsigned long long v = h[b * 8 + i] - t0; if (v < lo) lo = v; if (v > hi) { hi = v; amax = b; } }
-                    fprintf(stderr, "[fw dbg] %-18s min %7llu ns  max %7llu ns (cta %d)\n", nm[i], lo, hi, amax);
-                }
-            }
+            fw_persist_ring_kernel<<<q.G, FWS_THREADS, smem, s>>>(p, q, tmV);
+            ACCBPG_LAUNCHED("fw_persist_ring_kernel");
             return ACCBPG_OK;
         }
     }
@@ -1911,7 +1194,6 @@ int accbpg_fw_run(void* ctx, void* stream, const double* V, int m, int64_t n, in
         p.k = k + 1;                                        // the tail decides the next iteration ...
         p.decide = (k + 1 < k_start + k_count) ? 1 : 0;     // ... except after the last pass of the batch
         p.reverse = k & 1;
-        cfg.numAttrs = pass_attrs;
         {
             ProfScope ps(P_FW_PASS, s);
             ACCBPG_CUDA(fw_launch_pass(L, cfg, p));
@@ -2080,11 +1362,6 @@ int accbpg_fw_setup_from_gram(void* ctx, void* stream, const double* V, int m, i
     fw_hinv_kernel<<<grid, 256, 0, s>>>(Linv, m, mp, Hinv);
     ACCBPG_LAUNCHED("fw_hinv_kernel");
     return ACCBPG_OK;
-}
-
-// timing experiment: the stamps of two consecutive fw_pass_ring_kernel launches (8 per CTA, 2 x 256 CTAs at most)
-int accbpg_fw_debug_stamps(unsigned long long* host_out) {
-    return cudaMemcpyFromSymbol(host_out, g_fwr_dbg, sizeof(unsigned long long) * 512 * 8) == cudaSuccess ? 0 : -1;
 }
 
 }  // extern "C"

@@ -36,7 +36,7 @@
 extern "C" {
 #endif
 
-#define ACCBPG_ABI_VERSION 5
+#define ACCBPG_ABI_VERSION 6
 
 /* return codes */
 #define ACCBPG_OK      0
@@ -381,10 +381,11 @@ int accbpg_fw_setup(void* ctx, void* stream, const double* d_V, int m, int64_t n
                     const double* d_x0, void* d_ws, double* d_Hinv, double* d_w, double* d_ctrl);
 /* enqueue iterations k_start .. k_start+k_count-1 of the loop (:51-82 / :135-179): argmax w; masked argmin + step
  * rule + history entry + gather of the chosen column; u = Hinv v; Hinv <- (Hinv -/+ c u u^T)/(1 -/+ t); the single
- * pass over V that forms u^T V and updates w and x.  When V is 16-byte aligned with even n and ldv this is ONE
+ * pass over V that forms u^T V and updates w and x.  When V is 16-byte aligned with even n and ldv, n < 2^31,
+ * m <= 4096 and at least three 32 KB ring stages fit in shared memory next to three vectors of m doubles, this is ONE
  * persistent launch for the whole batch (one CTA per SM; the pass is fed by tensor copies into a shared-memory
  * ring, decisions and u are exchanged between the CTAs); otherwise two launches per iteration chained by
- * programmatic dependent launch.  Same bits either way (ACCBPG_FW_PERSIST=0 forces the launch chain).
+ * programmatic dependent launch.  Same bits either way.
  * away = 0: D_opt_FW, 1: D_opt_FW_away.  Once the optimality test fires (ctrl[0] = 1, ctrl[1] = k) the
  * remaining iterations are not executed; ctrl[14] counts the history entries written. */
 int accbpg_fw_run(void* ctx, void* stream, const double* d_V, int m, int64_t n, int64_t ldv, int away, double eps,

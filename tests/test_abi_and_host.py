@@ -43,9 +43,9 @@ def test_library_is_sm100a_with_dmma():
     assert tma.count("DMMA.8x8x4") >= 64 and "UTMALDG" in tma and "SYNCS" in tma
 
 
-def test_frank_wolfe_ring_kernels_are_tma_fed():
-    """The ring-fed Frank-Wolfe kernels stream V with tensor copies signalled on mbarriers (UTMALDG + SYNCS), the
-    persistent one also releases / acquires its flag words at GPU scope."""
+def test_frank_wolfe_persistent_loop_is_tma_fed():
+    """The persistent Frank-Wolfe loop streams V with tensor copies (3-D and 2-D) signalled on mbarriers (UTMALDG +
+    SYNCS) and releases / acquires its flag words at GPU scope."""
     from accbpg_and_fw_b200 import _native as nat
     sass = subprocess.run(["cuobjdump", "-sass", nat.LIB_PATH], capture_output=True, text=True).stdout
     funcs, cur = {}, None
@@ -61,10 +61,8 @@ def test_frank_wolfe_ring_kernels_are_tma_fed():
         assert hits, substr
         return "\n".join(funcs[hits[0]])
 
-    for k in ("fw_persist_ring_kernel", "fw_pass_ring_kernel"):
-        b = body(k)
-        assert "UTMALDG.3D" in b and "UTMALDG.2D" in b and "SYNCS" in b, k
     b = body("fw_persist_ring_kernel")
+    assert "UTMALDG.3D" in b and "UTMALDG.2D" in b and "SYNCS" in b
     assert re.search(r"ST\w*\.E\.64\.STRONG\.GPU", b) and re.search(r"LD\w*\.E\.64\.STRONG\.GPU", b)
 
 

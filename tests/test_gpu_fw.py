@@ -1,5 +1,7 @@
 """GPU parity: D_opt_FW / D_opt_FW_away (device-resident loop) against the oracle and the golden runs.
 F_k, the slacks SP/SN and the selected vertex indices; the FW vertex index must be bit-exact."""
+import hashlib
+
 import numpy as np
 import torch
 import pytest
@@ -174,45 +176,69 @@ def test_sharded_fw_building_blocks_on_one_gpu(acc, away, world):
         assert torch.equal(ctrl[r][:15], ctrl[0][:15]) and torch.equal(Hinv[r], Hinv[0])
 
 
-_FW_PATHS_SCRIPT = r"""
-import hashlib, sys, numpy as np
-sys.path.insert(0, {root!r})
-import accbpg_and_fw_b200 as acc
-out = []
-for (m, n, seed, eps, its, batch) in [(200, 5000, 2, 1e-8, 200, 64), (64, 3000, 5, 1e-2, 4000, 32), (10, 40, 4, 1e-3, 5000, 16)]:
-    np.random.seed(seed)
-    V = np.random.randn(m, n)
-    x0 = np.ones(n) / n
-    for fn in (acc.D_opt_FW_away, acc.D_opt_FW):
-        x, F, SP, SN, T = fn(V, x0, eps, its, verbose=False, batch=batch)
-        h = hashlib.sha256()
-        for a in (x, F, SP, SN):
-            h.update(np.ascontiguousarray(a).tobytes())
-        out.append(f"{{len(F)}}:{{h.hexdigest()[:16]}}")
-print("FWHASH " + " ".join(out))
-"""
+def _fw_loop(acc, V, start, away, eps, its, batch):
+    """The batches of D_opt_FW (away = 0) / D_opt_FW_away (away = 1) as dopt_fw drives them, on V as given, from a copy
+    of the set-up state `start` = (workspace, x, Hinv, w, ctrl).  Returns ((history length, sha256 of x, F, SP, SN),
+    kernels the loop launched)."""
+    from accbpg_and_fw_b200 import _native as nat
+    from accbpg_and_fw_b200.dopt_fw import C_NITER, C_STOP
+    lib, rt = nat.lib, acc.Runtime.get()
+    m, n = V.shape
+    ws = start[0]
+    x, Hinv, w, ctrl = (t.clone() for t in start[1:])
+    hist = torch.zeros(4, its, dtype=torch.float64, device="cuda")
+    before = nat.launch_count()
+    k = 0
+    while k < its:
+        cnt = min(batch, its - k)
+        nat.check(lib.accbpg_fw_run(rt.ctx, rt.stream, V.data_ptr(), m, n, n, away, eps, k, cnt, ws.data_ptr(),
+                                    Hinv.data_ptr(), x.data_ptr(), w.data_ptr(), ctrl.data_ptr(), hist[0].data_ptr(),
+                                    hist[1].data_ptr(), hist[2].data_ptr(), hist[3].data_ptr()))
+        k += cnt
+        if ctrl.cpu().numpy()[C_STOP] != 0:
+            break
+    launches = nat.launch_count() - before
+    done = int(ctrl.cpu().numpy()[C_NITER])
+    h = hashlib.sha256()
+    for a in (x, hist[0, :done], hist[1, :done], hist[2, :done]):
+        h.update(a.cpu().numpy().tobytes())
+    return (done, h.hexdigest()), launches
 
 
-def test_fw_paths_bit_identical():
-    """The three forms of the loop - ring-fed persistent launch (default on one GPU), launch chain with the register-fed
-    pass, launch chain with the ring-fed pass - give the same bits (iterates, histories, stopping iteration).  The
-    switches are read once per process, hence the subprocesses."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    res = {}
-    for name, env in (("persistent ring", {}), ("chain", {"ACCBPG_FW_PERSIST": "0"}),
-                      ("chain + ring pass", {"ACCBPG_FW_PERSIST": "0", "ACCBPG_FW_RING": "1"}),
-                      ("chain, nothing before the wait", {"ACCBPG_FW_PERSIST": "0", "ACCBPG_FW_EARLY": "0"})):
-        e = dict(os.environ)
-        for k in ("ACCBPG_FW_PERSIST", "ACCBPG_FW_RING", "ACCBPG_FW_EARLY"):
-            e.pop(k, None)
-        e.update(env)
-        r = subprocess.run([sys.executable, "-c", _FW_PATHS_SCRIPT.format(root=root)], env=e, capture_output=True,
-                           text=True, timeout=600)
-        assert r.returncode == 0, (name, r.stderr[-2000:])
-        line = [ln for ln in r.stdout.splitlines() if ln.startswith("FWHASH ")]
-        assert line, (name, r.stdout[-500:])
-        res[name] = line[-1]
-    assert len(set(res.values())) == 1, res
+def test_fw_paths_bit_identical(acc):
+    """The two forms of the loop, each reached by its input, give the same bits (iterates, histories, stopping
+    iteration) from the same set-up state.  m <= 4096: V contiguous runs the ring-fed persistent launch (one 3-D tensor
+    copy per stage when 4 | m, four 2-D copies otherwise), the same values 8 bytes into a buffer (not 16-byte aligned)
+    run the launch chain with the scalar-load pass.  m > 4096: V contiguous runs the launch chain with the vector-load
+    pass and its early fetch, the offset copy the chain with the scalar-load pass."""
+    from accbpg_and_fw_b200 import _native as nat
+    from accbpg_and_fw_b200.dopt_fw import NCTRL
+    lib, rt = nat.lib, acc.Runtime.get()
+    for (m, n, seed, eps, its, batch) in [(200, 5000, 2, 1e-8, 200, 64), (64, 3000, 5, 1e-2, 4000, 32),
+                                          (10, 40, 4, 1e-3, 5000, 16), (4100, 4200, 7, 1e-12, 40, 16)]:
+        np.random.seed(seed)
+        V = np.random.randn(m, n)
+        Va = torch.tensor(V, device="cuda")
+        buf = torch.empty(m * n + 1, dtype=torch.float64, device="cuda")
+        Vo = buf[1:].view(m, n)
+        Vo.copy_(Va)
+        assert Va.data_ptr() % 16 == 0 and Vo.data_ptr() % 16 == 8 and Vo.is_contiguous()
+        ws = torch.zeros(lib.accbpg_fw_workspace_bytes(m, n), dtype=torch.uint8, device="cuda")
+        x = torch.full((n,), 1.0 / n, dtype=torch.float64, device="cuda")
+        Hinv = torch.empty(m, m, dtype=torch.float64, device="cuda")
+        w = torch.empty(n, dtype=torch.float64, device="cuda")
+        ctrl = torch.zeros(NCTRL, dtype=torch.float64, device="cuda")
+        nat.check(lib.accbpg_fw_setup(rt.ctx, rt.stream, Va.data_ptr(), m, n, n, x.data_ptr(), ws.data_ptr(),
+                                      Hinv.data_ptr(), w.data_ptr(), ctrl.data_ptr()))
+        rt.read(0, 0)
+        start = (ws, x, Hinv, w, ctrl)
+        for away in (1, 0):
+            aligned, launches_aligned = _fw_loop(acc, Va, start, away, eps, its, batch)
+            offset, launches_offset = _fw_loop(acc, Vo, start, away, eps, its, batch)
+            assert aligned == offset, (m, n, away, aligned, offset)
+            done = aligned[0]
+            assert launches_offset >= 2 * done                          # the launch chain: two launches per iteration
+            if m <= 4096:
+                assert launches_offset - launches_aligned >= 2 * done   # the persistent loop: one launch per batch
+            else:
+                assert launches_aligned == launches_offset

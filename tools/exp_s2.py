@@ -5,7 +5,6 @@ import os, sys, time
 import numpy as np, torch
 sys.path.insert(0, ".")
 import accbpg_and_fw_b200 as acc
-from accbpg_and_fw_b200 import _native as nat
 
 what = sys.argv[1] if len(sys.argv) > 1 else "all"
 tag = " ".join(f"{k}={v}" for k, v in sorted(os.environ.items()) if k.startswith("ACCBPG_"))
@@ -45,25 +44,6 @@ if what in ("abpg", "all"):
         torch.cuda.synchronize()
         best = min(best, (time.perf_counter() - t0) / 200)
     print(f"[abpg] {tag} ms/it {best * 1e3:.4f} F_last {F[-1]!r}", flush=True)
-
-if what == "stamps":
-    import ctypes
-    acc.D_opt_FW_away(f._Hd, x0d, 1e-12, 200, verbose=False)
-    torch.cuda.synchronize()
-    buf = (ctypes.c_ulonglong * (512 * 8))()
-    nat.lib.accbpg_fw_debug_stamps.argtypes = [ctypes.c_void_p]
-    assert nat.lib.accbpg_fw_debug_stamps(buf) == 0
-    a = np.array(buf[:], dtype=np.int64).reshape(512, 8)
-    G = int((a[:255, 0] > 0).sum())
-    t0 = a[:G, 0].min()
-    names = ["entry", "after wait", "first stage full", "streaming done", "decision done"]
-    print(f"[stamps] {tag} G={G}  (ns after the first CTA of pass A entered)")
-    for which, base in (("pass A", 0), ("pass B", 256)):
-        for i, nm in enumerate(names):
-            v = a[base:base + G, i]
-            v = v[v > 0] - t0
-            if v.size:
-                print(f"   {which} {nm:18s} min {v.min():7d}  median {int(np.median(v)):7d}  max {v.max():7d}  (n={v.size})")
 
 if what == "fwc5":
     # D_opt_FW_away at 2000 x 1e6 (device-generated): iterations per second and a bit comparison between settings

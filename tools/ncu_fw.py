@@ -1,4 +1,4 @@
-"""ncu target: a few D_opt_FW_away iterations at 500 x 50000 (the pass over V); ACCBPG_FW_RING selects the kernel."""
+"""ncu target: a few D_opt_FW_away iterations at 500 x 50000 (one launch of the persistent loop, fw_persist_ring_kernel)."""
 import os, sys
 import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
