@@ -35,6 +35,11 @@ fused_small
     its own that holds more vectors) when linear_images is also on: the kernel follows that scheme - carried A x and
     A z, A x re-formed every `reanchor_every` iterations - so results differ from the operator loop only in the order
     of sums.  With linear_images off the operator loop evaluates every point from scratch, as that switch says.
+    ABPG and ABPG_gain on the D-optimal design objective with BurgEntropySimplex run as one launch as well
+    (accbpg_dopt_abpg_small, on the machinery of the BPG kernel with three more vectors) when H fits.  That kernel
+    evaluates every point from scratch, which is what linear_images = False asks for, and the carried Gram images agree
+    with it to rounding, so it is taken under both settings of linear_images.  SparseDOptimalObj stays on the operator
+    loop.
 """
 linear_images = True
 reanchor_every = 64

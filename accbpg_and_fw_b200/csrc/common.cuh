@@ -172,6 +172,34 @@ __device__ __forceinline__ bool last_block_ticket(unsigned int* counter, bool* s
 
 __device__ __forceinline__ double ld_cg(const double* p) { return __ldcg(p); }
 
+// ---- scalar control of the one-launch accelerated solves (linreg_small.cu, small.cu).  Written with explicit
+//      round-to-nearest operations: the two files are compiled with and without FMA contraction, and these values must
+//      round like the host's Python arithmetic in both.
+__device__ __forceinline__ unsigned long long ls_clock() {
+    unsigned long long ns;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns));
+    return ns;
+}
+
+// x**y.  The host's pow is correctly rounded at these exponents and CUDA's may be 2 ulp off; theta**gamma decides the
+// gain line search and the G / Gain histories that the golden runs compare exactly (gamma = 2), so the exponents 1 and
+// 2 take the exact forms.
+__device__ __forceinline__ double la_pow(double x, double y) {
+    return y == 1.0 ? x : y == 2.0 ? __dmul_rn(x, x) : pow(x, y);
+}
+
+// solve_theta: Newton solve of (1-t)/t^gamma = gainratio/theta^gamma from theta   (drivers.py, algorithms.py:75-91)
+__device__ inline double la_solve_theta(double theta, double gamma, double gainratio) {
+    const double ckg = __ddiv_rn(la_pow(theta, gamma), gainratio);
+    double cta = theta;
+    const double tol = __dmul_rn(1e-6, theta);
+    for (;;) {
+        const double phi = __dsub_rn(la_pow(cta, gamma), __dmul_rn(ckg, __dsub_rn(1.0, cta)));
+        if (!(fabs(phi) > tol)) return cta;
+        cta = __dsub_rn(cta, __ddiv_rn(phi, __dadd_rn(__dmul_rn(gamma, la_pow(cta, __dsub_rn(gamma, 1.0))), ckg)));
+    }
+}
+
 // ---- flag words in NVLink peer memory (symmetric buffers mapped into every rank) ----
 // A sender stores its payload into the receiver's buffer, fences at system scope and releases a monotonically increasing
 // epoch into its flag word on the receiver; the receiver acquires the word before touching the payload.

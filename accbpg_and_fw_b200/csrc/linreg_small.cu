@@ -406,12 +406,6 @@ __device__ __forceinline__ double ls_psi(const LsParams& p, const double (&sc)[L
     return 0.0;
 }
 
-__device__ __forceinline__ unsigned long long ls_clock() {
-    unsigned long long ns;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns));
-    return ns;
-}
-
 // ---- rank, column slice and the split of the matrix passes, for NL columns per CTA (the buffers are the caller's)
 template <int C>
 __device__ __forceinline__ void ls_split(LsCtx& c, const LsParams& p, int NL) {
@@ -523,25 +517,6 @@ struct LaParams : LsParams {
     double* hist;                    // rows of maxitrs: F, G / Gain, Gdiv, theta, D(x,y), D(z,z-), T
     // info: [0] entries written, [1] trips, [2] cluster size, [3] Gdr unbound, [4] last G / gain
 };
-
-// x**y for the scalar control.  The host's pow is correctly rounded at these exponents and CUDA's may be 2 ulp off;
-// theta**gamma decides the gain line search and the G / Gain histories that the golden runs compare exactly (gamma = 2),
-// so the exponents 1 and 2 take the exact forms.
-__device__ __forceinline__ double la_pow(double x, double y) {
-    return y == 1.0 ? x : y == 2.0 ? x * x : pow(x, y);
-}
-
-// solve_theta: Newton solve of (1-t)/t^gamma = gainratio/theta^gamma from theta   (drivers.py, algorithms.py:75-91)
-__device__ double la_solve_theta(double theta, double gamma, double gainratio) {
-    const double ckg = la_pow(theta, gamma) / gainratio;
-    double cta = theta;
-    const double tol = 1e-6 * theta;
-    for (;;) {
-        const double phi = la_pow(cta, gamma) - ckg * (1 - cta);
-        if (!(fabs(phi) > tol)) return cta;
-        cta = cta - phi / (gamma * la_pow(cta, gamma - 1) + ckg);
-    }
-}
 
 // Every iteration of the operator loop's default scheme (config.linear_images): the images A x- and A z- are carried,
 // A y and A x are combinations of them, A z is one matvec per trip and A x is re-formed from x every reanchor

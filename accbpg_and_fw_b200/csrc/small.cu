@@ -16,6 +16,11 @@
 //                                    refilled from global memory (L2) by cp.async under the prox   (functions.py:52-58)
 //   prox      Burg-simplex root-find (functions.py:341-356) with the CTA-wide sums of a Newton step in one barrier
 //   test      f(x+) > f(x) + <g, x+ - x> + L D(x+, x)  ->  L *= ls_ratio                      (algorithms.py:46-56)
+//
+// dopt_abpg_small_kernel<C, DRV> runs ABPG (algorithms.py:94-180) or ABPG_gain (:295-420) on the same functions, in a
+// plan with three more vectors, evaluating every point from scratch (see the kernel).  On a B200 at a 1000 W power
+// limit (profiles/dopt_small_accel_r01.json): ABPG 20.8 k it/s and ABPG_gain 9.6 k it/s at 80 x 200, 2.6x and 4.0x the
+// operator-by-operator loop (DESIGN.md section 9).
 #include <cooperative_groups.h>
 
 #include "dmma.cuh"
@@ -26,15 +31,17 @@ constexpr int SM_THREADS = 512;
 constexpr int SM_WARPS = SM_THREADS / 32;
 constexpr int SM_MAX_M = 128;
 constexpr int SM_SMEM_LIMIT = 220 * 1024;
+constexpr int SM_ACC_SUMS = 5;                 // values of dopt_abpg_small_kernel's CTA-wide sum of a trip
 #define kInf (__longlong_as_double(0x7ff0000000000000LL))
 
 struct SmallPlan {
     int MP, NP, NL, ldn, lda, nblk16;
-    size_t off_H, off_A, off_part, off_x, off_x1, off_g, off_d, off_rinv, off_cp, off_xd, off_red, bytes;
+    size_t off_H, off_A, off_part, off_x, off_x1, off_g, off_d, off_rinv, off_cp, off_xd, off_red, off_acc, bytes;
 };
 
-// C = CTAs of the cluster: CTA r holds columns [r NL, (r + 1) NL) of H (NL a multiple of 8); vectors are replicated
-__host__ __device__ inline SmallPlan small_plan(int m, int n, int C) {
+// C = CTAs of the cluster: CTA r holds columns [r NL, (r + 1) NL) of H (NL a multiple of 8); vectors are replicated.
+// acc: the plan of dopt_abpg_small_kernel, which appends three more vectors and the buffers of its wider CTA-wide sum.
+__host__ __device__ inline SmallPlan small_plan(int m, int n, int C, bool acc = false) {
     SmallPlan p;
     p.MP = (m + 15) / 16 * 16;
     p.NL = ((n + C - 1) / C + 7) / 8 * 8;
@@ -54,6 +61,7 @@ __host__ __device__ inline SmallPlan small_plan(int m, int n, int C) {
     p.off_cp = o;   o += (size_t)p.MP * 12 * 8;        // the unscaled panel of the factorisation, rows of 12 doubles
     p.off_xd = o;   o += (size_t)p.MP * 12 * 8;        // inverses of the 8 x 8 unit diagonal blocks, rows of 12 doubles
     p.off_red = o;  o += 256 * 8;                      // [0,128) CTA-wide reductions, [128,192) the prox group's
+    p.off_acc = o;  o += acc ? (size_t)3 * p.NP * 8 + (size_t)2 * SM_ACC_SUMS * SM_WARPS * 8 : 0;
     p.bytes = o;
     return p;
 }
@@ -107,21 +115,21 @@ __device__ __forceinline__ double cta_min(SmallCtx& c, double a) {
 
 // ---- this CTA's columns of H (global, L2 resident after the first pass) -> shared-memory copy; rows >= m and columns
 //      beyond the slice stay zero
-__device__ __forceinline__ void small_fill_H(const SmallCtx& c, const SmallParams& p, bool vec) {
+__device__ __forceinline__ void small_fill_H(const SmallCtx& c, const double* H, int64_t ldh, bool vec) {
     if (c.nloc <= 0) return;
     if (vec) {
         const int per_row = c.nloc >> 1;                // 16-byte chunks per row (col0 and nloc are even here)
         const int total = c.m * per_row;
         for (int e = c.tid; e < total; e += SM_THREADS) {
             const int i = e / per_row, q = e - i * per_row;
-            cp_async16(c.Hs + (size_t)i * c.ldn + 2 * q, p.H + (int64_t)i * p.ldh + c.col0 + 2 * q, 16);
+            cp_async16(c.Hs + (size_t)i * c.ldn + 2 * q, H + (int64_t)i * ldh + c.col0 + 2 * q, 16);
         }
         cp_async_commit();
     } else {
         const int total = c.m * c.nloc;
         for (int e = c.tid; e < total; e += SM_THREADS) {
             const int i = e / c.nloc, j = e - i * c.nloc;
-            c.Hs[(size_t)i * c.ldn + j] = p.H[(int64_t)i * p.ldh + c.col0 + j];
+            c.Hs[(size_t)i * c.ldn + j] = H[(int64_t)i * ldh + c.col0 + j];
         }
     }
 }
@@ -441,11 +449,12 @@ __device__ __forceinline__ void small_gradient_blocks(const SmallCtx& c, int cb0
         }
     }
 }
-template <int C>
+// NBMAX = 1: every warp walks one block at a time (same values; fewer registers, for a kernel that holds more state)
+template <int C, int NBMAX = 2>
 __device__ __forceinline__ void small_gradient(const SmallCtx& c) {
     const int ncb = c.NL >> 3;
-    for (int cb = c.warp; cb < ncb; cb += 2 * SM_WARPS) {
-        if (cb + SM_WARPS < ncb) small_gradient_blocks<2>(c, cb);
+    for (int cb = c.warp; cb < ncb; cb += NBMAX * SM_WARPS) {
+        if (NBMAX == 2 && cb + SM_WARPS < ncb) small_gradient_blocks<NBMAX>(c, cb);
         else small_gradient_blocks<1>(c, cb);
     }
     if (C > 1) {
@@ -462,7 +471,7 @@ __device__ __forceinline__ void small_gradient(const SmallCtx& c) {
     }
 }
 
-// ---- x1 <- argmin <g, x> + L D(x, y) on the simplex (Burg kernel); returns the Newton steps taken.
+// ---- out <- argmin <g, x> + L D(x, ctr) on the simplex (Burg kernel, g in c.gs); returns the Newton steps taken.
 //      Only the warps that hold elements (n / 32 of them, at most 16) run the root-find, on a named barrier of their own:
 //      the sums of a Newton step cost one barrier among those warps and the idle warps do not compete for issue slots.
 __device__ __forceinline__ void grp_bar(int nthreads) { asm volatile("bar.sync 1, %0;" ::"r"(nthreads) : "memory"); }
@@ -479,7 +488,8 @@ __device__ __forceinline__ void grp_sum2(const SmallCtx& c, int nw, int& gf, dou
     a = __shfl_sync(0xffffffffu, v, 0);
     b = __shfl_sync(0xffffffffu, v, SM_WARPS);
 }
-__device__ __forceinline__ int small_prox(SmallCtx& c, double L, double eps, uint32_t& st) {
+__device__ __forceinline__ int small_prox(SmallCtx& c, const double* ctr, double* out, double L, double eps,
+                                          uint32_t& st) {
     const int n = c.n;
     const int nw = min(SM_WARPS, (n + 31) >> 5);
     int nnewton = 0;
@@ -487,10 +497,10 @@ __device__ __forceinline__ int small_prox(SmallCtx& c, double L, double eps, uin
         int gf = 0;
         double lo = kInf;
         for (int i = c.tid; i < n; i += SM_THREADS) {
-            const double yi = c.xs[i];
+            const double yi = ctr[i];
             if (!(yi > 0.0)) st |= ACCBPG_ST_ARG_NOT_POS;
             const double v = __ddiv_rn(__dsub_rn(c.gs[i], __dmul_rn(L, -1.0 / yi)), L);      // no FMA contraction: NumPy's rounding
-            c.x1s[i] = v;
+            out[i] = v;
             lo = fmin(lo, v);
         }
         lo = warp_min(lo);
@@ -509,7 +519,7 @@ __device__ __forceinline__ int small_prox(SmallCtx& c, double L, double eps, uin
         auto sums = [&](double q) {
             double a = 0.0, b = 0.0;
             for (int i = c.tid; i < n; i += SM_THREADS) {
-                const double tq = c.x1s[i] + q;
+                const double tq = out[i] + q;
                 a += 1.0 / tq;
                 b += -1.0 / __dmul_rn(tq, tq);
             }
@@ -530,9 +540,28 @@ __device__ __forceinline__ int small_prox(SmallCtx& c, double L, double eps, uin
             fc = s1 - 1.0;
             if (++nnewton >= 200) { st |= ACCBPG_ST_NEWTON_MAXIT; break; }
         }
-        for (int i = c.tid; i < n; i += SM_THREADS) c.x1s[i] = 1.0 / (c.x1s[i] + cc);
+        for (int i = c.tid; i < n; i += SM_THREADS) out[i] = 1.0 / (out[i] + cc);
     }
     return nnewton;
+}
+
+// ---- the buffers of a plan, this CTA's rank and column slice, the thread's place in the CTA
+template <int C>
+__device__ __forceinline__ void small_ctx(SmallCtx& c, const SmallPlan& pl, unsigned char* sm_raw, int m, int n) {
+    namespace cg = cooperative_groups;
+    c.Hs = (double*)(sm_raw + pl.off_H);   c.A = (double*)(sm_raw + pl.off_A);
+    c.part = (double*)(sm_raw + pl.off_part);
+    c.xs = (double*)(sm_raw + pl.off_x);   c.x1s = (double*)(sm_raw + pl.off_x1);
+    c.gs = (double*)(sm_raw + pl.off_g);   c.dv = (double*)(sm_raw + pl.off_d);
+    c.rinv = (double*)(sm_raw + pl.off_rinv); c.Cp = (double*)(sm_raw + pl.off_cp);
+    c.Xd = (double*)(sm_raw + pl.off_xd);  c.red = (double*)(sm_raw + pl.off_red);
+    c.m = m; c.n = n; c.MP = pl.MP; c.NP = pl.NP; c.ldn = pl.ldn; c.lda = pl.lda;
+    c.C = C; c.rank = (C > 1) ? (int)cg::this_cluster().block_rank() : 0;
+    c.NL = pl.NL; c.col0 = c.rank * pl.NL; c.nloc = min(pl.NL, n - c.col0); c.nblk16 = pl.nblk16; c.gcount = 0;
+    if (c.nloc < 0) c.nloc = 0;
+    c.tid = threadIdx.x; c.lane = c.tid & 31; c.warp = c.tid >> 5; c.g = c.lane >> 2; c.t = c.lane & 3;
+    c.flip = 0;
+    c.tf0 = c.tf1 = c.tf2 = c.tf3 = 0;
 }
 
 template <int C>
@@ -541,19 +570,7 @@ __global__ void __launch_bounds__(SM_THREADS, 1) dopt_bpg_small_kernel(SmallPara
     namespace cg = cooperative_groups;
     const SmallPlan pl = small_plan(p.m, p.n, C);
     SmallCtx c;
-    c.Hs = (double*)(sm_raw + pl.off_H);   c.A = (double*)(sm_raw + pl.off_A);
-    c.part = (double*)(sm_raw + pl.off_part);
-    c.xs = (double*)(sm_raw + pl.off_x);   c.x1s = (double*)(sm_raw + pl.off_x1);
-    c.gs = (double*)(sm_raw + pl.off_g);   c.dv = (double*)(sm_raw + pl.off_d);
-    c.rinv = (double*)(sm_raw + pl.off_rinv); c.Cp = (double*)(sm_raw + pl.off_cp);
-    c.Xd = (double*)(sm_raw + pl.off_xd);  c.red = (double*)(sm_raw + pl.off_red);
-    c.m = p.m; c.n = p.n; c.MP = pl.MP; c.NP = pl.NP; c.ldn = pl.ldn; c.lda = pl.lda;
-    c.C = C; c.rank = (C > 1) ? (int)cg::this_cluster().block_rank() : 0;
-    c.NL = pl.NL; c.col0 = c.rank * pl.NL; c.nloc = min(pl.NL, p.n - c.col0); c.nblk16 = pl.nblk16; c.gcount = 0;
-    if (c.nloc < 0) c.nloc = 0;
-    c.tid = threadIdx.x; c.lane = c.tid & 31; c.warp = c.tid >> 5; c.g = c.lane >> 2; c.t = c.lane & 3;
-    c.flip = 0;
-    c.tf0 = c.tf1 = c.tf2 = c.tf3 = 0;
+    small_ctx<C>(c, pl, sm_raw, p.m, p.n);
     const bool vec = ((reinterpret_cast<uintptr_t>(p.H) & 15u) == 0) && (p.ldh % 2 == 0) && (p.n % 2 == 0);
     const bool writer = c.rank == 0;
     uint32_t st = 0;
@@ -561,7 +578,7 @@ __global__ void __launch_bounds__(SM_THREADS, 1) dopt_bpg_small_kernel(SmallPara
     for (size_t e = c.tid; e < pl.bytes / 8; e += SM_THREADS) ((double*)sm_raw)[e] = 0.0;
     __syncthreads();
     if (C > 1) cg::this_cluster().sync();               // no CTA's shared memory is written remotely before it is cleared
-    small_fill_H(c, p, vec);
+    small_fill_H(c, p.H, p.ldh, vec);
     for (int i = c.tid; i < p.n; i += SM_THREADS) {
         const double v = p.x[i];
         if (v < 0.0) st |= ACCBPG_ST_X_NEGATIVE;
@@ -588,12 +605,12 @@ __global__ void __launch_bounds__(SM_THREADS, 1) dopt_bpg_small_kernel(SmallPara
         small_gradient<C>(c);
         if (C > 1) cg::this_cluster().sync();           // the other CTAs' slices of the gradient have arrived
         else __syncthreads();
-        small_fill_H(c, p, vec);                        // refill the copy of H under the prox
+        small_fill_H(c, p.H, p.ldh, vec);                        // refill the copy of H under the prox
         SM_LAP(tp1);
         if (p.linesearch) L = L / p.ls_ratio;
         double f1 = 0.0;
         for (;;) {
-            newton += small_prox(c, L, p.eps_prox, st);
+            newton += small_prox(c, c.xs, c.x1s, L, p.eps_prox, st);
             ++trials;
             __syncthreads();                            // x1 complete
             SM_LAP(tp2);
@@ -639,9 +656,229 @@ __global__ void __launch_bounds__(SM_THREADS, 1) dopt_bpg_small_kernel(SmallPara
     }
 }
 
+// ---- ABPG / ABPG_gain (algorithms.py:94-180, :295-420) on the same machinery ---------------------------------------
+
+struct SmallAccParams {
+    const double* H; int m, n; int64_t ldh;
+    double* x;                       // in: x0, out: the last iterate
+    double L, gamma, epsilon, eps_prox, G0, ls_inc, ls_dec;
+    int maxitrs, theta_eq, restart, rule, checkdiv;
+    double* hist;                    // rows of maxitrs: F, G / Gain, Gdiv, theta, D(x,y), D(z,z-), T
+    double* info;                    // [0] entries written, [1] trips, [2] cluster size, [3] Gdr unbound, [4] last G / gain
+    uint32_t* status;
+};
+
+// ---- CTA-wide sums of K <= SM_ACC_SUMS values with one barrier: warps leave their partials in one of two alternating
+//      buffers, every thread adds them in warp order (the same bits in every thread, and in every CTA given the same
+//      inputs)
+template <int K>
+__device__ __forceinline__ void cta_sumk(const SmallCtx& c, double* red, int& flip, double (&v)[K]) {
+    double* s = red + flip * (SM_ACC_SUMS * SM_WARPS);
+    flip ^= 1;
+#pragma unroll
+    for (int q = 0; q < K; ++q) {
+        v[q] = warp_sum(v[q]);
+        if (c.lane == 0) s[q * SM_WARPS + c.warp] = v[q];
+    }
+    __syncthreads();
+#pragma unroll
+    for (int q = 0; q < K; ++q) {
+        double a = s[q * SM_WARPS];
+#pragma unroll
+        for (int w = 1; w < SM_WARPS; ++w) a = __dadd_rn(a, s[q * SM_WARPS + w]);
+        v[q] = a;
+    }
+}
+
+// ---- f(v) = -log det(H diag(v) H^T) from scratch: waits for this CTA's refill of its slice of H (only this CTA reads
+//      it), then Gram matrix and factorisation; the factor stays in c.A for small_gradient
+template <int C>
+__device__ __forceinline__ double small_value(SmallCtx& c, const double* v, bool vec, bool& bad) {
+    if (vec) cp_async_wait<0>();
+    __syncthreads();                                    // v complete, the refilled H visible
+    small_gram<C>(c, v);
+    __syncthreads();
+    return small_factor(c, bad);
+}
+
+// Every point is evaluated from scratch, as the reference does; carrying the Gram images M(x-), M(z-) and M(z) next to H
+// would not fit one SM at 80 x 200.  An iteration starts with f(x_k) = F[k] when no trip has formed it, then each trip:
+//   1. y = (1-theta) x- + theta z-; Gram, factor, f(y); gradient g at y in place on the copy of H, whose refill starts
+//   2. z = div_prox_map(z-, g, theta^(gamma-1) [G] L)
+//   3. x = (1-theta) x- + theta z; D(x, y), D(z, z-), dot(g, x - y), the restart dot dot(g, x - x-) and the status in
+//      one CTA-wide sum
+//   4. ABPG_gain without checkdiv, after the refill: Gram, factor, f(x) for the line search (:387); the accepted trip's
+//      value is F[k+1]
+// The scalar and elementwise expressions round like the host's Python / NumPy arithmetic and accbpg_vec_axpby (explicit
+// round-to-nearest operations: this file is compiled with FMA contraction).  Every CTA takes every decision from the
+// same bits: the vectors are replicated and the Gram matrix is summed in rank order.  What a decision needs after a
+// Gram pass is reduced to a few values before it (the restart tests, the line search's right-hand side), so the scalar
+// control does not add to the register pressure of the passes.
+template <int C, int DRV>
+__global__ void __launch_bounds__(SM_THREADS, 1) dopt_abpg_small_kernel(SmallAccParams p) {
+    extern __shared__ __align__(16) unsigned char sm_raw[];
+    namespace cg = cooperative_groups;
+    constexpr bool GAIN = DRV == ACCBPG_SMALL_DRV_ABPG_GAIN;
+    const unsigned long long ns0 = ls_clock();
+    const SmallPlan pl = small_plan(p.m, p.n, C, true);
+    SmallCtx c;
+    small_ctx<C>(c, pl, sm_raw, p.m, p.n);
+    double* const X1 = c.xs;                            // x-
+    double* const Z1 = c.x1s;                           // z-
+    double* const Y = (double*)(sm_raw + pl.off_acc);
+    double* const Z = Y + pl.NP;
+    double* const X = Z + pl.NP;
+    double* const red = X + pl.NP;
+    int rflip = 0;
+    const bool vec = ((reinterpret_cast<uintptr_t>(p.H) & 15u) == 0) && (p.ldh % 2 == 0) && (p.n % 2 == 0);
+    const bool writer = c.rank == 0 && c.tid == 0;
+    const int n = p.n, M = p.maxitrs;
+    auto hist = [&](int row, int k) -> double& { return p.hist[(size_t)row * M + k]; };   // rows: see SmallAccParams
+    uint32_t st = 0;
+
+    for (size_t e = c.tid; e < pl.bytes / 8; e += SM_THREADS) ((double*)sm_raw)[e] = 0.0;
+    __syncthreads();
+    if (C > 1) cg::this_cluster().sync();               // no CTA's shared memory is written remotely before it is cleared
+    small_fill_H(c, p.H, p.ldh, vec);
+    for (int i = c.tid; i < n; i += SM_THREADS) {       // x0 and z0 = x0
+        const double v = p.x[i];
+        if (v < 0.0) st |= ACCBPG_ST_X_NEGATIVE;
+        X1[i] = v;
+        Z1[i] = v;
+    }
+    bool stop;
+    {
+        double s0 = st ? 1.0 : 0.0, s1 = 0.0;           // a negative entry of x0 ends the solve before f(x0)
+        cta_sum2(c, s0, s1);
+        stop = s0 > 0.0;
+    }
+
+    double theta = 1.0, G = p.G0, gdr = 0.0, fx = 0.0, Fprev = 0.0;
+    bool have_fx = false, gdr_bound = false;
+    int kk = 0, k = 0, trips = 0, unbound = 0, newton = 0;
+    for (; k < M && !stop; ++k) {
+        if (writer) hist(6, k) = (double)(ls_clock() - ns0);
+        if (!have_fx) {                                 // F[k] = f(x_k) from scratch
+            bool bad = false;
+            fx = small_value<C>(c, X1, vec, bad);
+            if (bad) { st |= ACCBPG_ST_NOT_PD; break; }
+        }
+        if (writer) hist(0, k) = fx;
+        // restart rule 'f' (algorithms.py:168, :406): F[k] > F[k-1]; ABPG_gain's at k = 0 compares with F[-1], the
+        // reference's still-zero last slot
+        const bool rs_f = fx > (k > 0 ? Fprev : (M == 1 ? fx : 0.0));
+        Fprev = fx;
+        const double G_1 = G, theta_1 = theta;
+        if (GAIN) G = __ddiv_rn(G, p.ls_dec);
+        else theta = (p.theta_eq && kk > 0) ? la_solve_theta(theta, p.gamma, 1.0)
+                                            : __ddiv_rn(p.gamma, __dadd_rn((double)kk, p.gamma));
+        bool rs_g = false, dzz_small = false;
+        for (;;) {
+            ++trips;
+            have_fx = false;
+            if (GAIN && kk > 0) {
+                if (p.theta_eq) {
+                    theta = la_solve_theta(theta_1, p.gamma, __ddiv_rn(G, G_1));
+                } else {
+                    const double alpha = __ddiv_rn(G, G_1);                           // algorithms.py:367
+                    theta = __dmul_rn(theta_1, __ddiv_rn(__dadd_rn(1.0, __dmul_rn(alpha, __dsub_rn(p.gamma, 1.0))),
+                                                         __dadd_rn(__dmul_rn(p.gamma, alpha), theta_1)));
+                }
+            }
+            // 1. y, f(y), g = grad f(y); the copy of H is refilled under steps 2 and 3
+            {
+                const double omt = __dsub_rn(1.0, theta);
+                for (int i = c.tid; i < n; i += SM_THREADS)
+                    Y[i] = __dadd_rn(__dmul_rn(omt, X1[i]), __dmul_rn(theta, Z1[i]));
+            }
+            bool bad = false;
+            const double fy = small_value<C>(c, Y, vec, bad);
+            if (bad) { st |= ACCBPG_ST_NOT_PD; stop = true; break; }
+            small_gradient<C, 1>(c);
+            if (C > 1) cg::this_cluster().sync();       // the other CTAs' slices of the gradient have arrived
+            else __syncthreads();
+            small_fill_H(c, p.H, p.ldh, vec);
+            // 2. z
+            {
+                const double tg1 = la_pow(theta, __dsub_rn(p.gamma, 1.0));
+                const double Lz = GAIN ? __dmul_rn(__dmul_rn(tg1, G), p.L) : __dmul_rn(tg1, p.L);
+                newton += small_prox(c, Z1, Z, Lz, p.eps_prox, st);
+            }
+            __syncthreads();                            // z complete
+            // 3. x and the trip's sums: D(x, y), D(z, z-), dot(g, x - y), dot(g, x - x-), status
+            double a[SM_ACC_SUMS] = {0.0, 0.0, 0.0, 0.0, 0.0};
+            {
+                const double omt = __dsub_rn(1.0, theta);
+                for (int i = c.tid; i < n; i += SM_THREADS) {
+                    const double x1i = X1[i], z1i = Z1[i], zi = Z[i], yi = Y[i], gi = c.gs[i];
+                    const double xi = __dadd_rn(__dmul_rn(omt, x1i), __dmul_rn(theta, zi));
+                    X[i] = xi;
+                    if (!(xi > 0.0) || !(zi > 0.0)) st |= ACCBPG_ST_ARG_NOT_POS;
+                    const double r = __ddiv_rn(xi, yi), q = __ddiv_rn(zi, z1i);
+                    a[0] = __dadd_rn(a[0], __dsub_rn(__dsub_rn(r, log(r)), 1.0));
+                    a[1] = __dadd_rn(a[1], __dsub_rn(__dsub_rn(q, log(q)), 1.0));
+                    a[2] = __dadd_rn(a[2], __dmul_rn(gi, __dsub_rn(xi, yi)));
+                    a[3] = __dadd_rn(a[3], __dmul_rn(gi, __dsub_rn(xi, x1i)));
+                }
+            }
+            a[4] = st ? 1.0 : 0.0;
+            cta_sumk<SM_ACC_SUMS>(c, red, rflip, a);    // (its barrier also publishes x)
+            if (a[4] > 0.0) { stop = true; break; }
+            const double tg = la_pow(theta, p.gamma);
+            if (writer) { hist(3, k) = theta; hist(4, k) = a[0]; hist(5, k) = a[1]; }
+            rs_g = a[3] > 0.0;
+            dzz_small = a[1] < p.epsilon;
+            if (GAIN && dzz_small) break;               // Gdr keeps its previous value, as in the reference
+            gdr = __ddiv_rn(__ddiv_rn(a[0], a[1]), tg);
+            if (!GAIN) break;
+            gdr_bound = true;
+            bool again;
+            if (p.checkdiv) {
+                again = gdr > G;
+            } else {
+                const double rhs = __dadd_rn(__dadd_rn(fy, a[2]), __dmul_rn(__dmul_rn(__dmul_rn(tg, G), p.L), a[1]));
+                fx = small_value<C>(c, X, vec, bad);    // 4.
+                if (bad) { st |= ACCBPG_ST_NOT_PD; stop = true; break; }
+                have_fx = true;
+                again = fx > rhs;                       // algorithms.py:387
+            }
+            if (!again) break;
+            G = __dmul_rn(G, p.ls_inc);
+        }
+        if (stop) { ++k; break; }
+        if (GAIN && !gdr_bound) { unbound = 1; break; }  // the reference's Gdiv[k] = Gdr raises UnboundLocalError
+        if (writer) {
+            hist(1, k) = GAIN ? G : gdr;
+            if (GAIN) hist(2, k) = gdr;
+        }
+        ++kk;
+        // restart (algorithms.py:168, :406): ABPG only from k = 1, ABPG_gain from k = 0
+        bool rs = false;
+        if (p.restart && (GAIN || k > 0))
+            rs = p.rule == ACCBPG_SMALL_RESTART_F ? rs_f : p.rule == ACCBPG_SMALL_RESTART_G ? rs_g : false;
+        if (rs) { theta = 1.0; kk = 0; }
+        for (int i = c.tid; i < n; i += SM_THREADS) {  // x- <- x, z- <- z (x on a restart)
+            const double xi = X[i];
+            X1[i] = xi;
+            Z1[i] = rs ? xi : Z[i];
+        }
+        if (dzz_small) { ++k; break; }
+    }
+    if (vec) cp_async_wait<0>();                        // a refill still in flight when a status bit ended the solve
+    if (C > 1) cg::this_cluster().sync();               // nobody leaves while its shared memory may still be read
+    if (c.rank == 0)
+        for (int i = c.tid; i < n; i += SM_THREADS) p.x[i] = X1[i];
+    if (st) atomicOr(p.status, st);
+    if (writer) {
+        p.info[0] = (double)k; p.info[1] = (double)trips; p.info[2] = (double)C; p.info[3] = (double)unbound;
+        p.info[4] = GAIN ? G : gdr; p.info[5] = (double)newton;
+    }
+}
+
 // cluster size for a shape: the largest of {preferred, 2, 1} whose plan fits one SM's shared memory (a cluster also
 // admits shapes whose H does not fit a single CTA).  ACCBPG_SMALL_CLUSTER = 1 / 2 / 4 overrides the preference.
-static int small_pick_cluster(int m, int64_t n, size_t* bytes) {
+// acc: the plan of dopt_abpg_small_kernel.
+static int small_pick_cluster(int m, int64_t n, size_t* bytes, bool acc = false) {
     if (m < 1 || m > SM_MAX_M || n < 2 || n > 65536 || n <= m) return 0;
     static int pref = 0;
     if (pref == 0) { const char* e = getenv("ACCBPG_SMALL_CLUSTER"); pref = e ? atoi(e) : 4; if (pref != 1 && pref != 2 && pref != 4) pref = 4; }
@@ -649,17 +886,17 @@ static int small_pick_cluster(int m, int64_t n, size_t* bytes) {
     for (int q = 0; q < 3; ++q) {
         const int C = cand[q];
         if (C > 1 && n < 32 * C) continue;              // too few columns to be worth splitting
-        const SmallPlan pl = small_plan(m, (int)n, C);
+        const SmallPlan pl = small_plan(m, (int)n, C, acc);
         if (pl.bytes <= (size_t)SM_SMEM_LIMIT) { if (bytes) *bytes = pl.bytes; return C; }
     }
     return 0;
 }
 
-template <int C>
-static int small_launch(Ctx* c, cudaStream_t s, const SmallParams& p, size_t smem) {
+template <auto KERNEL, class P>
+static int small_launch(Ctx* c, cudaStream_t s, const P& p, int C, size_t smem) {
     static bool attr_done[kMaxDevices] = {};
     if (!(c->device >= 0 && c->device < kMaxDevices && attr_done[c->device])) {
-        ACCBPG_CUDA(cudaFuncSetAttribute(dopt_bpg_small_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, SM_SMEM_LIMIT));
+        ACCBPG_CUDA(cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, SM_SMEM_LIMIT));
         if (c->device >= 0 && c->device < kMaxDevices) attr_done[c->device] = true;
     }
     cudaLaunchConfig_t cfg = {};
@@ -674,8 +911,15 @@ static int small_launch(Ctx* c, cudaStream_t s, const SmallParams& p, size_t sme
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = C > 1 ? 1 : 0;
-    ACCBPG_CUDA(cudaLaunchKernelEx(&cfg, dopt_bpg_small_kernel<C>, p));
+    ACCBPG_CUDA(cudaLaunchKernelEx(&cfg, KERNEL, p));
     return ACCBPG_OK;
+}
+
+template <int DRV>
+static int small_acc_launch(Ctx* c, cudaStream_t s, const SmallAccParams& p, int C, size_t smem) {
+    return C == 4 ? small_launch<dopt_abpg_small_kernel<4, DRV>>(c, s, p, C, smem)
+         : C == 2 ? small_launch<dopt_abpg_small_kernel<2, DRV>>(c, s, p, C, smem)
+                  : small_launch<dopt_abpg_small_kernel<1, DRV>>(c, s, p, C, smem);
 }
 
 }  // namespace accbpg
@@ -704,9 +948,46 @@ int accbpg_dopt_bpg_small(void* ctx, void* stream, const double* H, int m, int64
     p.H = H; p.m = m; p.n = (int)n; p.ldh = ldh; p.x = x; p.L = L; p.ls_ratio = ls_ratio; p.epsilon = epsilon;
     p.eps_prox = eps_prox; p.linesearch = linesearch; p.maxitrs = maxitrs; p.F = F_out; p.Ls = Ls_out; p.info = info_out;
     p.status = c->d_status;
-    int rc = C == 4 ? small_launch<4>(c, s, p, smem) : C == 2 ? small_launch<2>(c, s, p, smem) : small_launch<1>(c, s, p, smem);
+    int rc = C == 4 ? small_launch<dopt_bpg_small_kernel<4>>(c, s, p, C, smem)
+           : C == 2 ? small_launch<dopt_bpg_small_kernel<2>>(c, s, p, C, smem)
+                    : small_launch<dopt_bpg_small_kernel<1>>(c, s, p, C, smem);
     if (rc) return rc;
     ACCBPG_LAUNCHED("dopt_bpg_small_kernel");
+    return ACCBPG_OK;
+}
+
+size_t accbpg_dopt_abpg_small_smem_bytes(int m, int64_t n) {
+    size_t bytes = 0;
+    return small_pick_cluster(m, n, &bytes, true) ? bytes : 0;
+}
+
+int accbpg_dopt_abpg_small(void* ctx, void* stream, int driver, const double* H, int m, int64_t n, int64_t ldh,
+                           double* x, double L, double gamma, int maxitrs, double epsilon, double eps_prox,
+                           int theta_eq, int restart, int restart_rule, double G0, double ls_inc, double ls_dec,
+                           int checkdiv, double* hist, double* info_out) {
+    Ctx* c = (Ctx*)ctx;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (!c || !H || !x || !hist || !info_out) return arg_err("dopt_abpg_small: NULL pointer");
+    ACCBPG_ON_DEVICE(c);
+    if (driver != ACCBPG_SMALL_DRV_ABPG && driver != ACCBPG_SMALL_DRV_ABPG_GAIN) return arg_err("dopt_abpg_small: driver");
+    size_t smem = 0;
+    const int C = small_pick_cluster(m, n, &smem, true);
+    if (C == 0 || ldh < n)
+        return arg_err("dopt_abpg_small: shape does not fit one SM (accbpg_dopt_abpg_small_smem_bytes)");
+    auto pos = [](double v) { return isfinite(v) && v > 0.0; };
+    if (!pos(L) || !pos(gamma) || !pos(G0) || !pos(ls_inc) || !pos(ls_dec) || !pos(eps_prox))
+        return arg_err("dopt_abpg_small: L, gamma, G0, ls_inc, ls_dec, eps_prox must be finite and > 0");
+    if (maxitrs < 1 || restart_rule < ACCBPG_SMALL_RESTART_NONE || restart_rule > ACCBPG_SMALL_RESTART_G)
+        return arg_err("dopt_abpg_small: maxitrs, restart_rule");
+    SmallAccParams p = {};
+    p.H = H; p.m = m; p.n = (int)n; p.ldh = ldh; p.x = x; p.L = L; p.gamma = gamma; p.epsilon = epsilon;
+    p.eps_prox = eps_prox; p.G0 = G0; p.ls_inc = ls_inc; p.ls_dec = ls_dec; p.maxitrs = maxitrs;
+    p.theta_eq = theta_eq != 0; p.restart = restart != 0; p.rule = restart_rule; p.checkdiv = checkdiv != 0;
+    p.hist = hist; p.info = info_out; p.status = c->d_status;
+    int rc = driver == ACCBPG_SMALL_DRV_ABPG_GAIN ? small_acc_launch<ACCBPG_SMALL_DRV_ABPG_GAIN>(c, s, p, C, smem)
+                                                  : small_acc_launch<ACCBPG_SMALL_DRV_ABPG>(c, s, p, C, smem);
+    if (rc) return rc;
+    ACCBPG_LAUNCHED("dopt_abpg_small_kernel");
     return ACCBPG_OK;
 }
 

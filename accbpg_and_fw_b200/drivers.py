@@ -280,40 +280,56 @@ def _bpg_small(f, h, L, x0, maxitrs, epsilon, linesearch, ls_ratio, verbose, ver
 
 def _abpg_small(gain, f, h, L, x0, gamma, maxitrs, epsilon, theta_eq, restart, restart_rule, G0=1.0, ls_inc=1.2,
                 ls_dec=1.2, checkdiv=False):
-    """config.fused_small: the whole ABPG / ABPG_gain solve as one kernel launch (accbpg_linreg_abpg_small) on a
-    PoissonRegression / KLdivRegression instance whose A fits the shared memory of a cluster of at most 8 SMs, with a
-    kernel that accbpg_linreg_bpg_small covers.  It reproduces the operator loop's default scheme (carried linear
-    images), so it is taken only with config.linear_images on.  Returns None when no fused solve applies, else
-    (x, hist rows, k, T): the history rows F, G / Gain, Gdiv, theta, D(x,y), D(z,z-) truncated to the k entries written,
-    and T from the device clock at the top of each iteration, offset by the host time of the launch.
-    `_abpg_small.last_info` keeps the kernel's info array."""
-    from .objectives import PoissonRegression, KLdivRegression
-    if not (config.fused_small and config.linear_images) or maxitrs < 1:
+    """config.fused_small: the whole ABPG / ABPG_gain solve as one kernel launch on an unsharded instance that fits:
+    - a DOptimalObj with BurgEntropySimplex whose H fits the shared memory of one SM or of a cluster of 2 or 4
+      (accbpg_dopt_abpg_small).  It evaluates every point from scratch, which is what config.linear_images = False
+      asks for; the operator loop's carried Gram images agree with that to rounding, so it is taken under both
+      settings of config.linear_images;
+    - a PoissonRegression / KLdivRegression instance whose A fits the shared memory of a cluster of at most 8 SMs, with
+      a kernel that accbpg_linreg_bpg_small covers (accbpg_linreg_abpg_small).  It reproduces the operator loop's
+      default scheme (carried linear images), so it is taken only with config.linear_images on.
+    Returns None when no fused solve applies, else (x, hist rows, k, T): the history rows F, G / Gain, Gdiv, theta,
+    D(x,y), D(z,z-) truncated to the k entries written, and T from the device clock at the top of each iteration, offset
+    by the host time of the launch.  `_abpg_small.last_info` keeps the kernel's info array."""
+    from .objectives import DOptimalObj, PoissonRegression, KLdivRegression
+    from .bregman import BurgEntropySimplex
+    if not config.fused_small or maxitrs < 1:
         return None
-    if type(f) not in (PoissonRegression, KLdivRegression) or _small_hkind(h) is None:
+    dopt = type(f) is DOptimalObj and type(h) is BurgEntropySimplex
+    if not dopt and (not config.linear_images or type(f) not in (PoissonRegression, KLdivRegression) or
+                     _small_hkind(h) is None):
         return None
     if f.shard is not None or h.shard is not None:
         return None
     if not all(np.isfinite(v) and v > 0 for v in (L, gamma, G0, ls_inc, ls_dec)):
         return None
-    if lib.accbpg_linreg_abpg_small_smem_bytes(f.m, f.n) == 0:
+    if dopt and (not (np.isfinite(h.eps) and h.eps > 0) or lib.accbpg_dopt_abpg_small_smem_bytes(f.m, f.n) == 0):
+        return None
+    if not dopt and lib.accbpg_linreg_abpg_small_smem_bytes(f.m, f.n) == 0:
         return None
     t0 = time.time()
     rt = f.rt
     x = rt.to_device(x0).clone()
     hist = torch.empty(7 * maxitrs + 16, dtype=torch.float64, device=rt.device)
     base = hist.data_ptr()
-    A = f._Ad
-    rule = {'f': "F", 'g': "G"}.get(restart_rule, "NONE")
-    drv = "ABPG_GAIN" if gain else "ABPG"
+    rule = nat.MACROS["ACCBPG_SMALL_RESTART_" + {'f': "F", 'g': "G"}.get(restart_rule, "NONE")]
+    drv = nat.MACROS["ACCBPG_SMALL_DRV_" + ("ABPG_GAIN" if gain else "ABPG")]
     with rt.on_device():
         t_launch = time.time() - t0
-        nat.check(lib.accbpg_linreg_abpg_small(
-            rt.ctx, rt.stream, nat.MACROS["ACCBPG_SMALL_DRV_" + drv], f._kind, A.data_ptr(), f.m, f.n, A.stride(0),
-            f._bd.data_ptr(), _small_hkind(h), float(h.lamda), float(getattr(h, "delta", 0.0)), x.data_ptr(), float(L),
-            float(gamma), int(maxitrs), float(epsilon), 1 if theta_eq else 0, 1 if restart else 0,
-            nat.MACROS["ACCBPG_SMALL_RESTART_" + rule], float(G0), float(ls_inc), float(ls_dec), 1 if checkdiv else 0,
-            max(int(config.reanchor_every), 1), base, base + 8 * 7 * maxitrs))
+        if dopt:
+            H = f._Hd
+            nat.check(lib.accbpg_dopt_abpg_small(
+                rt.ctx, rt.stream, drv, H.data_ptr(), f.m, f.n, H.stride(0), x.data_ptr(), float(L), float(gamma),
+                int(maxitrs), float(epsilon), float(h.eps), 1 if theta_eq else 0, 1 if restart else 0, rule, float(G0),
+                float(ls_inc), float(ls_dec), 1 if checkdiv else 0, base, base + 8 * 7 * maxitrs))
+        else:
+            A = f._Ad
+            nat.check(lib.accbpg_linreg_abpg_small(
+                rt.ctx, rt.stream, drv, f._kind, A.data_ptr(), f.m, f.n, A.stride(0), f._bd.data_ptr(),
+                _small_hkind(h), float(h.lamda), float(getattr(h, "delta", 0.0)), x.data_ptr(), float(L), float(gamma),
+                int(maxitrs), float(epsilon), 1 if theta_eq else 0, 1 if restart else 0, rule, float(G0),
+                float(ls_inc), float(ls_dec), 1 if checkdiv else 0, max(int(config.reanchor_every), 1), base,
+                base + 8 * 7 * maxitrs))
     rt.read(rt.S_F, 1)                                   # synchronises and raises on a status bit
     hh = hist.cpu().numpy()
     info = hh[7 * maxitrs:7 * maxitrs + 16].copy()

@@ -36,7 +36,7 @@
 extern "C" {
 #endif
 
-#define ACCBPG_ABI_VERSION 6
+#define ACCBPG_ABI_VERSION 7
 
 /* return codes */
 #define ACCBPG_OK      0
@@ -292,6 +292,36 @@ size_t accbpg_dopt_bpg_small_smem_bytes(int m, int64_t n);
 int accbpg_dopt_bpg_small(void* ctx, void* stream, const double* d_H, int m, int64_t n, int64_t ldh, double* d_x, double L,
                           double ls_ratio, int linesearch, int maxitrs, double epsilon, double eps_prox, double* d_F,
                           double* d_Ls, double* d_info);
+
+/* ---- small shapes: the WHOLE ABPG (accbpg/algorithms.py:94-180) or ABPG_gain (:295-420) solve in one launch, with
+ *      DOptimalObj and BurgEntropySimplex, on the machinery of accbpg_dopt_bpg_small (one CTA or a cluster of 2 / 4,
+ *      Gram matrix, factorisation, in-place gradient, Burg-simplex root-find) in a shared-memory plan of its own (three
+ *      more vectors: accbpg_dopt_abpg_small_smem_bytes).  Every point is evaluated from scratch, as the reference does
+ *      (no carried Gram images).  Per trip: y = (1-theta) x- + theta z- (:147, :369), f(y) and g = grad f(y)
+ *      (functions.py:43-58), z = div_prox_map(z-, g, theta^(gamma-1) [G] L) (functions.py:341-356),
+ *      x = (1-theta) x- + theta z (:150, :374), D(x, y) and D(z, z-), and for ABPG_gain's line search f(x) (:387),
+ *      which for the accepted trip is F[k+1].  ABPG, and ABPG_gain with checkdiv, evaluate F[k+1] = f(x_{k+1}) at the
+ *      top of the next iteration.
+ *      The decisions are those of accbpg_linreg_abpg_small: theta = gamma/(k+gamma), solve_theta (:75-91) when
+ *      theta_eq, the alpha form (:367) for ABPG_gain otherwise; G /= ls_dec per iteration and G *= ls_inc per rejected
+ *      trip; checkdiv; restart rules 'f' and 'g' (:168, :406; ABPG from k = 1, ABPG_gain from k = 0); the stop
+ *      D(z, z-) < epsilon.  Every CTA takes them from the same bits; the scalar and elementwise expressions round like
+ *      the host's arithmetic.
+ *      driver: ACCBPG_SMALL_DRV_*; restart_rule: ACCBPG_SMALL_RESTART_* (both defined below).  G0, ls_inc, ls_dec and
+ *      checkdiv are read by ABPG_gain only.  eps_prox: BurgEntropySimplex's root-find tolerance.
+ *      d_x: x0 in, last iterate out.  d_hist: 7 rows of maxitrs doubles, row r at d_hist + r * maxitrs: [0] F, [1] G
+ *      (ABPG) or Gain (ABPG_gain), [2] Gdiv (ABPG_gain; the previous value when a trip stops on D(z, z-) < epsilon),
+ *      [3] theta, [4] D(x, y), [5] D(z, z-), [6] T (%globaltimer nanoseconds at the top of the iteration since the kernel
+ *      started).  d_info (16 doubles): [0] entries written, [1] trips, [2] cluster size, [3] 1 when the very first trip
+ *      stopped on D(z, z-) < epsilon, where the reference's Gdr is unbound (the solve ends there), [4] the last G (ABPG)
+ *      or gain (ABPG_gain), [5] Newton steps of all root-finds.  Status bits as accbpg_dopt_bpg_small's; the first one
+ *      ends the solve.  ACCBPG_E_ARG on NULL pointers, a shape that does not fit, ldh < n, non-finite or non-positive L,
+ *      gamma, G0, ls_inc, ls_dec or eps_prox, maxitrs < 1, an unknown driver or restart rule. */
+size_t accbpg_dopt_abpg_small_smem_bytes(int m, int64_t n);
+int accbpg_dopt_abpg_small(void* ctx, void* stream, int driver, const double* d_H, int m, int64_t n, int64_t ldh,
+                           double* d_x, double L, double gamma, int maxitrs, double epsilon, double eps_prox,
+                           int theta_eq, int restart, int restart_rule, double G0, double ls_inc, double ls_dec,
+                           int checkdiv, double* d_hist, double* d_info);
 
 /* ---- Poisson / KL regression objectives (accbpg/functions.py:102-120, :140-158).  A is m x n_local. */
 #define ACCBPG_LINREG_POISSON 0   /* f = sum b log(b/Ax) + Ax - b ; r = 1 - b/Ax   */
