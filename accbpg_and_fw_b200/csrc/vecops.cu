@@ -317,10 +317,10 @@ __global__ void __launch_bounds__(kThreads) argext_kernel(int64_t n, const doubl
     double v = kInf;
     long long idx = 0x7fffffffffffffffLL;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
-        double xi = sign * x[i];
-        if (xi < v) { v = xi; idx = i; }       // strict: first index wins inside a thread
-    }
+    // i only grows, so a tie is taken only while idx still holds the empty marker: the first index wins inside a thread,
+    // and a thread whose elements are all +inf (after the sign) reports the first of them, as np.argmin does
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
+        arg_combine(v, idx, sign * x[i], i);
     block_argmin(v, idx, shv, shi);
     if (threadIdx.x == 0) { partials[blockIdx.x] = v; ipartials[blockIdx.x] = idx; }
     if (last_block_ticket(counter, &is_last)) {
